@@ -2,11 +2,15 @@
 """bench.py -- LightGCN train triples/s (+ full-rank eval users/s) on synthetic
 Gowalla-shaped data, B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  A "step" is one BPR batch of 2048 triples through
 the whole hot path: L=3 propagation forward, fused loss, backward, Adam
 (recommender/LightGCN.py:47-64 of the reference).  See DESIGN.md "Measurement".
+
+--dump-outputs DIR also writes the tables after the last timed step, that step's loss row and the last timed
+evaluation's top-K and per-user metrics as DIR/<name>.npy: the inputs are seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -42,19 +46,34 @@ def log(*a):
 
 # ----------------------------------------------------------------------------- data
 def make_data(name, alpha, seed=0):
+    # generated on every run (about a second at the Gowalla shape) rather than cached: a cached graph would outlive a
+    # change of the generator and feed two builds different inputs
     from arlib_b200.util.synth import synth_edges
     U, I, E, L, d, B = WORKLOADS[name]
-    cache = os.path.join("/tmp", "arlib_b200_synth_%s_%s_%d.npz" % (name, alpha, seed))
-    if os.path.exists(cache):
-        z = np.load(cache)
-        tu, ti, su, si = z["tu"], z["ti"], z["su"], z["si"]
-    else:
-        tu, ti, su, si = synth_edges(U, I, E, alpha, alpha, seed)
-        try:
-            np.savez(cache, tu=tu, ti=ti, su=su, si=si)
-        except OSError:
-            pass
+    tu, ti, su, si = synth_edges(U, I, E, alpha, alpha, seed)
     return dict(U=U, I=I, E=E, L=L, d=d, B=B, tu=tu, ti=ti, su=su, si=si)
+
+
+DUMP_BUDGET_BYTES = 63_000_000       # under 64 MB with the .npy headers
+
+
+def dump_outputs(out_dir, arrays, budget=DUMP_BUDGET_BYTES):
+    """Write ``{name: array}`` as ``out_dir/<name>.npy`` (float32 stays float32, everything else becomes float64).
+    When the arrays exceed ``budget`` bytes in all, every array of two or more dimensions keeps a fixed, seeded sample
+    of its rows (the same rows for arrays of the same length) and ``<name>_rows.npy`` holds the row numbers kept."""
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: v if v.dtype == np.float32 else v.astype(np.float64) for k, v in arrays.items()}
+    sampled = lambda v: v.ndim >= 2
+    total = sum(v.nbytes + (8 * v.shape[0] if sampled(v) else 0) for v in arrays.values())
+    keep = budget / total if total > budget else 1.0
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        if keep < 1.0 and sampled(v):
+            n = v.shape[0]
+            rows = np.sort(np.random.default_rng(0).choice(n, max(1, int(n * keep)), replace=False))
+            v = v[rows]
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+        np.save(os.path.join(out_dir, name + ".npy"), v)
 
 
 def xavier_tables(U, I, d, seed=2018):
@@ -375,6 +394,8 @@ def run_ours(args):
             eng.run_steps(c[0], c[1], use_graph=use_graph)
         e1.record()
         barrier()
+        if args.dump_outputs:           # what the last timed step left, before the untimed steps below train on
+            dump = {"table": eng.full_table(eng.E0).clone(), "loss": eng.out4[chunks[-1][0] + chunks[-1][1] - 1].clone()}
         # keep the GPU under the same load while NVML gets enough samples (not timed)
         for _ in range(3 if world > 1 else 8):
             eng.run_steps(chunks[0][0], min(chunks[0][1], 200), use_graph=use_graph)
@@ -524,6 +545,8 @@ def run_ours(args):
     ev_each = sorted(evs[k_].elapsed_time(evs[k_ + 1]) for k_ in range(reps))
     ev_ms_mean = max_over_ranks(evs[0].elapsed_time(evs[-1])) / reps
     ev_ms = max_over_ranks(ev_each[reps // 2])
+    if args.dump_outputs:
+        dump.update(topk_scores=vals, topk_items=idx, eval_metrics=per)
     t0 = time.perf_counter()
     vals, idx = ev.topk(F[:U], F[U:], TOPK)
     measure = ev.measure(idx, [TOPK])
@@ -638,6 +661,10 @@ def run_ours(args):
                     "speedup_eval_e2e": evald["e2e_users_per_s"] / g_["users_per_s"]}
             except Exception as ex:          # the baseline must never take the bench line down with it
                 line["gpu_eager_baseline"] = {"unavailable": repr(ex)[:300]}
+    if rank == 0 and args.dump_outputs:
+        table = dump.pop("table").cpu().numpy()
+        dump = {k: v.cpu().numpy() for k, v in dump.items()}
+        dump_outputs(args.dump_outputs, {"user_emb": table[:U], "item_emb": table[U:], **dump})
     if rank == 0:
         print(json.dumps(line), flush=True)
     if world > 1:
@@ -829,7 +856,13 @@ def main():
     ap.add_argument("--alpha", type=float, default=0.5)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-epoch-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed training step and the last timed evaluation computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload in SCALE_SHAPES):
+        ap.error("--dump-outputs needs --impl ours and a workload of %s" % ", ".join(sorted(WORKLOADS)))
     if args.workload in SCALE_SHAPES:
         if args.impl == "reference":
             if int(os.environ.get("RANK", "0")) == 0:

@@ -26,6 +26,18 @@ def pytest_collection_modifyitems(config, items):
             item.add_marker(skip)
 
 
+@pytest.fixture(scope="module")
+def one_cpu_thread():
+    """CPU torch on one thread: with several, the sparse backward of the oracle trainers sums in a different order
+    from run to run, and over an epoch of Adam (SimGCL's sign() perturbation above all) that drift can exceed the
+    tolerances the trainers are pinned to."""
+    import torch
+    n = torch.get_num_threads()
+    torch.set_num_threads(1)
+    yield
+    torch.set_num_threads(n)
+
+
 @pytest.fixture(scope="session")
 def golden():
     import numpy as np

@@ -8,6 +8,8 @@ import torch
 
 from oracle import port
 
+pytestmark = pytest.mark.usefixtures("one_cpu_thread")
+
 
 @pytest.fixture(scope="module")
 def pdata(golden_rows):

@@ -12,6 +12,8 @@ from oracle import port
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 NOISE_SEED = 20180
 
+pytestmark = pytest.mark.usefixtures("one_cpu_thread")
+
 
 def _meta(g):
     out = {}
@@ -105,7 +107,15 @@ def test_contrastive_epoch_and_forward(name, golden, pdata):
 
 
 def test_infonce_known_answers():
+    """The vectors were frozen on one CPU model, where the port matched the reference bit for bit.  Torch's CPU
+    matrix and vector-math kernels round differently on other CPU models (on some the loss moves by one float32 ulp
+    and gradient elements by up to 5e-7 of the gradient's largest magnitude), so the check is held at float32
+    rounding level: the loss to 5e-7 relative, every gradient value to 2e-6 of the largest one of its case."""
     g = np.load(os.path.join(GOLD, "infonce_kat.npz"), allow_pickle=False)
+
+    def close(got, want):
+        np.testing.assert_allclose(got, want, rtol=0, atol=2e-6 * np.abs(want).max())
+
     for n, d, tau, seed in g["cases"]:
         n, d, seed = int(n), int(d), int(seed)
         gen = torch.Generator().manual_seed(seed)
@@ -114,9 +124,10 @@ def test_infonce_known_answers():
         loss = port.infonce(v1, v2, float(tau))
         loss.backward()
         key = "n%d_d%d_s%d" % (n, d, seed)
-        assert float(loss) == float(g[key + "_loss"][0])
+        np.testing.assert_allclose(float(loss), float(g[key + "_loss"][0]), rtol=5e-7, atol=0)
         if key + "_g1" in g:
-            assert np.array_equal(v1.grad.numpy(), g[key + "_g1"]) and np.array_equal(v2.grad.numpy(), g[key + "_g2"])
+            close(v1.grad.numpy(), g[key + "_g1"])
+            close(v2.grad.numpy(), g[key + "_g2"])
         else:
-            np.testing.assert_allclose(v1.grad.double().sum(1).numpy(), g[key + "_g1rows"], rtol=0, atol=1e-12)
-            np.testing.assert_allclose(v2.grad.double().sum(1).numpy(), g[key + "_g2rows"], rtol=0, atol=1e-12)
+            close(v1.grad.double().sum(1).numpy(), g[key + "_g1rows"])
+            close(v2.grad.double().sum(1).numpy(), g[key + "_g2rows"])
