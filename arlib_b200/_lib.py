@@ -42,6 +42,7 @@ class SpmmArgs(ctypes.Structure):
         ("d", I32),
         ("flags", I32),
         ("mask_bits", I32),
+        ("acc_terms", P * 8), ("n_acc_terms", I32),
     ]
 
 

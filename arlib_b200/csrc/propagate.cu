@@ -82,6 +82,11 @@ struct SpmmParams {
   const float* adam_coefs;
   float beta1, beta2, adam_eps;
   float4* zero_rows;          // nullable (== acc_in): rows of acc_in that were non-zero are zeroed after the read
+  // layer sum formed in the epilogue (TERMS launches only, acc_in == nullptr): acc_in's row is replaced by
+  // ((acc_terms[0] + acc_terms[1]) + ...) -- the running sum the earlier layers would have written, same adds in the
+  // same order -- so those layers write only their Y and the sum is formed only at the rows this launch computes
+  const float4* acc_terms[AGCF_MAX_ACC_TERMS];
+  int n_acc_terms;
 };
 
 __device__ __forceinline__ bool bit_set(const uint32_t* __restrict__ m, int k) {
@@ -162,7 +167,7 @@ __device__ __forceinline__ void spmm_perturb(const SpmmParams& p, size_t rbase, 
   }
 }
 
-template <typename C, bool NOISE>
+template <typename C, bool NOISE, bool TERMS = false>
 __device__ __forceinline__ void spmm_epilogue(const SpmmParams& p, int row, bool valid,
                                               float4 (&t)[C::VPL], int gl, const float4* pre_add = nullptr) {
   const size_t rbase = (size_t)row * C::V4;
@@ -208,7 +213,18 @@ __device__ __forceinline__ void spmm_epilogue(const SpmmParams& p, int row, bool
     for (int v = 0; v < C::VPL; ++v) {
       const size_t at = rbase + v * C::LPR + gl;
       float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (p.acc_in != nullptr) {
+      if constexpr (TERMS) {
+        // four rows requested together per round trip (L <= 4: one), added in table order
+        for (int q0 = 0; q0 < p.n_acc_terms; q0 += 4) {
+          float4 term[4];
+#pragma unroll
+          for (int q = 0; q < 4; ++q)
+            if (q0 + q < p.n_acc_terms) term[q] = ld_stream_f4(p.acc_terms[q0 + q] + at);
+#pragma unroll
+          for (int q = 0; q < 4; ++q)
+            if (q0 + q < p.n_acc_terms) a = q0 + q == 0 ? term[0] : add4(a, term[q]);
+        }
+      } else if (p.acc_in != nullptr) {
         // (a table this kernel also writes must not go through the non-coherent path)
         a = p.zero_rows != nullptr ? __ldcg(p.acc_in + at) : ld_stream_f4(p.acc_in + at);
         // the batch's gradient rows are the only non-zero rows of G: put them back to zero for the next step
@@ -447,7 +463,7 @@ __device__ __forceinline__ void spmm_accumulate_masked(const SpmmParams& p, int 
 // the end of a work item, shared by the two accumulation schemes below: rows cut into several segments combine
 // through the partial-sum scratch (every segment stores its partial sum, the one that arrives last -- a ticket per
 // row -- adds them in segment order: deterministic, no floating-point atomics), then the fused epilogue
-template <typename C, bool NOISE>
+template <typename C, bool NOISE, bool TERMS = false>
 __device__ __forceinline__ void spmm_finish_item(const SpmmParams& p, bool valid, int row, int k, int nseg, long long slot,
                                                  float4 (&acc)[C::VPL], int gl, const float4* pre) {
   const bool multi = valid && nseg > 1;
@@ -506,11 +522,11 @@ __device__ __forceinline__ void spmm_finish_item(const SpmmParams& p, bool valid
       }
     }
   }
-  spmm_epilogue<C, NOISE>(p, row, do_epilogue, acc, gl, pre);
+  spmm_epilogue<C, NOISE, TERMS>(p, row, do_epilogue, acc, gl, pre);
 }
 
-// one block of RPB work items (one lane group each)
-template <int D, int LPR, bool NOISE, bool CMASK>
+// one block of RPB work items (one lane group each); TERMS: the layer sum is formed in the epilogue (acc_terms)
+template <int D, int LPR, bool NOISE, bool CMASK, bool TERMS = false>
 __device__ __forceinline__ void spmm_block(const SpmmParams& p, const int n_v, const int blk) {
 #ifdef AGCF_SPMM_TRACE
   TraceScope trace_scope(blk);
@@ -550,7 +566,7 @@ __device__ __forceinline__ void spmm_block(const SpmmParams& p, const int n_v, c
     spmm_accumulate_chunks<C, true>(p, s, len, 0, C::CH, iters, gl, acc);
   }
   AGCF_TRACE_AFTER(2, __float_as_int(acc[0].x));
-  spmm_finish_item<C, NOISE>(p, valid, row, k, nseg, slot, acc, gl, (CMASK && p.addend != nullptr) ? pre : nullptr);
+  spmm_finish_item<C, NOISE, TERMS>(p, valid, row, k, nseg, slot, acc, gl, (CMASK && p.addend != nullptr) ? pre : nullptr);
 }
 
 // ------------------------------------------------------------------ narrow rows (column-sharded tables)
@@ -707,7 +723,7 @@ __global__ void __launch_bounds__(256, MINB) spmm_coop_kernel(const SpmmParams p
 // first block by CTA id and every further one from a device counter, in plan order (long items first).  The ticket for
 // the next block is taken before the current block is processed, so its latency is hidden; the last CTA to finish
 // puts both counters back to zero for the next launch.
-template <int D, int LPR, bool NOISE, bool CMASK>
+template <int D, int LPR, bool NOISE, bool CMASK, bool TERMS = false>
 __device__ __forceinline__ void spmm_grid(const SpmmParams& p) {
   using C = RowCfg<D, LPR>;
   int n_v = p.n_v;
@@ -716,7 +732,7 @@ __device__ __forceinline__ void spmm_grid(const SpmmParams& p) {
     n_v = n_dev < n_v ? n_dev : n_v;
   }
   if (p.sched == nullptr) {
-    spmm_block<D, LPR, NOISE, CMASK>(p, n_v, (int)blockIdx.x);
+    spmm_block<D, LPR, NOISE, CMASK, TERMS>(p, n_v, (int)blockIdx.x);
     return;
   }
   __shared__ int s_next[2];
@@ -726,7 +742,7 @@ __device__ __forceinline__ void spmm_grid(const SpmmParams& p) {
   for (int it = 0; blk < n_blocks; ++it) {
     int nxt = 0;
     if (threadIdx.x == 0) nxt = atomicAdd(p.sched, 1) + (int)gridDim.x;
-    spmm_block<D, LPR, NOISE, CMASK>(p, n_v, blk);
+    spmm_block<D, LPR, NOISE, CMASK, TERMS>(p, n_v, blk);
     if (threadIdx.x == 0) s_next[it & 1] = nxt;
     __syncthreads();
     blk = s_next[it & 1];
@@ -737,9 +753,9 @@ __device__ __forceinline__ void spmm_grid(const SpmmParams& p) {
   }
 }
 
-template <int D, int LPR, int MINB, bool NOISE>
+template <int D, int LPR, int MINB, bool NOISE, bool TERMS = false>
 __global__ void __launch_bounds__(256, MINB) spmm_csr_kernel(const SpmmParams p) {
-  spmm_grid<D, LPR, NOISE, false>(p);
+  spmm_grid<D, LPR, NOISE, false, TERMS>(p);
 }
 
 // first backward layer: gathers only the rows in col_mask (spmm_accumulate_masked)
@@ -775,7 +791,7 @@ static int launch_spmm(const SpmmParams& p, cudaStream_t st) {
     // the L1 wavefronts per non-zero, but a warp now walks its 16 items one after the other, and with ~1 wave of CTAs per
     // launch the launch lasts as long as that serial chain of 16 dependent index -> gather -> reduce round trips.
     static const bool coop = [] { const char* e = getenv("AGCF_SPMM_COOP"); return e != nullptr && atoi(e) != 0; }();
-    if (coop && p.sched == nullptr && (p.col_mask == nullptr || cmask)) {
+    if (coop && p.sched == nullptr && p.n_acc_terms == 0 && (p.col_mask == nullptr || cmask)) {
       const bool noise = p.noise != nullptr || p.noise_main || p.aux_Y[0] != nullptr || p.aux_Y[1] != nullptr;
       if (cmask) {
         const int words = (p.mask_bits + 31) / 32;
@@ -821,6 +837,8 @@ static int launch_spmm(const SpmmParams& p, cudaStream_t st) {
   const int threads = p.sched == nullptr ? csr_threads : C::THREADS;
   if (p.noise != nullptr || p.noise_main || p.aux_Y[0] != nullptr || p.aux_Y[1] != nullptr)
     spmm_csr_kernel<D, LPR, AGCF_SPMM_MINB(D), true><<<(unsigned)blocks, threads, 0, st>>>(p);
+  else if (p.n_acc_terms > 0)
+    spmm_csr_kernel<D, LPR, AGCF_SPMM_MINB(D), false, true><<<(unsigned)blocks, threads, 0, st>>>(p);
   else
     spmm_csr_kernel<D, LPR, AGCF_SPMM_MINB(D), false><<<(unsigned)blocks, threads, 0, st>>>(p);
   AGCF_LAUNCH_OK();
@@ -987,6 +1005,9 @@ __global__ void __launch_bounds__(1024) batch_worklist_kernel(const int32_t* __r
 
 using namespace agcf;
 
+static_assert(sizeof(((agcf_spmm_args*)nullptr)->acc_terms) == AGCF_MAX_ACC_TERMS * sizeof(const float*),
+              "acc_terms holds AGCF_MAX_ACC_TERMS tables");
+
 extern "C" int agcf_spmm_csr_f32_ex(const agcf_spmm_args* a, agcf_stream_t stream) {
   if (a == nullptr) return AGCF_EINVAL;
   if (a->n_peers < 0 || a->n_peers > AGCF_MAX_PEERS) return AGCF_EINVAL;
@@ -1042,6 +1063,18 @@ extern "C" int agcf_spmm_csr_f32_ex(const agcf_spmm_args* a, agcf_stream_t strea
   p.beta1 = a->adam_beta1; p.beta2 = a->adam_beta2; p.adam_eps = a->adam_eps;
   p.zero_rows = a->zero_acc_in ? reinterpret_cast<float4*>(const_cast<float*>(a->acc_in)) : nullptr;
   if (a->flags != 0) return AGCF_EINVAL;
+  if (a->n_acc_terms < 0 || a->n_acc_terms > AGCF_MAX_ACC_TERMS) return AGCF_EINVAL;
+  p.n_acc_terms = a->n_acc_terms;
+  for (int q = 0; q < AGCF_MAX_ACC_TERMS; ++q) {
+    p.acc_terms[q] = q < a->n_acc_terms ? reinterpret_cast<const float4*>(a->acc_terms[q]) : nullptr;
+    if (q < a->n_acc_terms && (a->acc_terms[q] == nullptr || !aligned16(a->acc_terms[q]) || a->acc_terms[q] == a->acc_out))
+      return AGCF_EINVAL;
+  }
+  if (p.n_acc_terms > 0) {
+    const bool noisy = p.noise != nullptr || p.noise_main || p.aux_Y[0] != nullptr || p.aux_Y[1] != nullptr;
+    if (a->acc_in != nullptr || a->acc_out == nullptr || a->col_mask != nullptr || a->adam_p != nullptr || noisy)
+      return AGCF_EINVAL;
+  }
   p.sched = a->sched;
   cudaStream_t st = (cudaStream_t)stream;
   switch (a->d) {

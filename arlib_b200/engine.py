@@ -144,12 +144,15 @@ class LightGCNEngine:
         self.comm = comm
         self.mode = mode if (comm is not None and comm.world > 1) else "single"
         f = lambda: torch.empty_like(table)
+        # forward layers 1 .. L-1 of a training step keep their tables E_1 .. E_{L-1} (fw[k - 1]) for the last layer,
+        # which forms the layer sum at the batch's rows (_forward_batch)
+        n_fw = max(2, self.L - 1) if self.L > 1 else 0
         if self.mode == "single":
             self.comm = None
             self.g, self.E0 = graph.planned_for(self.d), table
             self.r0, self.r1 = 0, self.N
             self.F = f()
-            self.fw = [f(), f()] if self.L > 1 else []
+            self.fw = [f() for _ in range(n_fw)]
             self.bw = [f(), f()] if self.L > 1 else []
         elif self.mode == "dshard":
             c0, c1 = dshard_columns(self.d_full, comm.world, comm.rank)
@@ -161,7 +164,7 @@ class LightGCNEngine:
             table = self.E0                      # every per-step table below has the slice's shape
             f = lambda: torch.empty_like(self.E0)
             self.F = f()
-            self.fw = [f(), f()] if self.L > 1 else []
+            self.fw = [f() for _ in range(n_fw)]
             self.bw = [f(), f()] if self.L > 1 else []
             # exchange buffer of the partial scores: one symmetric allocation, every rank writes its slot everywhere
             nbytes = ops.bpr_xchg_bytes(self.B)
@@ -372,6 +375,21 @@ class LightGCNEngine:
             x = y
         return F
 
+    def _forward_batch(self, row_mask, worklist):
+        """The training step's forward: F = mean_k A^k E0 at the batch's rows only (row_mask / worklist).  Layers
+        1 .. L-1 write only E_k; the last layer's epilogue forms ((E0 + E1) + ... + E_{L-1} + t) / (L + 1), the same
+        adds in the same order as the running sum of forward_table, so F is bit-identical on those rows.  The
+        row-partitioned layout (whose layers also go to the peers) and more than 8 layers keep forward_table."""
+        if self.mode == "rows" or self.L > 8:
+            return self.forward_table(row_mask=row_mask, worklist=worklist)
+        x = self.E0
+        for k in range(1, self.L):
+            ops.spmm(self.g, x, Y=self.fw[k - 1])
+            x = self.fw[k - 1]
+        ops.spmm(self.g, x, acc_out=self.F, acc_div=float(self.L + 1), acc_terms=[self.E0] + self.fw[:self.L - 1],
+                 row_mask=row_mask if worklist is None else None, worklist=worklist)
+        return self.F
+
     def _launch_step(self, b):
         B, L = self.B, self.L
         t0 = b * B
@@ -383,7 +401,10 @@ class LightGCNEngine:
         n_seg = self.n_seg[b:]
         out4 = self.out4[b]
         mask = self.node_mask[b * self.mask_words:] if self.sparse_layers else None
-        F = self.forward_table(row_mask=mask, worklist=self._worklist(b) if mask is not None else None)
+        if mask is not None:
+            F = self._forward_batch(mask, self._worklist(b))
+        else:
+            F = self.forward_table()
         if self.mode == "dshard":
             # the step's only exchange: 32 B per triple to every peer, stamped with the step -- bpr_finish spins on
             # the words it needs, no barrier launch (csrc/bpr.cu)

@@ -36,7 +36,7 @@ def _p(t):
 
 def spmm(g: DeviceGraph, X, Y=None, addend=None, acc_in=None, acc_out=None, acc_div=1.0, noise=None, eps=0.0,
          row_mask=None, col_mask=None, peer_Y=None, peer_acc=None, mc_Y=None, mc_acc=None,
-         worklist=None, adam=None, zero_acc_in=False, persistent=None, philox=None, aux=None):
+         worklist=None, adam=None, zero_acc_in=False, persistent=None, philox=None, aux=None, acc_terms=None):
     """agcf_spmm_csr_f32_ex: t = A X (+addend) (+noise perturbation); Y = t;
     acc_out = (acc_in + t) / acc_div.
 
@@ -46,7 +46,8 @@ def spmm(g: DeviceGraph, X, Y=None, addend=None, acc_in=None, acc_out=None, acc_
     setting): persistent CTAs with dynamic block scheduling instead of one CTA per block; philox = (seed, stream,
     step_dev or None): draw the perturbation noise in the epilogue instead of reading ``noise`` (stream None: no
     main perturbation, the seed / step only serve ``aux``); aux = up to two (Y_q, noise table or None, stream) extra
-    outputs perturbed with their own noise."""
+    outputs perturbed with their own noise; acc_terms = up to 8 tables that take the place of acc_in:
+    acc_out = (((acc_terms[0] + acc_terms[1]) + ...) + t) / acc_div."""
     lib = _lib.load()
     _f32(X, "X"); _f32(Y, "Y"); _f32(addend, "addend"); _f32(acc_in, "acc_in"); _f32(acc_out, "acc_out"); _f32(noise, "noise")
     if X.shape[0] != g.n_rows:
@@ -103,6 +104,15 @@ def spmm(g: DeviceGraph, X, Y=None, addend=None, acc_in=None, acc_out=None, acc_
     if g.persistent if persistent is None else persistent:
         a.sched = g.sched.data_ptr()
     a.flags = 0
+    if acc_terms:
+        if len(acc_terms) > len(a.acc_terms):
+            raise ValueError("at most %d acc_terms" % len(a.acc_terms))
+        for q, t in enumerate(acc_terms):
+            _f32(t, "acc_terms")
+            if tuple(t.shape) != (g.n_rows, d):
+                raise ValueError("operand shape mismatch")
+            a.acc_terms[q] = t.data_ptr()
+        a.n_acc_terms = len(acc_terms)
     _lib.check(lib.agcf_spmm_csr_f32_ex(ctypes.byref(a), _lib.stream_ptr()), "agcf_spmm_csr_f32_ex")
 
 

@@ -36,6 +36,7 @@ extern "C" {
 
 typedef void* agcf_stream_t;    /* cudaStream_t */
 #define AGCF_MAX_PEERS 8        /* GPUs of one NVSwitch box */
+#define AGCF_MAX_ACC_TERMS 8    /* tables of agcf_spmm_args.acc_terms */
 
 int         agcf_abi_version(void);
 const char* agcf_strerror(int code);
@@ -124,7 +125,11 @@ int agcf_spmm_csr_f32(const int32_t* vrows, const int32_t* vpart, int32_t n_vrow
  *                 stream-ordered;
  *   flags         reserved, must be 0;
  *   mask_bits     number of bits of row_mask / col_mask (= rows of X), or 0 if unknown: the narrow-row (d <= 16) variant
- *                 of the column-masked launch copies the bitmap into shared memory when it is given and fits.
+ *                 of the column-masked launch copies the bitmap into shared memory when it is given and fits;
+ *   acc_terms     n_acc_terms (0 .. AGCF_MAX_ACC_TERMS) [rows, d] tables that take the place of acc_in (which must then be
+ *                 null): acc_out = (((acc_terms[0] + acc_terms[1]) + ...) + t) / acc_div, plain fp32 adds in that order.
+ *                 The last propagation layer forms the layer sum this way at the rows it computes, so the earlier
+ *                 layers need only write their Y.  Not with noise, col_mask or adam.
  * A launch with col_mask (and no noise) runs the sparse variant (ballot over the live entries of a chunk, only
  * those are gathered): identical results. */
 typedef struct agcf_spmm_args {
@@ -145,6 +150,8 @@ typedef struct agcf_spmm_args {
   int32_t d;
   int32_t flags;
   int32_t mask_bits;
+  const float* acc_terms[8];
+  int32_t n_acc_terms;
 } agcf_spmm_args;
 int agcf_spmm_csr_f32_ex(const agcf_spmm_args* args, agcf_stream_t stream);
 
