@@ -43,6 +43,7 @@ class SpmmArgs(ctypes.Structure):
         ("flags", I32),
         ("mask_bits", I32),
         ("acc_terms", P * 8), ("n_acc_terms", I32),
+        ("addend_mask", P),
     ]
 
 

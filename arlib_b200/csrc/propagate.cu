@@ -81,7 +81,10 @@ struct SpmmParams {
   float4* adam_v;
   const float* adam_coefs;
   float beta1, beta2, adam_eps;
-  float4* zero_rows;          // nullable (== acc_in): rows of acc_in that were non-zero are zeroed after the read
+  float4* zero_rows;          // nullable (== acc_in): rows of acc_in that were non-zero (AMASK: in addend_mask) are zeroed
+  // nullable bitmap over rows (AMASK launches): rows of addend / acc_in outside it are exactly zero -- not loaded, +0.0f is
+  // added instead.  The backward gradient G is non-zero only at the batch's <= 3B rows (~8 % at the Gowalla shape)
+  const uint32_t* addend_mask;
   // layer sum formed in the epilogue (TERMS launches only, acc_in == nullptr): acc_in's row is replaced by
   // ((acc_terms[0] + acc_terms[1]) + ...) -- the running sum the earlier layers would have written, same adds in the
   // same order -- so those layers write only their Y and the sum is formed only at the rows this launch computes
@@ -167,14 +170,17 @@ __device__ __forceinline__ void spmm_perturb(const SpmmParams& p, size_t rbase, 
   }
 }
 
-template <typename C, bool NOISE, bool TERMS = false>
-__device__ __forceinline__ void spmm_epilogue(const SpmmParams& p, int row, bool valid,
+// live: the row's bit of addend_mask (AMASK launches; always true otherwise)
+template <typename C, bool NOISE, bool TERMS = false, bool AMASK = false>
+__device__ __forceinline__ void spmm_epilogue(const SpmmParams& p, int row, bool valid, bool live,
                                               float4 (&t)[C::VPL], int gl, const float4* pre_add = nullptr) {
   const size_t rbase = (size_t)row * C::V4;
   if (p.addend != nullptr && valid) {
+    // a row outside addend_mask adds +0.0f: -0.0f + +0.0f is +0.0f, the bits of adding the zero row
 #pragma unroll
     for (int v = 0; v < C::VPL; ++v)
-      t[v] = add4(t[v], pre_add != nullptr ? pre_add[v] : ld_stream_f4(p.addend + rbase + v * C::LPR + gl));
+      t[v] = add4(t[v], pre_add != nullptr ? pre_add[v]
+                        : (live ? ld_stream_f4(p.addend + rbase + v * C::LPR + gl) : make_float4(0.f, 0.f, 0.f, 0.f)));
   }
   if (NOISE) {
 #pragma unroll
@@ -224,11 +230,11 @@ __device__ __forceinline__ void spmm_epilogue(const SpmmParams& p, int row, bool
           for (int q = 0; q < 4; ++q)
             if (q0 + q < p.n_acc_terms) a = q0 + q == 0 ? term[0] : add4(a, term[q]);
         }
-      } else if (p.acc_in != nullptr) {
+      } else if (p.acc_in != nullptr && live) {
         // (a table this kernel also writes must not go through the non-coherent path)
         a = p.zero_rows != nullptr ? __ldcg(p.acc_in + at) : ld_stream_f4(p.acc_in + at);
         // the batch's gradient rows are the only non-zero rows of G: put them back to zero for the next step
-        if (p.zero_rows != nullptr && (a.x != 0.f || a.y != 0.f || a.z != 0.f || a.w != 0.f))
+        if (!AMASK && p.zero_rows != nullptr && (a.x != 0.f || a.y != 0.f || a.z != 0.f || a.w != 0.f))
           p.zero_rows[at] = make_float4(0.f, 0.f, 0.f, 0.f);
       }
       float4 o = add4(a, t[v]);
@@ -256,6 +262,12 @@ __device__ __forceinline__ void spmm_epilogue(const SpmmParams& p, int row, bool
         adam_update(pp.w, o.w, mm.w, vv.w, w1, w2, p.beta2, step_size, bc2_sqrt, p.adam_eps);
         p.adam_p[at] = pp; __stcs(p.adam_m + at, mm); __stcs(p.adam_v + at, vv);
       }
+      // AMASK: every row of the bitmap is put back to zero, whatever it held (a -0.0f gradient does not outlive its step
+      // either).  Last, after the optimizer's stores: with no store ahead of them, the loads of p / m / v need not wait
+      // for it, and at the ~92 % of rows that read no gradient they are the epilogue's only round trip.  Requesting them
+      // together with the gradient row instead (ahead of the acc_out store too) measured slower: 65.1 vs 60.7 us per
+      // fused launch at the Gowalla shape (profiles/r4_summary.md)
+      if (AMASK && p.zero_rows != nullptr && live) p.zero_rows[at] = make_float4(0.f, 0.f, 0.f, 0.f);
     }
   }
 }
@@ -463,9 +475,9 @@ __device__ __forceinline__ void spmm_accumulate_masked(const SpmmParams& p, int 
 // the end of a work item, shared by the two accumulation schemes below: rows cut into several segments combine
 // through the partial-sum scratch (every segment stores its partial sum, the one that arrives last -- a ticket per
 // row -- adds them in segment order: deterministic, no floating-point atomics), then the fused epilogue
-template <typename C, bool NOISE, bool TERMS = false>
-__device__ __forceinline__ void spmm_finish_item(const SpmmParams& p, bool valid, int row, int k, int nseg, long long slot,
-                                                 float4 (&acc)[C::VPL], int gl, const float4* pre) {
+template <typename C, bool NOISE, bool TERMS = false, bool AMASK = false>
+__device__ __forceinline__ void spmm_finish_item(const SpmmParams& p, bool valid, bool live, int row, int k, int nseg,
+                                                 long long slot, float4 (&acc)[C::VPL], int gl, const float4* pre) {
   const bool multi = valid && nseg > 1;
   bool do_epilogue = valid;
   if (__any_sync(0xffffffffu, multi)) {
@@ -522,11 +534,12 @@ __device__ __forceinline__ void spmm_finish_item(const SpmmParams& p, bool valid
       }
     }
   }
-  spmm_epilogue<C, NOISE, TERMS>(p, row, do_epilogue, acc, gl, pre);
+  spmm_epilogue<C, NOISE, TERMS, AMASK>(p, row, do_epilogue, live, acc, gl, pre);
 }
 
-// one block of RPB work items (one lane group each); TERMS: the layer sum is formed in the epilogue (acc_terms)
-template <int D, int LPR, bool NOISE, bool CMASK, bool TERMS = false>
+// one block of RPB work items (one lane group each); TERMS: the layer sum is formed in the epilogue (acc_terms);
+// AMASK: addend / acc_in are read only at the rows of addend_mask
+template <int D, int LPR, bool NOISE, bool CMASK, bool TERMS = false, bool AMASK = false>
 __device__ __forceinline__ void spmm_block(const SpmmParams& p, const int n_v, const int blk) {
 #ifdef AGCF_SPMM_TRACE
   TraceScope trace_scope(blk);
@@ -546,6 +559,8 @@ __device__ __forceinline__ void spmm_block(const SpmmParams& p, const int n_v, c
   const int s = vr.x, row = vr.z, k = vr.w & 0xffff, nseg = vr.w >> 16;
   int len = vr.y;
   if (valid && p.row_mask != nullptr && !bit_set(p.row_mask, row)) { valid = false; len = 0; }
+  // the addend row's bit: requested with the item's first indices, needed only by the epilogue
+  const bool live = !AMASK || (valid && bit_set(p.addend_mask, row));
   int maxlen = len;
 #pragma unroll
   for (int o = C::LPR; o < 32; o <<= 1) {
@@ -556,7 +571,7 @@ __device__ __forceinline__ void spmm_block(const SpmmParams& p, const int n_v, c
   float4 pre[C::VPL];                                      // CMASK: the epilogue's addend row, fetched before the gathers
   if constexpr (CMASK) {
     const int iters = (maxlen + C::CH - 1) / C::CH;        // warp-uniform
-    const bool has_add = p.addend != nullptr && valid;
+    const bool has_add = p.addend != nullptr && valid && live;
 #pragma unroll
     for (int v = 0; v < C::VPL; ++v)
       pre[v] = has_add ? ld_stream_f4(p.addend + (size_t)row * C::V4 + v * C::LPR + gl) : make_float4(0.f, 0.f, 0.f, 0.f);
@@ -566,7 +581,8 @@ __device__ __forceinline__ void spmm_block(const SpmmParams& p, const int n_v, c
     spmm_accumulate_chunks<C, true>(p, s, len, 0, C::CH, iters, gl, acc);
   }
   AGCF_TRACE_AFTER(2, __float_as_int(acc[0].x));
-  spmm_finish_item<C, NOISE, TERMS>(p, valid, row, k, nseg, slot, acc, gl, (CMASK && p.addend != nullptr) ? pre : nullptr);
+  spmm_finish_item<C, NOISE, TERMS, AMASK>(p, valid, live, row, k, nseg, slot, acc, gl,
+                                          (CMASK && p.addend != nullptr) ? pre : nullptr);
 }
 
 // ------------------------------------------------------------------ narrow rows (column-sharded tables)
@@ -691,7 +707,7 @@ __device__ __forceinline__ void spmm_block_coop(const SpmmParams& p, const int n
     s_i = s_n; len_i = len_n; c0 = nc0; c1 = nc1; v0 = nv0; v1 = nv1;
   }
   float4 accv[1] = {res};
-  spmm_finish_item<C, NOISE>(p, valid, row, k, nseg, slot, accv, gl, (CMASK && p.addend != nullptr) ? pre : nullptr);
+  spmm_finish_item<C, NOISE>(p, valid, true, row, k, nseg, slot, accv, gl, (CMASK && p.addend != nullptr) ? pre : nullptr);
 }
 
 // the column bitmap of the first backward layer lives in shared memory while it fits (N <= 32 * kCoopMaskWords nodes)
@@ -723,7 +739,7 @@ __global__ void __launch_bounds__(256, MINB) spmm_coop_kernel(const SpmmParams p
 // first block by CTA id and every further one from a device counter, in plan order (long items first).  The ticket for
 // the next block is taken before the current block is processed, so its latency is hidden; the last CTA to finish
 // puts both counters back to zero for the next launch.
-template <int D, int LPR, bool NOISE, bool CMASK, bool TERMS = false>
+template <int D, int LPR, bool NOISE, bool CMASK, bool TERMS = false, bool AMASK = false>
 __device__ __forceinline__ void spmm_grid(const SpmmParams& p) {
   using C = RowCfg<D, LPR>;
   int n_v = p.n_v;
@@ -732,7 +748,7 @@ __device__ __forceinline__ void spmm_grid(const SpmmParams& p) {
     n_v = n_dev < n_v ? n_dev : n_v;
   }
   if (p.sched == nullptr) {
-    spmm_block<D, LPR, NOISE, CMASK, TERMS>(p, n_v, (int)blockIdx.x);
+    spmm_block<D, LPR, NOISE, CMASK, TERMS, AMASK>(p, n_v, (int)blockIdx.x);
     return;
   }
   __shared__ int s_next[2];
@@ -742,7 +758,7 @@ __device__ __forceinline__ void spmm_grid(const SpmmParams& p) {
   for (int it = 0; blk < n_blocks; ++it) {
     int nxt = 0;
     if (threadIdx.x == 0) nxt = atomicAdd(p.sched, 1) + (int)gridDim.x;
-    spmm_block<D, LPR, NOISE, CMASK, TERMS>(p, n_v, blk);
+    spmm_block<D, LPR, NOISE, CMASK, TERMS, AMASK>(p, n_v, blk);
     if (threadIdx.x == 0) s_next[it & 1] = nxt;
     __syncthreads();
     blk = s_next[it & 1];
@@ -753,18 +769,18 @@ __device__ __forceinline__ void spmm_grid(const SpmmParams& p) {
   }
 }
 
-template <int D, int LPR, int MINB, bool NOISE, bool TERMS = false>
+template <int D, int LPR, int MINB, bool NOISE, bool TERMS = false, bool AMASK = false>
 __global__ void __launch_bounds__(256, MINB) spmm_csr_kernel(const SpmmParams p) {
-  spmm_grid<D, LPR, NOISE, false, TERMS>(p);
+  spmm_grid<D, LPR, NOISE, false, TERMS, AMASK>(p);
 }
 
 // first backward layer: gathers only the rows in col_mask (spmm_accumulate_masked)
 #ifndef AGCF_SPMM_CM_THREADS
 #define AGCF_SPMM_CM_THREADS 128                   // 4-warp CTAs like the plain launches (d = 16: 19.6 -> 18.5 us, d = 128: 77.5 -> 74.3)
 #endif
-template <int D, int LPR, int MINB>
+template <int D, int LPR, int MINB, bool AMASK>
 __global__ void __launch_bounds__(AGCF_SPMM_CM_THREADS, MINB) spmm_colmask_kernel(const SpmmParams p) {
-  spmm_grid<D, LPR, false, true>(p);
+  spmm_grid<D, LPR, false, true, false, AMASK>(p);
 }
 
 // resident CTAs per SM the register allocation is held to: 4 (<= 64 registers) measured best at d <= 64
@@ -791,7 +807,7 @@ static int launch_spmm(const SpmmParams& p, cudaStream_t st) {
     // the L1 wavefronts per non-zero, but a warp now walks its 16 items one after the other, and with ~1 wave of CTAs per
     // launch the launch lasts as long as that serial chain of 16 dependent index -> gather -> reduce round trips.
     static const bool coop = [] { const char* e = getenv("AGCF_SPMM_COOP"); return e != nullptr && atoi(e) != 0; }();
-    if (coop && p.sched == nullptr && p.n_acc_terms == 0 && (p.col_mask == nullptr || cmask)) {
+    if (coop && p.sched == nullptr && p.n_acc_terms == 0 && p.addend_mask == nullptr && (p.col_mask == nullptr || cmask)) {
       const bool noise = p.noise != nullptr || p.noise_main || p.aux_Y[0] != nullptr || p.aux_Y[1] != nullptr;
       if (cmask) {
         const int words = (p.mask_bits + 31) / 32;
@@ -817,7 +833,10 @@ static int launch_spmm(const SpmmParams& p, cudaStream_t st) {
     const long long rpb = (AGCF_SPMM_CM_THREADS / 32) * C::RPW;
     long long cb = ((long long)p.n_v + rpb - 1) / rpb;
     if (p.sched != nullptr) cb = cb < blocks ? cb : blocks;
-    spmm_colmask_kernel<D, LPR, AGCF_SPMM_CM_MINB(D)><<<(unsigned)cb, AGCF_SPMM_CM_THREADS, 0, st>>>(p);
+    if (p.addend_mask != nullptr)
+      spmm_colmask_kernel<D, LPR, AGCF_SPMM_CM_MINB(D), true><<<(unsigned)cb, AGCF_SPMM_CM_THREADS, 0, st>>>(p);
+    else
+      spmm_colmask_kernel<D, LPR, AGCF_SPMM_CM_MINB(D), false><<<(unsigned)cb, AGCF_SPMM_CM_THREADS, 0, st>>>(p);
     AGCF_LAUNCH_OK();
     return AGCF_OK;
   }
@@ -839,6 +858,8 @@ static int launch_spmm(const SpmmParams& p, cudaStream_t st) {
     spmm_csr_kernel<D, LPR, AGCF_SPMM_MINB(D), true><<<(unsigned)blocks, threads, 0, st>>>(p);
   else if (p.n_acc_terms > 0)
     spmm_csr_kernel<D, LPR, AGCF_SPMM_MINB(D), false, true><<<(unsigned)blocks, threads, 0, st>>>(p);
+  else if (p.addend_mask != nullptr)
+    spmm_csr_kernel<D, LPR, AGCF_SPMM_MINB(D), false, false, true><<<(unsigned)blocks, threads, 0, st>>>(p);
   else
     spmm_csr_kernel<D, LPR, AGCF_SPMM_MINB(D), false><<<(unsigned)blocks, threads, 0, st>>>(p);
   AGCF_LAUNCH_OK();
@@ -1062,6 +1083,7 @@ extern "C" int agcf_spmm_csr_f32_ex(const agcf_spmm_args* a, agcf_stream_t strea
   p.adam_coefs = a->adam_coefs;
   p.beta1 = a->adam_beta1; p.beta2 = a->adam_beta2; p.adam_eps = a->adam_eps;
   p.zero_rows = a->zero_acc_in ? reinterpret_cast<float4*>(const_cast<float*>(a->acc_in)) : nullptr;
+  p.addend_mask = a->addend_mask;
   if (a->flags != 0) return AGCF_EINVAL;
   if (a->n_acc_terms < 0 || a->n_acc_terms > AGCF_MAX_ACC_TERMS) return AGCF_EINVAL;
   p.n_acc_terms = a->n_acc_terms;
@@ -1072,9 +1094,12 @@ extern "C" int agcf_spmm_csr_f32_ex(const agcf_spmm_args* a, agcf_stream_t strea
   }
   if (p.n_acc_terms > 0) {
     const bool noisy = p.noise != nullptr || p.noise_main || p.aux_Y[0] != nullptr || p.aux_Y[1] != nullptr;
-    if (a->acc_in != nullptr || a->acc_out == nullptr || a->col_mask != nullptr || a->adam_p != nullptr || noisy)
+    if (a->acc_in != nullptr || a->acc_out == nullptr || a->col_mask != nullptr || a->adam_p != nullptr || noisy ||
+        a->addend_mask != nullptr)
       return AGCF_EINVAL;
   }
+  if (a->addend_mask != nullptr && (p.noise != nullptr || p.noise_main || p.aux_Y[0] != nullptr || p.aux_Y[1] != nullptr))
+    return AGCF_EINVAL;
   p.sched = a->sched;
   cudaStream_t st = (cudaStream_t)stream;
   switch (a->d) {

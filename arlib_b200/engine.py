@@ -145,7 +145,8 @@ class LightGCNEngine:
         self.mode = mode if (comm is not None and comm.world > 1) else "single"
         f = lambda: torch.empty_like(table)
         # forward layers 1 .. L-1 of a training step keep their tables E_1 .. E_{L-1} (fw[k - 1]) for the last layer,
-        # which forms the layer sum at the batch's rows (_forward_batch)
+        # which forms the layer sum at the batch's rows (_forward_batch).  Once it has, they are dead: the backward layers
+        # run in them (bw), so that the step's full tables -- E0, two layer tables, m, v -- and the graph fit in L2
         n_fw = max(2, self.L - 1) if self.L > 1 else 0
         if self.mode == "single":
             self.comm = None
@@ -153,7 +154,7 @@ class LightGCNEngine:
             self.r0, self.r1 = 0, self.N
             self.F = f()
             self.fw = [f() for _ in range(n_fw)]
-            self.bw = [f(), f()] if self.L > 1 else []
+            self.bw = [self.fw[1], self.fw[0]] if self.L > 1 else []
         elif self.mode == "dshard":
             c0, c1 = dshard_columns(self.d_full, comm.world, comm.rank)
             self.d = c1 - c0
@@ -165,7 +166,7 @@ class LightGCNEngine:
             f = lambda: torch.empty_like(self.E0)
             self.F = f()
             self.fw = [f() for _ in range(n_fw)]
-            self.bw = [f(), f()] if self.L > 1 else []
+            self.bw = [self.fw[1], self.fw[0]] if self.L > 1 else []
             # exchange buffer of the partial scores: one symmetric allocation, every rank writes its slot everywhere
             nbytes = ops.bpr_xchg_bytes(self.B)
             bufs = comm.allocate({"xchg": ((nbytes,), torch.uint8)})
@@ -414,6 +415,12 @@ class LightGCNEngine:
             ops.bpr_forward(F, u, i, j, nb, self.U, self.reg, out4, self.coef, self.ws)
         ops.bpr_backward(F, u, i, j, nb, self.U, self.reg, 1.0, out4, self.coef, occ, seg_off, seg_node, n_seg, self.G)
         H = self.G
+        # G is non-zero only at the batch's rows: the backward layers read it (addend / acc_in) only there, and the fused
+        # optimizer puts exactly those rows back to zero.  That pays where the batch covers few rows (Gowalla, 8 %: the
+        # middle layer 43.2 -> 42.2 us); where it covers many, the bitmap load per work item costs more than the loads it
+        # saves (ml-1m, 42 %: 37.1 -> 39.0 us), so graphs with fewer than 4 x 3B rows read G everywhere.  The
+        # row-partitioned layout keeps the full reads too.
+        g_mask = mask if self.mode != "rows" and 12 * self.B <= self.N else None
         # first backward layer: only the batch's gradient rows of H are non-zero.  The column-masked kernel skips the others
         # (27 vs 44 us at d = 64); on 8-column slices its extra bitmap round trip per chunk costs more than the zero rows it
         # avoids (26.4 vs 23.4 us, profiles/r2_summary.md section 5), so there the plain kernel gathers the zeros
@@ -422,7 +429,7 @@ class LightGCNEngine:
         for k in range(L, 0, -1):
             if k > 1:
                 nxt = self.bw[k % 2]
-                ops.spmm(self.g, H, Y=nxt, addend=self.G, col_mask=mask if k == L else None,
+                ops.spmm(self.g, H, Y=nxt, addend=self.G, col_mask=mask if k == L else None, addend_mask=g_mask,
                          peer_Y=self._peers("bw%d" % (k % 2)), mc_Y=self._mcast("bw%d" % (k % 2)))
                 self._barrier()
                 H = nxt
@@ -432,7 +439,7 @@ class LightGCNEngine:
                 self._join_coefs()                  # this step's Adam coefficients (side branch of the previous step)
                 ops.spmm(self.g, H, acc_in=self.G, acc_div=float(L + 1), col_mask=mask if k == L else None,
                          adam=(self.E0, self.m, self.v, self.adam_coefs, self.betas[0], self.betas[1], self.adam_eps),
-                         zero_acc_in=L > 1)
+                         zero_acc_in=L > 1, addend_mask=g_mask)
             else:
                 ops.spmm(self.g, H, acc_in=self.G, acc_out=self.dE0, acc_div=float(L + 1),
                          col_mask=mask if k == L else None)

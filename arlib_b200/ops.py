@@ -36,7 +36,8 @@ def _p(t):
 
 def spmm(g: DeviceGraph, X, Y=None, addend=None, acc_in=None, acc_out=None, acc_div=1.0, noise=None, eps=0.0,
          row_mask=None, col_mask=None, peer_Y=None, peer_acc=None, mc_Y=None, mc_acc=None,
-         worklist=None, adam=None, zero_acc_in=False, persistent=None, philox=None, aux=None, acc_terms=None):
+         worklist=None, adam=None, zero_acc_in=False, persistent=None, philox=None, aux=None, acc_terms=None,
+         addend_mask=None):
     """agcf_spmm_csr_f32_ex: t = A X (+addend) (+noise perturbation); Y = t;
     acc_out = (acc_in + t) / acc_div.
 
@@ -47,7 +48,8 @@ def spmm(g: DeviceGraph, X, Y=None, addend=None, acc_in=None, acc_out=None, acc_
     step_dev or None): draw the perturbation noise in the epilogue instead of reading ``noise`` (stream None: no
     main perturbation, the seed / step only serve ``aux``); aux = up to two (Y_q, noise table or None, stream) extra
     outputs perturbed with their own noise; acc_terms = up to 8 tables that take the place of acc_in:
-    acc_out = (((acc_terms[0] + acc_terms[1]) + ...) + t) / acc_div."""
+    acc_out = (((acc_terms[0] + acc_terms[1]) + ...) + t) / acc_div; addend_mask = a row bitmap outside which addend /
+    acc_in are known to be zero (not loaded; with zero_acc_in the rows inside it are re-zeroed)."""
     lib = _lib.load()
     _f32(X, "X"); _f32(Y, "Y"); _f32(addend, "addend"); _f32(acc_in, "acc_in"); _f32(acc_out, "acc_out"); _f32(noise, "noise")
     if X.shape[0] != g.n_rows:
@@ -85,7 +87,7 @@ def spmm(g: DeviceGraph, X, Y=None, addend=None, acc_in=None, acc_out=None, acc_
         if tuple(y_q.shape) != (g.n_rows, d) or (tab_q is not None and tuple(tab_q.shape) != (g.n_rows, d)):
             raise ValueError("aux operand shape mismatch")
         a.aux_Y[q], a.aux_noise[q], a.aux_stream[q] = y_q.data_ptr(), _p(tab_q), int(stream_q or 0)
-    a.row_mask, a.col_mask = _p(row_mask), _p(col_mask)
+    a.row_mask, a.col_mask, a.addend_mask = _p(row_mask), _p(col_mask), _p(addend_mask)
     a.mask_bits = g.n_rows
     a.peer_Y_host = ctypes.cast(py, ctypes.c_void_p) if py is not None else None
     a.peer_acc_host = ctypes.cast(pa, ctypes.c_void_p) if pa is not None else None

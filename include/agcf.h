@@ -130,6 +130,11 @@ int agcf_spmm_csr_f32(const int32_t* vrows, const int32_t* vpart, int32_t n_vrow
  *                 null): acc_out = (((acc_terms[0] + acc_terms[1]) + ...) + t) / acc_div, plain fp32 adds in that order.
  *                 The last propagation layer forms the layer sum this way at the rows it computes, so the earlier
  *                 layers need only write their Y.  Not with noise, col_mask or adam.
+ *   addend_mask   nullable bitmap over rows (like row_mask): rows of addend / acc_in whose bit is clear are known to be
+ *                 exactly zero and are not loaded; +0.0f is added in their place.  With zero_acc_in, every row whose bit
+ *                 is set is set to +0.0f (instead of the rows that read non-zero).  The backward layers of the training
+ *                 step pass the batch's node bitmap: the gradient G is non-zero only at the batch's rows.  Not with
+ *                 acc_terms or noise.
  * A launch with col_mask (and no noise) runs the sparse variant (ballot over the live entries of a chunk, only
  * those are gathered): identical results. */
 typedef struct agcf_spmm_args {
@@ -152,6 +157,7 @@ typedef struct agcf_spmm_args {
   int32_t mask_bits;
   const float* acc_terms[8];
   int32_t n_acc_terms;
+  const uint32_t* addend_mask;
 } agcf_spmm_args;
 int agcf_spmm_csr_f32_ex(const agcf_spmm_args* args, agcf_stream_t stream);
 
