@@ -662,7 +662,7 @@ extern "C" int agcf_bpr_forward(const float* F, const int32_t* u, const int32_t*
                                 int32_t nb, int32_t n_users, int32_t d, float reg,
                                 float* out4, float* coef, void* ws, agcf_stream_t stream) {
   if (!F || !u || !i || !j || !out4 || !coef || !ws || nb <= 0 || n_users < 0) return AGCF_EINVAL;
-  if (!supported_row_d(d)) return AGCF_EUNSUPPORTED;
+  if (!supported_d(d)) return AGCF_EUNSUPPORTED;
   if (!aligned16(F) || !aligned16(ws)) return AGCF_EINVAL;
   cudaStream_t st = (cudaStream_t)stream;
   const float4* F4 = reinterpret_cast<const float4*>(F);
@@ -696,7 +696,7 @@ extern "C" int agcf_bpr_partial(const float* F, const int32_t* u, const int32_t*
                                 agcf_stream_t stream) {
   if (!F || !u || !i || !j || nb <= 0 || n_users < 0 || !xchg_all_host) return AGCF_EINVAL;
   if (world < 1 || world > AGCF_MAX_PEERS || rank < 0 || rank >= world || nb > cap) return AGCF_EINVAL;
-  if (!supported_row_d(d)) return AGCF_EUNSUPPORTED;
+  if (!supported_d(d)) return AGCF_EUNSUPPORTED;
   if (!aligned16(F)) return AGCF_EINVAL;
   XchgPeers x;
   x.n = world;
@@ -741,7 +741,7 @@ extern "C" int agcf_bpr_backward(const float* F, const int32_t* u, const int32_t
                                  const int32_t* occ, const int32_t* seg_off, const int32_t* seg_node,
                                  const int32_t* n_seg, float* G, agcf_stream_t stream) {
   if (!F || !u || !i || !j || !out4 || !coef || !occ || !seg_off || !seg_node || !n_seg || !G || nb <= 0) return AGCF_EINVAL;
-  if (!supported_row_d(d)) return AGCF_EUNSUPPORTED;
+  if (!supported_d(d)) return AGCF_EUNSUPPORTED;
   if (!aligned16(F) || !aligned16(G) || F == G) return AGCF_EINVAL;
   cudaStream_t st = (cudaStream_t)stream;
   const float4* F4 = reinterpret_cast<const float4*>(F);
@@ -768,7 +768,7 @@ extern "C" int agcf_bpr_backward(const float* F, const int32_t* u, const int32_t
 extern "C" int agcf_zero_rows(const int32_t* seg_node, const int32_t* n_seg, int32_t max_seg,
                               float* G, int32_t d, agcf_stream_t stream) {
   if (!seg_node || !n_seg || !G || max_seg < 0) return AGCF_EINVAL;
-  if (!supported_row_d(d)) return AGCF_EUNSUPPORTED;
+  if (!supported_d(d)) return AGCF_EUNSUPPORTED;
   if (!aligned16(G)) return AGCF_EINVAL;
   if (max_seg == 0) return AGCF_OK;
   cudaStream_t st = (cudaStream_t)stream;

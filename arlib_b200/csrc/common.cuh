@@ -30,9 +30,8 @@ inline int cuda_fail(cudaError_t e, const char* file = "", int line = 0) {
   } while (0)
 
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
-inline bool supported_d(int d) { return d == 32 || d == 64 || d == 128 || d == 256; }
-// row kernels (propagation, loss, optimizer) also take the narrow column slices of the d-sharded multi-GPU tables
-inline bool supported_row_d(int d) { return d == 8 || d == 16 || supported_d(d); }
+// embedding widths every kernel family is compiled for (the NGCF dense layer and the tcgen05 scoring stage take subsets)
+inline bool supported_d(int d) { return d == 8 || d == 16 || d == 32 || d == 64 || d == 128 || d == 256; }
 
 constexpr int kSMs = 148;  // B200
 

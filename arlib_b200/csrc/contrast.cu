@@ -23,7 +23,12 @@ template <int D>
 struct NceCfg {
   static constexpr int TM = D <= 64 ? 64 : 32;      // vectors per tile (own side and reduced side)
   static constexpr int RS = TM / 16;                // tile rows / cols per thread in the logit product
-  static constexpr int KS = D / 16;                 // embedding columns per thread in the second product
+  // second product P.V: thread (ty, tx) owns KS consecutive columns, KS (tx % CT) ..., and PA of the RS own rows,
+  // ty + 16 (PA (tx / CT) + a).  D >= 16: CT = 16 threads cover the D columns, every thread takes all RS rows;
+  // D = 8: the 8 columns need only 8 threads, so the two halves of tx split the rows instead
+  static constexpr int KS = D >= 16 ? D / 16 : 1;   // embedding columns per thread
+  static constexpr int CT = D / KS;                 // threads across the columns (16, or 8 at D = 8)
+  static constexpr int PA = RS * CT / 16;           // own rows per thread
   static constexpr int LD = D + 4;                  // padded row stride (floats): 16-byte aligned rows whose float4
   static constexpr int PLD = TM + 4;                // reads by 16 different rows need the minimal 2 wavefronts
   static constexpr size_t smem_fwd = (size_t)(2 * TM * LD) * sizeof(float);
@@ -199,9 +204,10 @@ __global__ void __launch_bounds__(kNceThreads) nce_bwd_kernel(const float* __res
   const int n_tiles = (n + C::TM - 1) / C::TM;
   nce_load_tile<D>(own, h_own, row0, n);
   if (threadIdx.x < C::TM) ttl_own[threadIdx.x] = (row0 + (int)threadIdx.x < n) ? ttl[row0 + threadIdx.x] : 1.f;
-  float acc[C::RS][C::KS];
+  const int cx = tx % C::CT, a0 = C::PA * (tx / C::CT);  // columns KS cx .. KS cx + KS - 1, own rows ty + 16 (a0 + a)
+  float acc[C::PA][C::KS];
 #pragma unroll
-  for (int a = 0; a < C::RS; ++a)
+  for (int a = 0; a < C::PA; ++a)
 #pragma unroll
     for (int b = 0; b < C::KS; ++b) acc[a][b] = 0.f;
   for (int ct = sp; ct < n_tiles; ct += split) {
@@ -220,28 +226,30 @@ __global__ void __launch_bounds__(kNceThreads) nce_bwd_kernel(const float* __res
         Ps[o * C::PLD + x] = (ct * C::TM + x < n) ? __fdiv_rn(expf(s[a][b] * inv_t), den) : 0.f;
       }
     __syncthreads();
-    // acc[o][k] += sum_x P[o][x] * other[x][k];  thread (ty, tx) owns o = ty + 16a and the KS consecutive columns
-    // k = KS tx + b; P is read 4 x at a time, the operand row KS floats at a time (x ascending in every accumulator)
+    // acc[o][k] += sum_x P[o][x] * other[x][k];  thread (ty, tx) owns o = ty + 16 (a0 + a) and the KS consecutive
+    // columns k = KS cx + b; P is read 4 x at a time, the operand row KS floats at a time (x ascending in every accumulator)
     for (int x4 = 0; x4 < C::TM; x4 += 4) {
-      float4 pv[C::RS];
+      float4 pv[C::PA];
 #pragma unroll
-      for (int a = 0; a < C::RS; ++a) pv[a] = *reinterpret_cast<const float4*>(Ps + (ty + 16 * a) * C::PLD + x4);
+      for (int a = 0; a < C::PA; ++a) pv[a] = *reinterpret_cast<const float4*>(Ps + (ty + 16 * (a0 + a)) * C::PLD + x4);
 #pragma unroll
       for (int xx = 0; xx < 4; ++xx) {
         float ov[C::KS];
-        const float* orow = other + (x4 + xx) * C::LD + C::KS * tx;
+        const float* orow = other + (x4 + xx) * C::LD + C::KS * cx;
         if constexpr (C::KS % 4 == 0) {
 #pragma unroll
           for (int q = 0; q < C::KS / 4; ++q) {
             const float4 t4 = *reinterpret_cast<const float4*>(orow + 4 * q);
             ov[4 * q] = t4.x; ov[4 * q + 1] = t4.y; ov[4 * q + 2] = t4.z; ov[4 * q + 3] = t4.w;
           }
-        } else {
+        } else if constexpr (C::KS == 2) {
           const float2 t2 = *reinterpret_cast<const float2*>(orow);
           ov[0] = t2.x; ov[1] = t2.y;
+        } else {
+          ov[0] = orow[0];
         }
 #pragma unroll
-        for (int a = 0; a < C::RS; ++a) {
+        for (int a = 0; a < C::PA; ++a) {
           const float pa = xx == 0 ? pv[a].x : (xx == 1 ? pv[a].y : (xx == 2 ? pv[a].z : pv[a].w));
 #pragma unroll
           for (int b = 0; b < C::KS; ++b) acc[a][b] = fmaf(pa, ov[b], acc[a][b]);
@@ -250,10 +258,10 @@ __global__ void __launch_bounds__(kNceThreads) nce_bwd_kernel(const float* __res
     }
   }
 #pragma unroll
-  for (int a = 0; a < C::RS; ++a) {
-    const int r = row0 + ty + 16 * a;
+  for (int a = 0; a < C::PA; ++a) {
+    const int r = row0 + ty + 16 * (a0 + a);
     if (r >= n) continue;
-    float* dst = partial_acc + ((size_t)sp * n_max + r) * D + C::KS * tx;
+    float* dst = partial_acc + ((size_t)sp * n_max + r) * D + C::KS * cx;
 #pragma unroll
     for (int b = 0; b < C::KS; ++b) dst[b] = acc[a][b];
   }
@@ -413,6 +421,8 @@ extern "C" int agcf_infonce_forward(const float* view1, const float* view2, cons
   const float inv_t = 1.f / temperature;
   cudaStream_t st = (cudaStream_t)stream;
   switch (d) {
+    case 8: return nce_forward_d<8>(view1, view2, rows, n, n_dev, inv_t, loss, w, st);
+    case 16: return nce_forward_d<16>(view1, view2, rows, n, n_dev, inv_t, loss, w, st);
     case 32: return nce_forward_d<32>(view1, view2, rows, n, n_dev, inv_t, loss, w, st);
     case 64: return nce_forward_d<64>(view1, view2, rows, n, n_dev, inv_t, loss, w, st);
     case 128: return nce_forward_d<128>(view1, view2, rows, n, n_dev, inv_t, loss, w, st);
@@ -434,6 +444,8 @@ extern "C" int agcf_infonce_backward(int32_t n, const int32_t* n_dev, int32_t d,
   const NceGrad g1 = {grad_view1, rows1, accumulate1}, g2 = {grad_view2, rows2, accumulate2};
   cudaStream_t st = (cudaStream_t)stream;
   switch (d) {
+    case 8: return nce_backward_d<8>(n, n_dev, inv_t, grad_loss, scale, w, g1, g2, st);
+    case 16: return nce_backward_d<16>(n, n_dev, inv_t, grad_loss, scale, w, g1, g2, st);
     case 32: return nce_backward_d<32>(n, n_dev, inv_t, grad_loss, scale, w, g1, g2, st);
     case 64: return nce_backward_d<64>(n, n_dev, inv_t, grad_loss, scale, w, g1, g2, st);
     case 128: return nce_backward_d<128>(n, n_dev, inv_t, grad_loss, scale, w, g1, g2, st);

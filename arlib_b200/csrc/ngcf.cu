@@ -14,6 +14,7 @@
 //   agcf_ngcf_dense_forward    E' (and the running layer mean)               from P, E, W = [W1 ; W2]
 //   agcf_ngcf_dense_backward   dP, dE_direct and per-CTA partials of dW       from dE', E' (sign of Z), P, E, W^T
 //   agcf_ngcf_reduce_wgrad     dW = sum of the partials in CTA order (deterministic)
+// d in {8, 16, 32, 64}: a 64-row tile on a 16 x 16 thread grid at 32 and 64, a row per thread at 8 and 16.
 //
 // Backward:  dZ = dE' * (E' > 0 ? 1 : 0.01)      (leaky_relu keeps the sign, so E' tells which branch Z took)
 //            [dA | dB] = dZ [W1 ; W2]^T ;  dP = dA + dB * E ;  dE_direct = dA + dB * P ;  dW = [P + E | P * E]^T dZ
@@ -234,6 +235,126 @@ __global__ void __launch_bounds__(256, 2) dense_bwd_kernel(const float* __restri
     for (int c = 0; c < CW; ++c) out[(size_t)(jy * JW + q) * D + cx * CW + c] = wacc[q][c];
 }
 
+// ------------------------------------------------------------------- d = 8 and 16
+// The 16 x 16 thread grid above gives each thread D / 16 output columns: none at D = 8, and the k chunk of 64 is wider
+// than 2D.  At these widths a row is 2D inputs and D outputs, so a thread owns a whole row: it reads its row of P and E
+// (two or four float4 each), keeps [P + E | P * E] and the D accumulators in registers, and walks W (512 or 2 048 B, in
+// shared memory, the same word for every lane: a broadcast).  Every output is the same chain as the tiled kernels'
+// (fmaf, k ascending from 0).  The weight gradient is reduced per CTA through shared memory in row order, then across
+// CTAs by reduce_wgrad_kernel in CTA order: deterministic.
+constexpr int kSmallTM = 128;    // rows per CTA (one per thread)
+
+template <int D>
+__device__ __forceinline__ void load_row(const float* __restrict__ src, size_t row, float (&x)[D]) {
+#pragma unroll
+  for (int q = 0; q < D / 4; ++q) {
+    const float4 v = __ldg(reinterpret_cast<const float4*>(src + row * D) + q);
+    x[4 * q] = v.x; x[4 * q + 1] = v.y; x[4 * q + 2] = v.z; x[4 * q + 3] = v.w;
+  }
+}
+
+template <int D>
+__global__ void __launch_bounds__(kSmallTM) dense_fwd_small_kernel(const float* __restrict__ P, const float* __restrict__ E,
+                                                                   const float* __restrict__ W, float* __restrict__ Enext,
+                                                                   const float* __restrict__ acc_in, float* __restrict__ acc_out,
+                                                                   float acc_div, int N) {
+  __shared__ __align__(16) float Ws[2 * D * D];
+  for (int f = threadIdx.x; f < 2 * D * D; f += kSmallTM) Ws[f] = __ldg(W + f);
+  __syncthreads();
+  const int row = blockIdx.x * kSmallTM + threadIdx.x;
+  if (row >= N) return;
+  float p[D], e[D], acc[D];
+  load_row<D>(P, (size_t)row, p);
+  load_row<D>(E, (size_t)row, e);
+#pragma unroll
+  for (int c = 0; c < D; ++c) acc[c] = 0.f;
+#pragma unroll
+  for (int k = 0; k < 2 * D; ++k) {
+    const float a = k < D ? p[k] + e[k] : p[k - D] * e[k - D];
+#pragma unroll
+    for (int c = 0; c < D; ++c) acc[c] = fmaf(a, Ws[k * D + c], acc[c]);
+  }
+  const size_t at = (size_t)row * D;
+#pragma unroll
+  for (int c = 0; c < D; ++c) {
+    const float z = acc[c];
+    const float o = z > 0.f ? z : kSlope * z;                        // F.leaky_relu(z, 0.01)
+    Enext[at + c] = o;
+    if (acc_out != nullptr) {
+      float m = (acc_in != nullptr ? acc_in[at + c] : 0.f) + o;
+      if (acc_div != 1.0f) m = __fdiv_rn(m, acc_div);
+      acc_out[at + c] = m;
+    }
+  }
+}
+
+template <int D>
+__global__ void __launch_bounds__(kSmallTM) dense_bwd_small_kernel(const float* __restrict__ dOut, const float* __restrict__ Enext,
+                                                                   const float* __restrict__ P, const float* __restrict__ E,
+                                                                   const float* __restrict__ WT, float* __restrict__ dP,
+                                                                   float* __restrict__ dEdir, float* __restrict__ dWpart, int N) {
+  constexpr int NW = 2 * D * D, WPT = NW / kSmallTM;                // dW entries, and per thread in the reduction (1 or 4)
+  __shared__ __align__(16) float WTs[NW];                            // W^T: [D][2D]
+  __shared__ float As[kSmallTM][2 * D + 1];                          // [P + E | P * E] of the tile's rows (+1: odd stride)
+  __shared__ float Zs[kSmallTM][D + 1];                              // dZ of the tile's rows
+  for (int f = threadIdx.x; f < NW; f += kSmallTM) WTs[f] = __ldg(WT + f);
+  float wacc[WPT];
+#pragma unroll
+  for (int q = 0; q < WPT; ++q) wacc[q] = 0.f;
+  const int n_tiles = (N + kSmallTM - 1) / kSmallTM;
+  for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+    const int lr = threadIdx.x, row = tile * kSmallTM + lr;
+    __syncthreads();                                                 // WTs staged / the previous tile's rows consumed
+    if (row < N) {
+      float p[D], e[D], z[D];
+      load_row<D>(P, (size_t)row, p);
+      load_row<D>(E, (size_t)row, e);
+      {
+        float g[D], y[D];
+        load_row<D>(dOut, (size_t)row, g);
+        load_row<D>(Enext, (size_t)row, y);
+#pragma unroll
+        for (int c = 0; c < D; ++c) z[c] = y[c] > 0.f ? g[c] : kSlope * g[c];
+      }
+      // [dA | dB] = dZ W^T, k ascending from 0
+      float dA[D], dB[D];
+#pragma unroll
+      for (int j = 0; j < D; ++j) { dA[j] = 0.f; dB[j] = 0.f; }
+#pragma unroll
+      for (int k = 0; k < D; ++k)
+#pragma unroll
+        for (int j = 0; j < D; ++j) {
+          dA[j] = fmaf(z[k], WTs[k * 2 * D + j], dA[j]);
+          dB[j] = fmaf(z[k], WTs[k * 2 * D + D + j], dB[j]);
+        }
+      const size_t at = (size_t)row * D;
+#pragma unroll
+      for (int j = 0; j < D; ++j) {
+        dP[at + j] = fmaf(dB[j], e[j], dA[j]);
+        dEdir[at + j] = fmaf(dB[j], p[j], dA[j]);
+        As[lr][j] = p[j] + e[j];
+        As[lr][D + j] = p[j] * e[j];
+        Zs[lr][j] = z[j];
+      }
+    } else {
+#pragma unroll
+      for (int j = 0; j < D; ++j) { As[lr][j] = 0.f; As[lr][D + j] = 0.f; Zs[lr][j] = 0.f; }
+    }
+    __syncthreads();
+    // dW[j'][c] += sum_n A'[n][j'] dZ[n][c], n ascending; thread t owns the entries t, t + 128, ...
+#pragma unroll
+    for (int q = 0; q < WPT; ++q) {
+      const int w = threadIdx.x + q * kSmallTM, jr = w / D, c = w - jr * D;
+      float s_ = wacc[q];
+      for (int n = 0; n < kSmallTM; ++n) s_ = fmaf(As[n][jr], Zs[n][c], s_);
+      wacc[q] = s_;
+    }
+  }
+  float* out = dWpart + (size_t)blockIdx.x * NW;
+#pragma unroll
+  for (int q = 0; q < WPT; ++q) out[threadIdx.x + q * kSmallTM] = wacc[q];
+}
+
 __global__ void __launch_bounds__(256) reduce_wgrad_kernel(const float* __restrict__ part, int n_part, int n, float* __restrict__ dW) {
   const int k = blockIdx.x * 256 + threadIdx.x;
   if (k >= n) return;
@@ -251,12 +372,19 @@ extern "C" int agcf_ngcf_dense_forward(const float* P, const float* E, const flo
                                        const float* acc_in, float* acc_out, float acc_div,
                                        int32_t n_rows, int32_t d, agcf_stream_t stream) {
   if (!P || !E || !W || !Enext || n_rows < 0 || acc_div == 0.f) return AGCF_EINVAL;
-  if (d != 32 && d != 64) return AGCF_EUNSUPPORTED;
+  if (d != 8 && d != 16 && d != 32 && d != 64) return AGCF_EUNSUPPORTED;
   if (!aligned16(P) || !aligned16(E) || !aligned16(W) || !aligned16(Enext) || !aligned16(acc_in) || !aligned16(acc_out)) return AGCF_EINVAL;
   if (Enext == P || Enext == E) return AGCF_EINVAL;
   if (n_rows == 0) return AGCF_OK;
-  const unsigned blocks = (unsigned)((n_rows + ngcf::kTM - 1) / ngcf::kTM);
   cudaStream_t st = (cudaStream_t)stream;
+  if (d <= 16) {
+    const unsigned small_blocks = (unsigned)((n_rows + ngcf::kSmallTM - 1) / ngcf::kSmallTM);
+    if (d == 16) ngcf::dense_fwd_small_kernel<16><<<small_blocks, ngcf::kSmallTM, 0, st>>>(P, E, W, Enext, acc_in, acc_out, acc_div, n_rows);
+    else ngcf::dense_fwd_small_kernel<8><<<small_blocks, ngcf::kSmallTM, 0, st>>>(P, E, W, Enext, acc_in, acc_out, acc_div, n_rows);
+    AGCF_LAUNCH_OK();
+    return AGCF_OK;
+  }
+  const unsigned blocks = (unsigned)((n_rows + ngcf::kTM - 1) / ngcf::kTM);
   if (d == 64) ngcf::dense_fwd_kernel<64><<<blocks, 256, 0, st>>>(P, E, W, Enext, acc_in, acc_out, acc_div, n_rows);
   else ngcf::dense_fwd_kernel<32><<<blocks, 256, 0, st>>>(P, E, W, Enext, acc_in, acc_out, acc_div, n_rows);
   AGCF_LAUNCH_OK();
@@ -267,12 +395,18 @@ extern "C" int agcf_ngcf_dense_backward(const float* dOut, const float* Enext, c
                                         const float* WT, float* dP, float* dEdir, float* dW_partial,
                                         int32_t n_partials, int32_t n_rows, int32_t d, agcf_stream_t stream) {
   if (!dOut || !Enext || !P || !E || !WT || !dP || !dEdir || !dW_partial || n_rows < 0 || n_partials < 1) return AGCF_EINVAL;
-  if (d != 32 && d != 64) return AGCF_EUNSUPPORTED;
+  if (d != 8 && d != 16 && d != 32 && d != 64) return AGCF_EUNSUPPORTED;
   if (!aligned16(dOut) || !aligned16(Enext) || !aligned16(P) || !aligned16(E) || !aligned16(WT) || !aligned16(dP) ||
       !aligned16(dEdir) || !aligned16(dW_partial))
     return AGCF_EINVAL;
   if (dP == dOut || dEdir == dOut || dP == dEdir) return AGCF_EINVAL;
   cudaStream_t st = (cudaStream_t)stream;
+  if (d <= 16) {
+    if (d == 16) ngcf::dense_bwd_small_kernel<16><<<(unsigned)n_partials, ngcf::kSmallTM, 0, st>>>(dOut, Enext, P, E, WT, dP, dEdir, dW_partial, n_rows);
+    else ngcf::dense_bwd_small_kernel<8><<<(unsigned)n_partials, ngcf::kSmallTM, 0, st>>>(dOut, Enext, P, E, WT, dP, dEdir, dW_partial, n_rows);
+    AGCF_LAUNCH_OK();
+    return AGCF_OK;
+  }
 #define AGCF_NGCF_BWD(DD)                                                                                      \
   {                                                                                                            \
     AGCF_CUDA_OK(cudaFuncSetAttribute(ngcf::dense_bwd_kernel<DD>, cudaFuncAttributeMaxDynamicSharedMemorySize,  \
@@ -289,7 +423,7 @@ extern "C" int agcf_ngcf_dense_backward(const float* dOut, const float* Enext, c
 extern "C" int agcf_ngcf_reduce_wgrad(const float* dW_partial, int32_t n_partials, float* dW, int32_t d,
                                       agcf_stream_t stream) {
   if (!dW_partial || !dW || n_partials < 1) return AGCF_EINVAL;
-  if (d != 32 && d != 64) return AGCF_EUNSUPPORTED;
+  if (d != 8 && d != 16 && d != 32 && d != 64) return AGCF_EUNSUPPORTED;
   const int n = 2 * d * d;
   ngcf::reduce_wgrad_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(dW_partial, n_partials, n, dW);
   AGCF_LAUNCH_OK();

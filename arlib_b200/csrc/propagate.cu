@@ -1034,7 +1034,7 @@ extern "C" int agcf_spmm_csr_f32_ex(const agcf_spmm_args* a, agcf_stream_t strea
   if (a->n_peers < 0 || a->n_peers > AGCF_MAX_PEERS) return AGCF_EINVAL;
   if (!a->vrows || !a->vpart || !a->col || !a->val || !a->partial || !a->tickets || !a->X || a->n_vrows < 0) return AGCF_EINVAL;
   if (a->Y == nullptr && a->acc_out == nullptr && a->adam_p == nullptr) return AGCF_EINVAL;
-  if (!supported_row_d(a->d)) return AGCF_EUNSUPPORTED;
+  if (!supported_d(a->d)) return AGCF_EUNSUPPORTED;
   if (!aligned16(a->vrows) || !aligned16(a->partial)) return AGCF_EINVAL;
   if (!aligned16(a->X) || !aligned16(a->Y) || !aligned16(a->addend) || !aligned16(a->acc_in) || !aligned16(a->acc_out) ||
       !aligned16(a->noise) || !aligned16(a->mc_Y) || !aligned16(a->mc_acc))
@@ -1163,6 +1163,8 @@ extern "C" int agcf_sddmm_csr_f32(const int32_t* rowptr, const int32_t* col, con
     sddmm_csr_kernel<DD><<<blocks, 256, 0, st>>>(rowptr, col, H4, E4, gval, accumulate, row_order, n_rows); \
   }
   switch (d) {
+    case 8: AGCF_SDDMM(8) break;
+    case 16: AGCF_SDDMM(16) break;
     case 32: AGCF_SDDMM(32) break;
     case 64: AGCF_SDDMM(64) break;
     case 128: AGCF_SDDMM(128) break;

@@ -29,6 +29,9 @@
 //   a_i >= tau - 2*delta, so its group's maximum is >= tau - 2*delta: it is in a candidate group.
 //   Candidates are re-scored exactly and the selection / tie rule only look at items with
 //   e >= s*, all of which are candidates.  For impl 0, a == e bit for bit and delta = 0.
+//   delta holds at every d, d = 8 and 16 included: the truncation term and Cauchy-Schwarz do not depend on d, and the
+//   fp32 accumulation inside the tensor core adds at most ~d 2^-24 sum_k |u_k v_ik|, which the factor 1.01 covers for
+//   d <= 256 (smaller d only shrinks it).  Zero columns (padded operands) add exact zeros and change neither a nor e.
 #include "common.cuh"
 #include <float.h>
 #include <stdlib.h>
@@ -1360,7 +1363,7 @@ static int run_stage01(const float* Uemb, const int32_t* user_rows, int n_u, con
   if (impl == 1) {
     AGCF_CUDA_OK(cudaMemsetAsync(norm, 0, 4, st));
 #define AGCF_NORM(DD) max_row_norm_kernel<DD><<<(unsigned)((n_items + 255) / 256), 256, 0, st>>>(I4, n_items, norm);
-    switch (d) { case 32: AGCF_NORM(32) break; case 64: AGCF_NORM(64) break; case 128: AGCF_NORM(128) break; case 256: AGCF_NORM(256) break; }
+    switch (d) { case 8: AGCF_NORM(8) break; case 16: AGCF_NORM(16) break; case 32: AGCF_NORM(32) break; case 64: AGCF_NORM(64) break; case 128: AGCF_NORM(128) break; case 256: AGCF_NORM(256) break; }
 #undef AGCF_NORM
     AGCF_LAUNCH_OK();
     const int rc = launch_group_max_tc(Uemb, user_rows, n_u, Iemb, n_items, d, bits, L.n_groups, L.pitch, gmax,
@@ -1384,7 +1387,7 @@ static int run_stage01(const float* Uemb, const int32_t* user_rows, int n_u, con
     group_max_fp32_kernel<DD><<<grid, 256, S1Smem<DD>::bytes, st>>>(U4, user_rows, n_u, I4, n_items, bits,    \
                                                                     L.n_groups, L.pitch, tps, gmax);          \
   }
-    switch (d) { case 32: AGCF_S1(32) break; case 64: AGCF_S1(64) break; case 128: AGCF_S1(128) break; case 256: AGCF_S1(256) break; }
+    switch (d) { case 8: AGCF_S1(8) break; case 16: AGCF_S1(16) break; case 32: AGCF_S1(32) break; case 64: AGCF_S1(64) break; case 128: AGCF_S1(128) break; case 256: AGCF_S1(256) break; }
 #undef AGCF_S1
     AGCF_LAUNCH_OK();
   }
@@ -1519,7 +1522,7 @@ extern "C" int agcf_score_topk(const float* Uemb, const int32_t* user_rows, int3
     }                                                                                                            \
     topk_select_kernel<DD><<<(unsigned)L.grid2, 256, dyn, st>>>(p);                                              \
   }
-    switch (d) { case 32: AGCF_S2G(32) break; case 64: AGCF_S2G(64) break; case 128: AGCF_S2G(128) break; case 256: AGCF_S2G(256) break; }
+    switch (d) { case 8: AGCF_S2G(8) break; case 16: AGCF_S2G(16) break; case 32: AGCF_S2G(32) break; case 64: AGCF_S2G(64) break; case 128: AGCF_S2G(128) break; case 256: AGCF_S2G(256) break; }
 #undef AGCF_S2G
     AGCF_LAUNCH_OK();
     return AGCF_OK;
@@ -1534,7 +1537,7 @@ extern "C" int agcf_score_topk(const float* Uemb, const int32_t* user_rows, int3
     topk_select_warp_kernel<DD><<<(unsigned)L.grid_w, 32 * S2W<DD>::WPC, dyn_w, st>>>(p);                        \
     topk_select_kernel<DD><<<(unsigned)L.grid2, 256, dyn, st>>>(p);                                              \
   }
-  switch (d) { case 32: AGCF_S2(32) break; case 64: AGCF_S2(64) break; case 128: AGCF_S2(128) break; case 256: AGCF_S2(256) break; }
+  switch (d) { case 8: AGCF_S2(8) break; case 16: AGCF_S2(16) break; case 32: AGCF_S2(32) break; case 64: AGCF_S2(64) break; case 128: AGCF_S2(128) break; case 256: AGCF_S2(256) break; }
 #undef AGCF_S2
   AGCF_LAUNCH_OK();
   return AGCF_OK;
@@ -1567,6 +1570,8 @@ extern "C" int agcf_score_rows(const float* Uemb, const int32_t* user_rows, int3
   const float4* U4 = reinterpret_cast<const float4*>(Uemb);
   const float4* I4 = reinterpret_cast<const float4*>(Iemb);
   switch (d) {
+    case 8: score_rows_kernel<8><<<grid, 256, 0, st>>>(U4, user_rows, I4, n_items, out); break;
+    case 16: score_rows_kernel<16><<<grid, 256, 0, st>>>(U4, user_rows, I4, n_items, out); break;
     case 32: score_rows_kernel<32><<<grid, 256, 0, st>>>(U4, user_rows, I4, n_items, out); break;
     case 64: score_rows_kernel<64><<<grid, 256, 0, st>>>(U4, user_rows, I4, n_items, out); break;
     case 128: score_rows_kernel<128><<<grid, 256, 0, st>>>(U4, user_rows, I4, n_items, out); break;

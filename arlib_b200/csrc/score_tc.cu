@@ -6,9 +6,10 @@
 // one GEMV per user in the reference) as a persistent, warp-specialised tcgen05 GEMM:
 //   * operands are the fp32 embedding tables themselves, consumed as TF32
 //     (kind::tf32 reads the upper 19 bits of each fp32 word): no conversion pass;
-//   * TMA (cp.async.bulk.tensor.2d, 128-byte swizzle) stages a 128-user A tile once per
-//     work unit and streams 256-item B tiles through a 2-stage ring;
-//   * one elected thread issues 8 x tcgen05.mma (M128 x N256 x K8) per tile into one of
+//   * TMA (cp.async.bulk.tensor.2d, 128-byte swizzle; 32- / 64-byte at d = 8 / 16, whose rows are
+//     narrower than one 128-byte atom row) stages a 128-user A tile once per work unit and streams
+//     256-item B tiles through a 2-stage ring;
+//   * one elected thread issues d/8 x tcgen05.mma (M128 x N256 x K8) per tile into one of
 //     two 256-column TMEM accumulators, tcgen05.commit signals the mbarriers;
 //   * four epilogue warps read the accumulator with tcgen05.ld (32 lanes x 32 columns =
 //     one user x one 32-item group per thread), apply the train-item mask bits, reduce
@@ -25,7 +26,6 @@ namespace agcf {
 namespace tc {
 
 constexpr int kTileM = 128;            // users per tile (UMMA M)
-constexpr int kKBlock = 32;            // fp32 elements per 128-byte swizzle atom row
 constexpr int kUmmaK = 8;              // K per tcgen05.mma for tf32 (32 bytes)
 constexpr int kStages = 2;
 #ifndef AGCF_TC_EPI_WG
@@ -74,16 +74,19 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* t
       : "memory");
 }
 
-// K-major, 128-byte-swizzle shared-memory matrix descriptor (cute::UMMA::SmemDescriptor):
-// start address >> 4, LBO = 1 (ignored for swizzled K-major), SBO = 8 rows x 128 B = 1024 B,
-// version 1 (Blackwell), layout type 2 = SWIZZLE_128B.
+// K-major, swizzled shared-memory matrix descriptor (cute::UMMA::SmemDescriptor) for atom rows of
+// ROW_BYTES = 128, 64 or 32: start address >> 4, LBO = 1 (ignored for swizzled K-major),
+// SBO = 8 rows x ROW_BYTES, version 1 (Blackwell), layout type 2 / 4 / 6 = SWIZZLE_128B / 64B / 32B.
+template <int ROW_BYTES>
 __device__ __forceinline__ uint64_t make_smem_desc(uint32_t smem_addr) {
+  static_assert(ROW_BYTES == 128 || ROW_BYTES == 64 || ROW_BYTES == 32, "swizzle width");
+  constexpr uint64_t layout = ROW_BYTES == 128 ? 2 : (ROW_BYTES == 64 ? 4 : 6);
   uint64_t d = 0;
   d |= (uint64_t)((smem_addr >> 4) & 0x3FFF);
   d |= (uint64_t)1 << 16;
-  d |= (uint64_t)(1024 >> 4) << 32;
+  d |= (uint64_t)((8 * ROW_BYTES) >> 4) << 32;
   d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
+  d |= layout << 61;
   return d;
 }
 
@@ -129,9 +132,11 @@ struct alignas(8) Barriers {
 template <int D>
 struct Smem {
   static constexpr int kTileN = D <= 64 ? 256 : 128;   // items per tile (UMMA N); smaller for d = 128 (smem)
+  static constexpr int kKBlock = D < 32 ? D : 32;       // fp32 elements per swizzle atom row (a row of 128, 64 or 32 B)
+  static constexpr int kRowBytes = kKBlock * 4;
   static constexpr int kKBlocks = D / kKBlock;
-  static constexpr int kABytes = kKBlocks * kTileM * 128;
-  static constexpr int kBBytes = kKBlocks * kTileN * 128;
+  static constexpr int kABytes = kKBlocks * kTileM * kRowBytes;
+  static constexpr int kBBytes = kKBlocks * kTileN * kRowBytes;
   static constexpr int kTotal = kABytes + kStages * kBBytes + 1024 /*alignment slack*/ + 256 /*barriers*/;
 };
 
@@ -180,12 +185,13 @@ group_max_tc_kernel(const __grid_constant__ CUtensorMap tmap_u, const __grid_con
         mbar_wait(&bars->a_empty, (unit_iter & 1) ^ 1);            // MMA finished with the previous A tile
         mbar_arrive_expect_tx(&bars->a_full, S::kABytes);
         for (int kb = 0; kb < S::kKBlocks; ++kb)
-          tma_load_2d(sA + kb * kTileM * 128, &tmap_u, &bars->a_full, kb * kKBlock, ut * kTileM);
+          tma_load_2d(sA + kb * kTileM * S::kRowBytes, &tmap_u, &bars->a_full, kb * S::kKBlock, ut * kTileM);
         for (int t = t0; t < t1; ++t) {
           mbar_wait(&bars->b_empty[stage], b_phase ^ 1);
           mbar_arrive_expect_tx(&bars->b_full[stage], S::kBBytes);
           for (int kb = 0; kb < S::kKBlocks; ++kb)
-            tma_load_2d(sB + stage * S::kBBytes + kb * kTileN * 128, &tmap_i, &bars->b_full[stage], kb * kKBlock, t * kTileN);
+            tma_load_2d(sB + stage * S::kBBytes + kb * kTileN * S::kRowBytes, &tmap_i, &bars->b_full[stage], kb * S::kKBlock,
+                        t * kTileN);
           if (++stage == kStages) { stage = 0; b_phase ^= 1; }
         }
       }
@@ -207,10 +213,10 @@ group_max_tc_kernel(const __grid_constant__ CUtensorMap tmap_u, const __grid_con
           const uint32_t d_tmem = tmem_base + acc * kTileN;
 #pragma unroll
           for (int kb = 0; kb < S::kKBlocks; ++kb) {
-            const uint64_t adesc = make_smem_desc(smem_u32(sA + kb * kTileM * 128));
-            const uint64_t bdesc = make_smem_desc(smem_u32(sB + stage * S::kBBytes + kb * kTileN * 128));
+            const uint64_t adesc = make_smem_desc<S::kRowBytes>(smem_u32(sA + kb * kTileM * S::kRowBytes));
+            const uint64_t bdesc = make_smem_desc<S::kRowBytes>(smem_u32(sB + stage * S::kBBytes + kb * kTileN * S::kRowBytes));
 #pragma unroll
-            for (int k = 0; k < kKBlock / kUmmaK; ++k)            // +32 bytes along K inside the swizzle atom
+            for (int k = 0; k < S::kKBlock / kUmmaK; ++k)         // +32 bytes along K inside the swizzle atom
               umma_tf32(d_tmem, adesc + (uint64_t)(k * 2), bdesc + (uint64_t)(k * 2), idesc, (kb | k) != 0);
           }
           umma_commit(&bars->b_empty[stage]);                      // smem stage reusable once these MMAs retire
@@ -334,16 +340,18 @@ static EncodeTiledFn get_encode_fn() {
   return fn;
 }
 
-// [rows, d] fp32 row-major; box = 32 floats (one 128-byte swizzle row) x box_rows
-static int make_tmap(CUtensorMap* m, const float* base, int rows, int d, int box_rows) {
+// [rows, d] fp32 row-major; box = box_cols floats (one swizzle atom row of 4 box_cols bytes) x box_rows
+static int make_tmap(CUtensorMap* m, const float* base, int rows, int d, int box_cols, int box_rows) {
   EncodeTiledFn enc = get_encode_fn();
   if (enc == nullptr) return AGCF_ECUDA;
   cuuint64_t dims[2] = {(cuuint64_t)d, (cuuint64_t)rows};
   cuuint64_t strides[1] = {(cuuint64_t)d * sizeof(float)};
-  cuuint32_t box[2] = {(cuuint32_t)kKBlock, (cuuint32_t)box_rows};
+  cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
+  const CUtensorMapSwizzle swz = box_cols == 32 ? CU_TENSOR_MAP_SWIZZLE_128B
+                                                : (box_cols == 16 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
   cuuint32_t estr[2] = {1, 1};
   CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   return r == CUDA_SUCCESS ? AGCF_OK : AGCF_ECUDA;
 }
@@ -352,10 +360,10 @@ template <int D>
 static int launch(const float* U, int n_u, const float* I, int n_items, const uint32_t* bits, int n_groups, int pitch,
                   float* gmax, cudaStream_t st) {
   CUtensorMap tu, ti;
-  int rc = make_tmap(&tu, U, n_u, D, kTileM);
+  int rc = make_tmap(&tu, U, n_u, D, Smem<D>::kKBlock, kTileM);
   if (rc != AGCF_OK) return rc;
   constexpr int kTileN = Smem<D>::kTileN;
-  rc = make_tmap(&ti, I, n_items, D, kTileN);
+  rc = make_tmap(&ti, I, n_items, D, Smem<D>::kKBlock, kTileN);
   if (rc != AGCF_OK) return rc;
   const int n_user_tiles = (n_u + kTileM - 1) / kTileM;
   const int n_item_tiles = (n_items + kTileN - 1) / kTileN;
@@ -390,6 +398,8 @@ int launch_group_max_tc(const float* Uemb, const int32_t* user_rows, int n_u, co
     U = u_dense;
   }
   switch (d) {
+    case 8: return tc::launch<8>(U, n_u, Iemb, n_items, bits, n_groups, pitch, gmax, st);
+    case 16: return tc::launch<16>(U, n_u, Iemb, n_items, bits, n_groups, pitch, gmax, st);
     case 32: return tc::launch<32>(U, n_u, Iemb, n_items, bits, n_groups, pitch, gmax, st);
     case 64: return tc::launch<64>(U, n_u, Iemb, n_items, bits, n_groups, pitch, gmax, st);
     case 128: return tc::launch<128>(U, n_u, Iemb, n_items, bits, n_groups, pitch, gmax, st);

@@ -806,8 +806,8 @@ class NGCFEngine(LightGCNEngine):
     def __init__(self, graph, table, W, n_users, lr, reg, batch_size, max_triples, betas=(0.9, 0.999), adam_eps=1e-8):
         n_layers = int(W.shape[0])
         d = table.shape[1]
-        if d not in (32, 64) or tuple(W.shape) != (n_layers, 2 * d, d) or not W.is_contiguous():
-            raise ValueError("NGCFEngine: d in {32, 64} and W packed as [L, 2d, d]")
+        if d not in (8, 16, 32, 64) or tuple(W.shape) != (n_layers, 2 * d, d) or not W.is_contiguous():
+            raise ValueError("NGCFEngine: d in {8, 16, 32, 64} and W packed as [L, 2d, d]")
         super().__init__(graph, table, n_users, n_layers, lr, reg, batch_size, max_triples, betas=betas, adam_eps=adam_eps,
                          sparse_layers=False)
         f = lambda: torch.empty_like(table)

@@ -1,7 +1,7 @@
 """NGCF -- drop-in for the reference's recommender/NGCF.py (train loop :31-79, encoder :163-212).
 
 ``train()`` has two paths with the same mathematics:
-  * fused (the recommender owns the optimizer, no gradient export, d in {32, 64}): arlib_b200.engine.NGCFEngine -- one
+  * fused (the recommender owns the optimizer, no gradient export, d in {8, 16, 32, 64}): arlib_b200.engine.NGCFEngine -- one
     propagation per layer (A (E W1) = (A E) W1) + the fused dense layer kernels of csrc/ngcf.cu, forward and backward,
     Adam on the table fused into the last SpMM, replayed from a CUDA graph;
   * general (caller's optimizer, requires_adjgrad / requires_embgrad): the reference loop on torch autograd with the
@@ -24,7 +24,7 @@ class NGCF(GraphRecommender):
         self.bestPerformance = []
         model = self.model.cuda()
         if optimizer is None and not (requires_adjgrad or requires_embgrad) and self._fused_ok() \
-                and int(self.args.emb_size) in (32, 64) and model.layers >= 1:
+                and int(self.args.emb_size) in (8, 16, 32, 64) and model.layers >= 1:
             self._train_fused_ngcf(model, Epoch if Epoch else self.args.maxEpoch, evalNum)
             self.user_emb, self.item_emb = self.best_user_emb, self.best_item_emb
             return None

@@ -32,8 +32,8 @@ class GraphRecommender(object):
         self.max_N = max(self.topN)
         # the row kernels hold a row as d/4 float4 lanes and are compiled for these widths only (csrc/common.cuh);
         # there is no fallback path by design, so say so here instead of failing inside the first propagation
-        if int(self.args.emb_size) not in (32, 64, 128, 256):
-            raise ValueError("arlib_b200: emb_size must be one of 32, 64, 128, 256 (got %r); the sm_100a row kernels "
+        if int(self.args.emb_size) not in (8, 16, 32, 64, 128, 256):
+            raise ValueError("arlib_b200: emb_size must be one of 8, 16, 32, 64, 128, 256 (got %r); the sm_100a kernels "
                              "are compiled for these widths and there is no CPU / generic fallback" % (self.args.emb_size,))
         self._evaluator = None
         self._train_set = None                # device mirrors are derived from ``data``: a re-__init__ drops both

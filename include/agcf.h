@@ -14,8 +14,7 @@
  *     enqueues work on it and is capturable in a CUDA graph;
  *   - return value: 0 = ok, <0 = AGCF_E* below; nothing throws;
  *   - fp32 everywhere, int32 indices; tables are row-major [rows, d], 16-byte
- *     aligned, d in {32, 64, 128, 256}; the row kernels (propagation, loss, optimizer) also take
- *     d in {8, 16}: the column slices of d-sharded multi-GPU tables;
+ *     aligned, d in {8, 16, 32, 64, 128, 256} (the NGCF dense layer: d in {8, 16, 32, 64});
  *   - a "node" id is a row of the stacked table [users; items] (N = U + I); item
  *     ids handed to the loss / sampler / eval calls are item-local (0..I-1).
  */
@@ -292,7 +291,7 @@ int agcf_zero_rows(const int32_t* seg_node, const int32_t* n_seg, int32_t max_se
  * n_dev), and produces scale * grad_loss[0] * d loss / d view (grad_loss nullable = 1): grad_viewK is [n, d], or
  * -- with rowsK -- a table whose rows rowsK[r] receive the rows of the gradient (ids must be unique);
  * accumulateK != 0 adds to what is there.  Either gradient may be null.
- * Deterministic (partials combined in a fixed order).  d in {32, 64, 128, 256}. */
+ * Deterministic (partials combined in a fixed order).  d in {8, 16, 32, 64, 128, 256}. */
 int64_t agcf_infonce_ws_bytes(int32_t n, int32_t d);
 int agcf_infonce_forward(const float* view1, const float* view2, const int32_t* rows, int32_t n, const int32_t* n_dev,
                          int32_t d, float temperature, float* loss, void* ws, int64_t ws_bytes, agcf_stream_t stream);
@@ -310,7 +309,7 @@ int agcf_infonce_backward(int32_t n, const int32_t* n_dev, int32_t d, float temp
  *             ([n_partials][2d*d]; the launch runs n_partials persistent CTAs);
  *             the gradient of E is then A dP + dEdir (next agcf_spmm_csr_f32, addend = dEdir);
  *   reduce    dW = sum_b dW_partial[b] in b order (deterministic).
- * Uses A (E W1) = (A E) W1: one propagation per layer where the reference runs two.  d in {32, 64}.
+ * Uses A (E W1) = (A E) W1: one propagation per layer where the reference runs two.  d in {8, 16, 32, 64}.
  * Replaces: the loop body of NGCF_Encoder.forward (recommender/NGCF.py:197-212: torch.mm x 2,
  * torch.sparse.mm x 2, leaky_relu, the element-wise product / sums) and its autograd. */
 int agcf_ngcf_dense_forward(const float* P, const float* E, const float* W, float* Enext,
