@@ -14,7 +14,8 @@
 //   agcf_ngcf_dense_forward    E' (and the running layer mean)               from P, E, W = [W1 ; W2]
 //   agcf_ngcf_dense_backward   dP, dE_direct and per-CTA partials of dW       from dE', E' (sign of Z), P, E, W^T
 //   agcf_ngcf_reduce_wgrad     dW = sum of the partials in CTA order (deterministic)
-// d in {8, 16, 32, 64}: a 64-row tile on a 16 x 16 thread grid at 32 and 64, a row per thread at 8 and 16.
+// d in {8, 16, 32, 64, 128, 256}: a 64-row tile on a 16 x 16 thread grid at 32 and 64, a row per thread at 8 and 16, and
+// at 128 and 256 a 128 x 128 tile per product, with dW split over row slices (one partial per slice).
 //
 // Backward:  dZ = dE' * (E' > 0 ? 1 : 0.01)      (leaky_relu keeps the sign, so E' tells which branch Z took)
 //            [dA | dB] = dZ [W1 ; W2]^T ;  dP = dA + dB * E ;  dE_direct = dA + dB * P ;  dW = [P + E | P * E]^T dZ
@@ -42,21 +43,21 @@ __device__ __forceinline__ void load_cols(const float* __restrict__ src, float (
   }
 }
 
-// acc[4][CN] += As[ty*4 + r][0 .. KC) . Bs[0 .. KC)[tx*CN + c]      (As rows padded to KC + 4 floats)
-template <int D, int CN>
+// acc[RM][CN] += As[ty*RM + r][0 .. KC) . Bs[0 .. KC)[tx*CN + c]      (As rows padded to KC + 4 floats)
+template <int RM, int CN>
 __device__ __forceinline__ void tile_mac(const float (*As)[kKC + 4], const float* __restrict__ Bs, int ldb, int ty, int tx,
-                                         float (&acc)[4][CN]) {
+                                         float (&acc)[RM][CN]) {
 #pragma unroll 4
   for (int k = 0; k < kKC; k += 4) {
-    float4 a[4];
+    float4 a[RM];
 #pragma unroll
-    for (int r = 0; r < 4; ++r) a[r] = *reinterpret_cast<const float4*>(&As[ty * 4 + r][k]);
+    for (int r = 0; r < RM; ++r) a[r] = *reinterpret_cast<const float4*>(&As[ty * RM + r][k]);
 #pragma unroll
     for (int kk = 0; kk < 4; ++kk) {
       float w[CN];
       load_cols<CN>(Bs + (size_t)(k + kk) * ldb + tx * CN, w);
 #pragma unroll
-      for (int r = 0; r < 4; ++r) {
+      for (int r = 0; r < RM; ++r) {
         const float av = kk == 0 ? a[r].x : (kk == 1 ? a[r].y : (kk == 2 ? a[r].z : a[r].w));
 #pragma unroll
         for (int c = 0; c < CN; ++c) acc[r][c] = fmaf(av, w[c], acc[r][c]);
@@ -99,7 +100,7 @@ __global__ void __launch_bounds__(256) dense_fwd_kernel(const float* __restrict_
     for (int f = tid; f < kKC * D / 4; f += 256)
       reinterpret_cast<float4*>(Ws)[f] = __ldg(reinterpret_cast<const float4*>(W + (size_t)kc * D) + f);
     __syncthreads();
-    tile_mac<D, CN>(As, Ws, D, ty, tx, acc);
+    tile_mac<4, CN>(As, Ws, D, ty, tx, acc);
     __syncthreads();
   }
 #pragma unroll
@@ -191,8 +192,8 @@ __global__ void __launch_bounds__(256, 2) dense_bwd_kernel(const float* __restri
           reinterpret_cast<float4*>(Bs)[f] = v;
         }
         __syncthreads();
-        if (half == 0) tile_mac<D, CN>(As, Bs, D, ty, tx, accA);
-        else tile_mac<D, CN>(As, Bs, D, ty, tx, accB);
+        if (half == 0) tile_mac<4, CN>(As, Bs, D, ty, tx, accA);
+        else tile_mac<4, CN>(As, Bs, D, ty, tx, accB);
         __syncthreads();
       }
     }
@@ -355,11 +356,193 @@ __global__ void __launch_bounds__(kSmallTM) dense_bwd_small_kernel(const float* 
   for (int q = 0; q < WPT; ++q) out[threadIdx.x + q * kSmallTM] = wacc[q];
 }
 
+// ------------------------------------------------------------------ d = 128 and 256
+// The 64-row tiles above do not fit these widths: the forward's weight chunk takes its static shared memory past 48 KB,
+// the backward would stage 150 / 281 KB and hold 128 / 512 dW accumulators per thread.  So each of the three products
+// is a kernel of its own on one tile shape -- 128 rows x 128 columns on the 16 x 16 thread grid, 8 x 8 outputs per
+// thread, K in chunks of 64 staged in 66 KB of dynamic shared memory -- over column blocks of its output:
+//   dense_fwd_wide_kernel    Z = A' W                  grid (row tiles, D / 128)
+//   dense_dzwt_wide_kernel   [dA | dB] = dZ W^T        grid (row tiles, D / 64); the tile's columns interleave dA_j and
+//                            dB_j, so the thread that holds both forms dP and dE_direct
+//   dense_wgrad_wide_kernel  dW = A'^T dZ, split over K: grid (dW tiles, n_partials row slices), one partial per slice,
+//                            which reduce_wgrad_kernel adds in slice order
+// dZ and A' are recomputed from dOut, Enext, P and E wherever a kernel stages them.  Every output is one fmaf chain, k
+// ascending (dW: within its slice): exact fp32 and deterministic, like the narrower kernels.
+constexpr int kWM = 128;          // rows and columns of a wide tile
+constexpr int kWR = kWM / 16;     // rows and columns per thread
+constexpr size_t kWideSmemBytes = (size_t)(kWM * (kKC + 4) + kKC * kWM) * 4;
+
+__device__ __forceinline__ float4 dz_of(float4 g, float4 y) {        // dZ = dE' * (E' > 0 ? 1 : 0.01)
+  return make_float4(y.x > 0.f ? g.x : kSlope * g.x, y.y > 0.f ? g.y : kSlope * g.y,
+                     y.z > 0.f ? g.z : kSlope * g.z, y.w > 0.f ? g.w : kSlope * g.w);
+}
+
+template <int D>
+__global__ void __launch_bounds__(256) dense_fwd_wide_kernel(const float* __restrict__ P, const float* __restrict__ E,
+                                                             const float* __restrict__ W, float* __restrict__ Enext,
+                                                             const float* __restrict__ acc_in, float* __restrict__ acc_out,
+                                                             float acc_div, int N) {
+  extern __shared__ __align__(16) unsigned char wide_smem[];
+  float (*As)[kKC + 4] = reinterpret_cast<float (*)[kKC + 4]>(wide_smem);   // [WM][KC + 4]: A' chunk
+  float* Ws = reinterpret_cast<float*>(wide_smem) + kWM * (kKC + 4);         // [KC][WM]: W chunk of the column block
+  const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
+  const int row0 = blockIdx.x * kWM, c0 = blockIdx.y * kWM;
+  float acc[kWR][kWR];
+#pragma unroll
+  for (int r = 0; r < kWR; ++r)
+#pragma unroll
+    for (int c = 0; c < kWR; ++c) acc[r][c] = 0.f;
+  for (int kc = 0; kc < 2 * D; kc += kKC) {
+    const int part = kc / D, col = kc - part * D;                   // a chunk stays inside one part (D % KC == 0)
+    for (int f = tid; f < kWM * (kKC / 4); f += 256) {
+      const int r = f / (kKC / 4), k4 = f - r * (kKC / 4);
+      const int row = row0 + r;
+      float4 p = make_float4(0.f, 0.f, 0.f, 0.f), e = p;
+      if (row < N) {
+        p = __ldg(reinterpret_cast<const float4*>(P + (size_t)row * D + col) + k4);
+        e = __ldg(reinterpret_cast<const float4*>(E + (size_t)row * D + col) + k4);
+      }
+      *reinterpret_cast<float4*>(&As[r][4 * k4]) = part == 0 ? make_float4(p.x + e.x, p.y + e.y, p.z + e.z, p.w + e.w)
+                                                             : make_float4(p.x * e.x, p.y * e.y, p.z * e.z, p.w * e.w);
+    }
+    for (int f = tid; f < kKC * (kWM / 4); f += 256) {
+      const int k = f / (kWM / 4), c4 = f - k * (kWM / 4);
+      reinterpret_cast<float4*>(Ws)[f] = __ldg(reinterpret_cast<const float4*>(W + (size_t)(kc + k) * D + c0) + c4);
+    }
+    __syncthreads();
+    tile_mac<kWR, kWR>(As, Ws, kWM, ty, tx, acc);
+    __syncthreads();
+  }
+#pragma unroll
+  for (int r = 0; r < kWR; ++r) {
+    const int row = row0 + ty * kWR + r;
+    if (row >= N) continue;
+    const size_t at = (size_t)row * D + c0 + tx * kWR;
+#pragma unroll
+    for (int c = 0; c < kWR; ++c) {
+      const float z = acc[r][c];
+      const float o = z > 0.f ? z : kSlope * z;                      // F.leaky_relu(z, 0.01)
+      Enext[at + c] = o;
+      if (acc_out != nullptr) {
+        float m = (acc_in != nullptr ? acc_in[at + c] : 0.f) + o;
+        if (acc_div != 1.0f) m = __fdiv_rn(m, acc_div);
+        acc_out[at + c] = m;
+      }
+    }
+  }
+}
+
+template <int D>
+__global__ void __launch_bounds__(256) dense_dzwt_wide_kernel(const float* __restrict__ dOut, const float* __restrict__ Enext,
+                                                              const float* __restrict__ P, const float* __restrict__ E,
+                                                              const float* __restrict__ WT, float* __restrict__ dP,
+                                                              float* __restrict__ dEdir, int N) {
+  extern __shared__ __align__(16) unsigned char wide_smem[];
+  float (*As)[kKC + 4] = reinterpret_cast<float (*)[kKC + 4]>(wide_smem);   // [WM][KC + 4]: dZ chunk
+  float* Bs = reinterpret_cast<float*>(wide_smem) + kWM * (kKC + 4);         // [KC][WM]: Bs[k][2j + h] = W^T[k][h D + j0 + j]
+  const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
+  const int row0 = blockIdx.x * kWM, j0 = blockIdx.y * (kWM / 2);
+  float acc[kWR][kWR];                                                // acc[r][2q] = dA, acc[r][2q + 1] = dB of column j0 + 4 tx + q
+#pragma unroll
+  for (int r = 0; r < kWR; ++r)
+#pragma unroll
+    for (int c = 0; c < kWR; ++c) acc[r][c] = 0.f;
+  for (int kc = 0; kc < D; kc += kKC) {
+    for (int f = tid; f < kWM * (kKC / 4); f += 256) {
+      const int r = f / (kKC / 4), k4 = f - r * (kKC / 4);
+      const int row = row0 + r;
+      float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (row < N) {
+        const size_t at = (size_t)row * D + kc + 4 * k4;
+        z = dz_of(__ldg(reinterpret_cast<const float4*>(dOut + at)), __ldg(reinterpret_cast<const float4*>(Enext + at)));
+      }
+      *reinterpret_cast<float4*>(&As[r][4 * k4]) = z;
+    }
+    for (int f = tid; f < kKC * (kWM / 8); f += 256) {
+      const int k = f / (kWM / 8), j4 = f - k * (kWM / 8);
+      const float* src = WT + (size_t)(kc + k) * 2 * D + j0 + 4 * j4;
+      const float4 a = __ldg(reinterpret_cast<const float4*>(src)), b = __ldg(reinterpret_cast<const float4*>(src + D));
+      float4* dst = reinterpret_cast<float4*>(Bs + k * kWM + 8 * j4);
+      dst[0] = make_float4(a.x, b.x, a.y, b.y);
+      dst[1] = make_float4(a.z, b.z, a.w, b.w);
+    }
+    __syncthreads();
+    tile_mac<kWR, kWR>(As, Bs, kWM, ty, tx, acc);
+    __syncthreads();
+  }
+#pragma unroll
+  for (int r = 0; r < kWR; ++r) {
+    const int row = row0 + ty * kWR + r;
+    if (row >= N) continue;
+    const size_t at = (size_t)row * D + j0 + 4 * tx;
+    const float4 e = __ldg(reinterpret_cast<const float4*>(E + at)), p = __ldg(reinterpret_cast<const float4*>(P + at));
+    *reinterpret_cast<float4*>(dP + at) = make_float4(fmaf(acc[r][1], e.x, acc[r][0]), fmaf(acc[r][3], e.y, acc[r][2]),
+                                                      fmaf(acc[r][5], e.z, acc[r][4]), fmaf(acc[r][7], e.w, acc[r][6]));
+    *reinterpret_cast<float4*>(dEdir + at) = make_float4(fmaf(acc[r][1], p.x, acc[r][0]), fmaf(acc[r][3], p.y, acc[r][2]),
+                                                         fmaf(acc[r][5], p.z, acc[r][4]), fmaf(acc[r][7], p.w, acc[r][6]));
+  }
+}
+
+template <int D>
+__global__ void __launch_bounds__(256) dense_wgrad_wide_kernel(const float* __restrict__ dOut, const float* __restrict__ Enext,
+                                                               const float* __restrict__ P, const float* __restrict__ E,
+                                                               float* __restrict__ dWpart, int N) {
+  extern __shared__ __align__(16) unsigned char wide_smem[];
+  float (*As)[kKC + 4] = reinterpret_cast<float (*)[kKC + 4]>(wide_smem);   // [WM][KC + 4]: As[j][n] = A'[n0 + n][j0 + j]
+  float* Zs = reinterpret_cast<float*>(wide_smem) + kWM * (kKC + 4);         // [KC][WM]:     Zs[n][c] = dZ[n0 + n][c0 + c]
+  const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
+  constexpr int kColTiles = D / kWM;
+  const int j0 = (blockIdx.x / kColTiles) * kWM, c0 = (blockIdx.x % kColTiles) * kWM;
+  const int part = j0 / D, col0 = j0 - part * D;                   // a 128-row block of dW stays inside one part
+  const int n_chunks = (N + kKC - 1) / kKC, per = (n_chunks + gridDim.y - 1) / gridDim.y;
+  const int ch0 = blockIdx.y * per, ch1 = min(n_chunks, ch0 + per);
+  float acc[kWR][kWR];
+#pragma unroll
+  for (int r = 0; r < kWR; ++r)
+#pragma unroll
+    for (int c = 0; c < kWR; ++c) acc[r][c] = 0.f;
+  for (int ch = ch0; ch < ch1; ++ch) {
+    const int n0 = ch * kKC;
+    for (int f = tid; f < kKC * (kWM / 4); f += 256) {              // n fastest across a warp: conflict-free stores
+      const int n = f % kKC, j4 = f / kKC;
+      const int row = n0 + n;
+      float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (row < N) {
+        const float4 p = __ldg(reinterpret_cast<const float4*>(P + (size_t)row * D + col0) + j4);
+        const float4 e = __ldg(reinterpret_cast<const float4*>(E + (size_t)row * D + col0) + j4);
+        v = part == 0 ? make_float4(p.x + e.x, p.y + e.y, p.z + e.z, p.w + e.w)
+                      : make_float4(p.x * e.x, p.y * e.y, p.z * e.z, p.w * e.w);
+      }
+      As[4 * j4][n] = v.x; As[4 * j4 + 1][n] = v.y; As[4 * j4 + 2][n] = v.z; As[4 * j4 + 3][n] = v.w;
+    }
+    for (int f = tid; f < kKC * (kWM / 4); f += 256) {
+      const int n = f / (kWM / 4), c4 = f - n * (kWM / 4);
+      const int row = n0 + n;
+      float4 z = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (row < N) {
+        const size_t at = (size_t)row * D + c0 + 4 * c4;
+        z = dz_of(__ldg(reinterpret_cast<const float4*>(dOut + at)), __ldg(reinterpret_cast<const float4*>(Enext + at)));
+      }
+      reinterpret_cast<float4*>(Zs)[f] = z;
+    }
+    __syncthreads();
+    tile_mac<kWR, kWR>(As, Zs, kWM, ty, tx, acc);
+    __syncthreads();
+  }
+  float* out = dWpart + (size_t)blockIdx.y * 2 * D * D;
+#pragma unroll
+  for (int r = 0; r < kWR; ++r) {
+    float4* dst = reinterpret_cast<float4*>(out + (size_t)(j0 + ty * kWR + r) * D + c0 + tx * kWR);
+    dst[0] = make_float4(acc[r][0], acc[r][1], acc[r][2], acc[r][3]);
+    dst[1] = make_float4(acc[r][4], acc[r][5], acc[r][6], acc[r][7]);
+  }
+}
+
 __global__ void __launch_bounds__(256) reduce_wgrad_kernel(const float* __restrict__ part, int n_part, int n, float* __restrict__ dW) {
   const int k = blockIdx.x * 256 + threadIdx.x;
   if (k >= n) return;
   float s = 0.f;
-  for (int b = 0; b < n_part; ++b) s += part[(size_t)b * n + k];      // CTA order: deterministic
+  for (int b = 0; b < n_part; ++b) s += part[(size_t)b * n + k];      // CTA (d >= 128: slice) order: deterministic
   dW[k] = s;
 }
 
@@ -372,11 +555,25 @@ extern "C" int agcf_ngcf_dense_forward(const float* P, const float* E, const flo
                                        const float* acc_in, float* acc_out, float acc_div,
                                        int32_t n_rows, int32_t d, agcf_stream_t stream) {
   if (!P || !E || !W || !Enext || n_rows < 0 || acc_div == 0.f) return AGCF_EINVAL;
-  if (d != 8 && d != 16 && d != 32 && d != 64) return AGCF_EUNSUPPORTED;
+  if (d != 8 && d != 16 && d != 32 && d != 64 && d != 128 && d != 256) return AGCF_EUNSUPPORTED;
   if (!aligned16(P) || !aligned16(E) || !aligned16(W) || !aligned16(Enext) || !aligned16(acc_in) || !aligned16(acc_out)) return AGCF_EINVAL;
   if (Enext == P || Enext == E) return AGCF_EINVAL;
   if (n_rows == 0) return AGCF_OK;
   cudaStream_t st = (cudaStream_t)stream;
+  if (d >= 128) {
+    const dim3 grid((unsigned)((n_rows + ngcf::kWM - 1) / ngcf::kWM), (unsigned)(d / ngcf::kWM));
+#define AGCF_NGCF_FWD_WIDE(DD)                                                                                      \
+  {                                                                                                                 \
+    AGCF_CUDA_OK(cudaFuncSetAttribute(ngcf::dense_fwd_wide_kernel<DD>, cudaFuncAttributeMaxDynamicSharedMemorySize,  \
+                                      (int)ngcf::kWideSmemBytes));                                                  \
+    ngcf::dense_fwd_wide_kernel<DD><<<grid, 256, ngcf::kWideSmemBytes, st>>>(P, E, W, Enext, acc_in, acc_out, acc_div, \
+                                                                             n_rows);                               \
+  }
+    if (d == 256) AGCF_NGCF_FWD_WIDE(256) else AGCF_NGCF_FWD_WIDE(128)
+#undef AGCF_NGCF_FWD_WIDE
+    AGCF_LAUNCH_OK();
+    return AGCF_OK;
+  }
   if (d <= 16) {
     const unsigned small_blocks = (unsigned)((n_rows + ngcf::kSmallTM - 1) / ngcf::kSmallTM);
     if (d == 16) ngcf::dense_fwd_small_kernel<16><<<small_blocks, ngcf::kSmallTM, 0, st>>>(P, E, W, Enext, acc_in, acc_out, acc_div, n_rows);
@@ -395,12 +592,32 @@ extern "C" int agcf_ngcf_dense_backward(const float* dOut, const float* Enext, c
                                         const float* WT, float* dP, float* dEdir, float* dW_partial,
                                         int32_t n_partials, int32_t n_rows, int32_t d, agcf_stream_t stream) {
   if (!dOut || !Enext || !P || !E || !WT || !dP || !dEdir || !dW_partial || n_rows < 0 || n_partials < 1) return AGCF_EINVAL;
-  if (d != 8 && d != 16 && d != 32 && d != 64) return AGCF_EUNSUPPORTED;
+  if (d != 8 && d != 16 && d != 32 && d != 64 && d != 128 && d != 256) return AGCF_EUNSUPPORTED;
   if (!aligned16(dOut) || !aligned16(Enext) || !aligned16(P) || !aligned16(E) || !aligned16(WT) || !aligned16(dP) ||
       !aligned16(dEdir) || !aligned16(dW_partial))
     return AGCF_EINVAL;
   if (dP == dOut || dEdir == dOut || dP == dEdir) return AGCF_EINVAL;
   cudaStream_t st = (cudaStream_t)stream;
+  if (d >= 128) {                       // [dA | dB] over row tiles, then dW split over n_partials row slices
+    const dim3 grid_dz((unsigned)((n_rows + ngcf::kWM - 1) / ngcf::kWM), (unsigned)(d / (ngcf::kWM / 2)));
+    const dim3 grid_w((unsigned)((2 * d / ngcf::kWM) * (d / ngcf::kWM)), (unsigned)n_partials);
+#define AGCF_NGCF_BWD_WIDE(DD)                                                                                       \
+  {                                                                                                                  \
+    AGCF_CUDA_OK(cudaFuncSetAttribute(ngcf::dense_dzwt_wide_kernel<DD>, cudaFuncAttributeMaxDynamicSharedMemorySize,  \
+                                      (int)ngcf::kWideSmemBytes));                                                   \
+    AGCF_CUDA_OK(cudaFuncSetAttribute(ngcf::dense_wgrad_wide_kernel<DD>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+                                      (int)ngcf::kWideSmemBytes));                                                   \
+    if (n_rows > 0)                                                                                                  \
+      ngcf::dense_dzwt_wide_kernel<DD><<<grid_dz, 256, ngcf::kWideSmemBytes, st>>>(dOut, Enext, P, E, WT, dP, dEdir,  \
+                                                                                   n_rows);                          \
+    ngcf::dense_wgrad_wide_kernel<DD><<<grid_w, 256, ngcf::kWideSmemBytes, st>>>(dOut, Enext, P, E, dW_partial,       \
+                                                                                 n_rows);                            \
+  }
+    if (d == 256) AGCF_NGCF_BWD_WIDE(256) else AGCF_NGCF_BWD_WIDE(128)
+#undef AGCF_NGCF_BWD_WIDE
+    AGCF_LAUNCH_OK();
+    return AGCF_OK;
+  }
   if (d <= 16) {
     if (d == 16) ngcf::dense_bwd_small_kernel<16><<<(unsigned)n_partials, ngcf::kSmallTM, 0, st>>>(dOut, Enext, P, E, WT, dP, dEdir, dW_partial, n_rows);
     else ngcf::dense_bwd_small_kernel<8><<<(unsigned)n_partials, ngcf::kSmallTM, 0, st>>>(dOut, Enext, P, E, WT, dP, dEdir, dW_partial, n_rows);
@@ -423,7 +640,7 @@ extern "C" int agcf_ngcf_dense_backward(const float* dOut, const float* Enext, c
 extern "C" int agcf_ngcf_reduce_wgrad(const float* dW_partial, int32_t n_partials, float* dW, int32_t d,
                                       agcf_stream_t stream) {
   if (!dW_partial || !dW || n_partials < 1) return AGCF_EINVAL;
-  if (d != 8 && d != 16 && d != 32 && d != 64) return AGCF_EUNSUPPORTED;
+  if (d != 8 && d != 16 && d != 32 && d != 64 && d != 128 && d != 256) return AGCF_EUNSUPPORTED;
   const int n = 2 * d * d;
   ngcf::reduce_wgrad_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(dW_partial, n_partials, n, dW);
   AGCF_LAUNCH_OK();

@@ -801,20 +801,23 @@ class NGCFEngine(LightGCNEngine):
 
     launches per step: L x (SpMM + dense) + loss fwd/bwd + L x (dense + reduce + SpMM) + W transpose + 2 optimizer."""
 
-    N_PARTIALS = 296          # persistent CTAs of the backward dense kernel (two per SM): rows of the dW partial buffer
+    # rows of the dW partial buffer.  d <= 64: the persistent CTAs of the backward dense kernel (two per SM).  d = 128 and
+    # 256: the row slices of the split-K weight-gradient kernel, whose 2 / 8 output tiles times the slices fill the 148 SMs
+    # once or twice; a partial is a whole 2d x d matrix (512 KB at d = 256), so 296 of them would be 150 MB
+    N_PARTIALS = {8: 296, 16: 296, 32: 296, 64: 296, 128: 74, 256: 37}
 
     def __init__(self, graph, table, W, n_users, lr, reg, batch_size, max_triples, betas=(0.9, 0.999), adam_eps=1e-8):
         n_layers = int(W.shape[0])
         d = table.shape[1]
-        if d not in (8, 16, 32, 64) or tuple(W.shape) != (n_layers, 2 * d, d) or not W.is_contiguous():
-            raise ValueError("NGCFEngine: d in {8, 16, 32, 64} and W packed as [L, 2d, d]")
+        if d not in self.N_PARTIALS or tuple(W.shape) != (n_layers, 2 * d, d) or not W.is_contiguous():
+            raise ValueError("NGCFEngine: d in {8, 16, 32, 64, 128, 256} and W packed as [L, 2d, d]")
         super().__init__(graph, table, n_users, n_layers, lr, reg, batch_size, max_triples, betas=betas, adam_eps=adam_eps,
                          sparse_layers=False)
         f = lambda: torch.empty_like(table)
         self.W = W
         self.Wm, self.Wv, self.dW = torch.zeros_like(W), torch.zeros_like(W), torch.zeros_like(W)
         self.WT = torch.empty((n_layers, d, 2 * d), dtype=torch.float32, device=table.device)
-        self.dW_partial = torch.empty((self.N_PARTIALS, 2 * d * d), dtype=torch.float32, device=table.device)
+        self.dW_partial = torch.empty((self.N_PARTIALS[d], 2 * d * d), dtype=torch.float32, device=table.device)
         self.P = [f() for _ in range(self.L)]            # A E_{k-1}
         self.Ek = [f() for _ in range(self.L)]           # layer outputs E_1 .. E_L
         self.dP, self.dEdir = f(), f()

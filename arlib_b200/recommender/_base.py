@@ -78,44 +78,60 @@ class GraphRecommender(object):
         can stand in for ``optimizer.step()``: it starts from the optimizer's state and writes it back.  Anything
         else (another optimizer class, stale parameters built before a re-``__init__`` -- a reference quirk callers
         rely on, SURVEY.md 8b) returns None and takes the reference-shaped loop."""
+        if len(list(model.parameters())) != 2:
+            return None
+        return GraphRecommender._plain_adam(optimizer, [model.embedding_dict['user_emb'], model.embedding_dict['item_emb']])
+
+    @staticmethod
+    def _fusable_adam_all(optimizer, model):
+        """``_fusable_adam`` for a model with parameters besides the two tables (NGCF's 2L weight matrices): the one
+        param group must hold exactly the set ``model.parameters()``, every one of which the fused engine steps."""
+        return GraphRecommender._plain_adam(optimizer, list(model.parameters()))
+
+    @staticmethod
+    def _plain_adam(optimizer, want):
+        """{lr, betas, eps} of a plain torch.optim.Adam with one param group over exactly the tensors ``want`` whose state
+        is either empty or initialised for all of them at one step count; None for anything else."""
         if type(optimizer) is not torch.optim.Adam or len(optimizer.param_groups) != 1:
             return None
         g = optimizer.param_groups[0]
-        want = [model.embedding_dict['user_emb'], model.embedding_dict['item_emb']]
         params = list(g['params'])
-        if len(params) != 2 or {id(a) for a in params} != {id(b) for b in want} or len(list(model.parameters())) != 2:
+        if len(params) != len(want) or {id(a) for a in params} != {id(b) for b in want}:
             return None
         if g.get('amsgrad') or g.get('weight_decay', 0) != 0 or g.get('maximize') or g.get('differentiable'):
             return None
         if torch.is_tensor(g['lr']) or g.get('decoupled_weight_decay'):
             return None
         steps = [float(optimizer.state[p]['step']) for p in params if len(optimizer.state.get(p, {}))]
-        if len(steps) == 1 or (len(steps) == 2 and steps[0] != steps[1]):
+        if 0 < len(steps) < len(params) or len(set(steps)) > 1:
             return None
         return {"lr": float(g['lr']), "betas": (float(g['betas'][0]), float(g['betas'][1])), "eps": float(g['eps'])}
 
-    @staticmethod
-    def _adam_state_to_engine(optimizer, model, eng, n_users):
-        pu, pi = model.embedding_dict['user_emb'], model.embedding_dict['item_emb']
-        su, si = optimizer.state.get(pu, {}), optimizer.state.get(pi, {})
-        if len(su) and len(si):
-            eng.m[:n_users].copy_(su['exp_avg']); eng.m[n_users:].copy_(si['exp_avg'])
-            eng.v[:n_users].copy_(su['exp_avg_sq']); eng.v[n_users:].copy_(si['exp_avg_sq'])
-            eng.step_dev.fill_(int(float(su['step'])))
+    def _adam_slots(self, model, eng, n_users):
+        """(parameter, the engine's exp_avg of it, the engine's exp_avg_sq of it) for every parameter the engine steps"""
+        return [(model.embedding_dict['user_emb'], eng.m[:n_users], eng.v[:n_users]),
+                (model.embedding_dict['item_emb'], eng.m[n_users:], eng.v[n_users:])]
+
+    def _adam_state_to_engine(self, optimizer, model, eng, n_users):
+        slots = self._adam_slots(model, eng, n_users)
+        states = [optimizer.state.get(p, {}) for p, _, _ in slots]
+        if all(len(st) for st in states):
+            for (_, m, v), st in zip(slots, states):
+                m.copy_(st['exp_avg']); v.copy_(st['exp_avg_sq'])
+            eng.step_dev.fill_(int(float(states[0]['step'])))
             eng._refresh_adam_coefs()
 
-    @staticmethod
-    def _adam_state_from_engine(optimizer, model, eng, n_users):
+    def _adam_state_from_engine(self, optimizer, model, eng, n_users):
         g = optimizer.param_groups[0]
         steps = int(eng.step_dev.item())
-        for p, lo, hi in ((model.embedding_dict['user_emb'], 0, n_users), (model.embedding_dict['item_emb'], n_users, None)):
+        for p, m, v in self._adam_slots(model, eng, n_users):
             st = optimizer.state[p]
             if len(st) == 0:                                  # what torch.optim.Adam._init_group creates lazily
                 on_dev = bool(g.get('capturable') or g.get('fused'))
                 st['step'] = torch.zeros((), dtype=torch.float32, device=p.device) if on_dev else torch.tensor(0.0)
                 st['exp_avg'] = torch.zeros_like(p, memory_format=torch.preserve_format)
                 st['exp_avg_sq'] = torch.zeros_like(p, memory_format=torch.preserve_format)
-            st['exp_avg'].copy_(eng.m[lo:hi]); st['exp_avg_sq'].copy_(eng.v[lo:hi])
+            st['exp_avg'].copy_(m); st['exp_avg_sq'].copy_(v)
             st['step'].fill_(float(steps))
 
     @staticmethod

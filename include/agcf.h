@@ -14,7 +14,7 @@
  *     enqueues work on it and is capturable in a CUDA graph;
  *   - return value: 0 = ok, <0 = AGCF_E* below; nothing throws;
  *   - fp32 everywhere, int32 indices; tables are row-major [rows, d], 16-byte
- *     aligned, d in {8, 16, 32, 64, 128, 256} (the NGCF dense layer: d in {8, 16, 32, 64});
+ *     aligned, d in {8, 16, 32, 64, 128, 256};
  *   - a "node" id is a row of the stacked table [users; items] (N = U + I); item
  *     ids handed to the loss / sampler / eval calls are item-local (0..I-1).
  */
@@ -306,10 +306,11 @@ int agcf_infonce_backward(int32_t n, const int32_t* n_dev, int32_t d, float temp
  *             if acc_out: acc_out = ((acc_in ? acc_in : 0) + Enext) / acc_div   (running layer mean)
  *   backward  dZ = dOut * (Enext > 0 ? 1 : 0.01);  [dA | dB] = dZ W^T  (WT = W transposed, [d, 2d]);
  *             dP = dA + dB * E;  dEdir = dA + dB * P;  dW_partial[b] = this CTA's share of [P + E | P * E]^T dZ
- *             ([n_partials][2d*d]; the launch runs n_partials persistent CTAs);
+ *             ([n_partials][2d*d]; d <= 64: the launch runs n_partials persistent CTAs, d = 128 and 256: the
+ *             weight gradient is split into n_partials row slices, dW_partial[b] the share of slice b);
  *             the gradient of E is then A dP + dEdir (next agcf_spmm_csr_f32, addend = dEdir);
  *   reduce    dW = sum_b dW_partial[b] in b order (deterministic).
- * Uses A (E W1) = (A E) W1: one propagation per layer where the reference runs two.  d in {8, 16, 32, 64}.
+ * Uses A (E W1) = (A E) W1: one propagation per layer where the reference runs two.  d in {8, 16, 32, 64, 128, 256}.
  * Replaces: the loop body of NGCF_Encoder.forward (recommender/NGCF.py:197-212: torch.mm x 2,
  * torch.sparse.mm x 2, leaky_relu, the element-wise product / sums) and its autograd. */
 int agcf_ngcf_dense_forward(const float* P, const float* E, const float* W, float* Enext,

@@ -1,8 +1,13 @@
-"""NGCF at the Gowalla shape (BASELINE configs[1] graph, NGCF encoder of recommender/NGCF.py:197-212, L = 3, d = 64): the
-fused NGCFEngine (one propagation per layer + the fused dense kernels of csrc/ngcf.cu, CUDA-graph replay) against the
+"""NGCF at the Gowalla shape (BASELINE configs[1] graph, NGCF encoder of recommender/NGCF.py:197-212, L = 3): the fused
+NGCFEngine (one propagation per layer + the fused dense kernels of csrc/ngcf.cu, CUDA-graph replay) against the
 reference-shaped loop (torch autograd over the agcf SpMM, torch.mm for the d x d products, torch.optim.Adam) on the same
-graph / parameters.  One JSON line each."""
-import json, os, sys, time
+graph / parameters, in ms per step.  Then the attack pattern at the ml-1M shape: ``NGCF.train(Epoch=1,
+optimizer=torch.optim.Adam(model.parameters()))`` on the drop-in class, fused against the loop (``fused=False``), in
+seconds per call (each call includes the class's end-of-epoch evaluation, on both paths).  One JSON line each, after a
+line with the card's name and power limit.
+
+    python tools/ngcf_bench.py [workload] [--d 64] [--attack-calls 3]"""
+import argparse, contextlib, io, json, os, subprocess, sys, time, types
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, scipy.sparse as sp, torch
 
@@ -11,9 +16,22 @@ from arlib_b200 import ops
 from arlib_b200.engine import DeviceTrainSet, NGCFEngine
 from arlib_b200.graph import DeviceGraph
 
-name = sys.argv[1] if len(sys.argv) > 1 else "gowalla"
+ap = argparse.ArgumentParser()
+ap.add_argument("workload", nargs="?", default="gowalla")
+ap.add_argument("--d", type=int, default=64, choices=sorted(NGCFEngine.N_PARTIALS))
+ap.add_argument("--attack-calls", type=int, default=3, help="timed train(Epoch=1) calls per path at ml-1M; 0 skips the leg")
+cli = ap.parse_args()
+if not torch.cuda.is_available():
+    raise SystemExit("needs a CUDA device")
+try:
+    card = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"],
+                          capture_output=True, text=True, timeout=30).stdout.strip()
+except (OSError, subprocess.SubprocessError):
+    card = ""
+print(json.dumps({"card": card or torch.cuda.get_device_name(0)}), flush=True)
+name = cli.workload
 D = make_data(name, 0.5)
-U, I, E, L, d, B = D["U"], D["I"], D["E"], D["L"], 64, D["B"]
+U, I, E, L, d, B = D["U"], D["I"], D["E"], D["L"], cli.d, D["B"]
 N = U + I
 dev = torch.device("cuda:0")
 half = sp.csr_matrix((np.ones(E, dtype=np.float32), (D["tu"], D["ti"] + U)), shape=(N, N), dtype=np.float32)
@@ -45,7 +63,7 @@ def t(fn, n=50):
     return e0.elapsed_time(e1) / n * 1e3
 fwd_us = t(lambda: ops.ngcf_dense_forward(P, X, W[0], Y))
 dP, dE = torch.empty_like(P), torch.empty_like(P)
-part, dW = torch.empty((296, 2 * d * d), device=dev), torch.empty((2 * d, d), device=dev)
+part, dW = torch.empty((NGCFEngine.N_PARTIALS[d], 2 * d * d), device=dev), torch.empty((2 * d, d), device=dev)
 WT = W[0].t().contiguous()
 bwd_us = t(lambda: ops.ngcf_dense_backward(P, Y, P, X, WT, dP, dE, part, dW))
 spmm_us = t(lambda: ops.spmm(g, X, Y=Y))
@@ -57,7 +75,6 @@ print(json.dumps({"workload": name, "engine": "ngcf-fused", "L": L, "d": d, "ste
                   "spmm_us": spmm_us}), flush=True)
 
 # ---- reference-shaped loop on autograd (what train() runs with a caller's optimizer)
-import types
 from arlib_b200.encoder import spmm_autograd
 from arlib_b200.util.loss import bpr_l2_fused
 import torch.nn.functional as F
@@ -82,5 +99,37 @@ n_ref = 50
 for b in range(5, 5 + n_ref): step(b)
 torch.cuda.synchronize()
 ms_ref = (time.perf_counter() - t0) / n_ref * 1e3
-print(json.dumps({"workload": name, "engine": "ngcf-reference-shaped-loop", "steps_timed": n_ref, "ms_per_step": ms_ref,
+print(json.dumps({"workload": name, "engine": "ngcf-reference-shaped-loop", "L": L, "d": d, "steps_timed": n_ref, "ms_per_step": ms_ref,
                   "triples_per_s": B / (ms_ref * 1e-3)}), flush=True)
+
+# ---- the attack pattern at the ml-1M shape: the caller's Adam handed to train() on the drop-in class
+if cli.attack_calls > 0:
+    from arlib_b200.recommender.NGCF import NGCF
+    from arlib_b200.util.DataLoader import DataLoader
+    from arlib_b200.util.synth import synth_edges
+    del eng, opt
+    torch.cuda.empty_cache()
+    Um, Im, Em, Lm, _, Bm = __import__("bench").WORKLOADS["ml-1m"]
+    tu, ti, su, si = synth_edges(Um, Im, Em, 0.5, 0.5, 0)
+    data = DataLoader.from_arrays(tu, ti, su, si, name="ml-1m")
+    for fused in (True, False):
+        args = types.SimpleNamespace(topK="50", emb_size=d, n_layers=Lm, batch_size=Bm, lRate=0.005, reg=1e-4, maxEpoch=1,
+                                     seed=2018, sampler="device", model_name="NGCF", fused=fused)
+        torch.manual_seed(2018)
+        rec = NGCF(args, data)
+        adam = torch.optim.Adam(rec.model.cuda().parameters(), lr=0.005)
+        on_engine, run_engine = [], rec._train_fused_ngcf
+        rec._train_fused_ngcf = lambda *a, **k: (on_engine.append(1), run_engine(*a, **k))[1]
+        took = []
+        for c in range(cli.attack_calls + 1):                     # the first call warms up (module load, graph plans)
+            torch.cuda.synchronize(); t0 = time.perf_counter()
+            with contextlib.redirect_stdout(io.StringIO()):
+                rec.train(Epoch=1, optimizer=adam)
+            torch.cuda.synchronize(); took.append(time.perf_counter() - t0)
+        st = adam.state[rec.model.embedding_dict["user_emb"]]
+        print(json.dumps({"workload": "ml-1m", "pattern": "train(Epoch=1, optimizer=Adam(model.parameters()))",
+                          "args.fused": fused, "path": "fused" if on_engine else "reference-shaped-loop", "L": Lm, "d": d, "calls_timed": cli.attack_calls,
+                          "s_per_call": float(np.mean(took[1:])), "s_per_call_each": took[1:], "batches_per_call":
+                          (len(data.training_data) + Bm - 1) // Bm, "adam_step_after": float(st["step"])}), flush=True)
+        del rec, adam
+        torch.cuda.empty_cache()
