@@ -1,99 +1,27 @@
 """LightGCN -- drop-in for the reference's recommender/LightGCN.py.
 
-``train()`` has two paths with identical mathematics (SURVEY.md App. A):
-  * fused (optimizer is None, no gradient export): arlib_b200.engine.LightGCNEngine --
-    on-device Philox sampling (or the host sampler for seed-parity), 2L+5 kernels per
-    batch replayed from a CUDA graph, Adam state owned by the engine;
-  * general (caller's optimizer, requires_adjgrad / requires_embgrad): the reference
-    loop on torch autograd, with the encoder forward/backward on the agcf SpMM kernels
-    and ``.grad`` populated on the real nn.Parameters.
+``train()`` (GraphRecommender) runs arlib_b200.engine.LightGCNEngine on its fused path -- 2L+5 kernels per batch
+replayed from a CUDA graph -- and otherwise the reference loop on torch autograd, with the encoder forward/backward on
+the agcf SpMM kernels and ``.grad`` populated on the real nn.Parameters.
 """
-import torch
+import torch  # noqa: F401
 
 from ..encoder import LGCN_Encoder, TorchGraphInterface  # noqa: F401  (re-exported like the reference module)
 from ..engine import LightGCNEngine
 from ..util.loss import bpr_l2_fused, bpr_loss, l2_reg_loss  # noqa: F401
-from ..util.sampler import next_batch_pairwise
+from ..util.sampler import next_batch_pairwise  # noqa: F401
 from ._base import GraphRecommender
 
 
 class LightGCN(GraphRecommender):
     model_name = "LightGCN"
+    PRINT_EVERY = 1000
+    KEEPS_OPTIMIZER = True
 
     def _build_model(self):
         return LGCN_Encoder(self.data, self.args.emb_size, self.args.n_layers)
 
-    def train(self, requires_adjgrad=False, requires_embgrad=False, gradIterationNum=10, Epoch=0, optimizer=None,
-              evalNum=5):
-        self.bestPerformance = []
-        model = self.model.cuda()
-        maxEpoch = Epoch if Epoch else self.args.maxEpoch
-        exports = requires_adjgrad or requires_embgrad
-        adam = self._fusable_adam(optimizer, model) if optimizer is not None and not exports else None
-        if (optimizer is None or adam is not None) and not exports and self._fused_ok():
-            self._train_fused(model, maxEpoch, evalNum, optimizer, adam)
-            self.user_emb, self.item_emb = self.best_user_emb, self.best_item_emb
-            return None
-        if optimizer is None:
-            self.optimizer = torch.optim.Adam(model.parameters(), lr=self.args.lRate)
-        else:
-            self.optimizer = optimizer
-        self._grad_buffers(requires_adjgrad, requires_embgrad, model)
-        dev = model.embedding_dict['user_emb'].device
-        for epoch in range(maxEpoch):
-            for n, batch in enumerate(self._epoch_batches(dev)):
-                user_idx, pos_idx, neg_idx = batch
-                model.train()
-                rec_user_emb, rec_item_emb = model()
-                # the three gathers + bpr_loss + l2_reg_loss(reg, user_emb, pos_item_emb) of the reference, one fused op
-                batch_loss = bpr_l2_fused(rec_user_emb, rec_item_emb, user_idx, pos_idx, neg_idx, self.args.reg)
-                self.optimizer.zero_grad()
-                batch_loss.backward()
-                self._accumulate_grads(requires_adjgrad, requires_embgrad, maxEpoch, epoch, gradIterationNum)
-                self.optimizer.step()
-                if n % 1000 == 0:
-                    print('training:', epoch + 1, 'batch', n, 'batch_loss:', batch_loss.item())
-            model.eval()
-            with torch.no_grad():
-                self.user_emb, self.item_emb = self.model()
-            if epoch % evalNum == 0:
-                self.evaluate(epoch)
-        self.user_emb, self.item_emb = self.best_user_emb, self.best_item_emb
-        return self._train_returns(requires_adjgrad, requires_embgrad)
-
-    # -------------------------------------------------------------- fused path
-    def _train_fused(self, model, maxEpoch, evalNum, optimizer=None, adam=None):
-        """optimizer / adam: the caller's plain torch.optim.Adam over the two embedding parameters (_fusable_adam);
-        the engine starts from its state and hands it back, so the caller can keep stepping it."""
-        table = model.parameter_table()
-        dev = table.device
-        mode = self._sampler_mode()
-        n_edges = len(self.data.training_data)
-        adam = adam or {"lr": self.args.lRate, "betas": (0.9, 0.999), "eps": 1e-8}
-        eng = LightGCNEngine(model._graph, table, self.data.user_num, model.layers, adam["lr"], self.args.reg,
-                             self.args.batch_size, n_edges, betas=adam["betas"], adam_eps=adam["eps"])
-        if optimizer is not None:
-            self._adam_state_to_engine(optimizer, model, eng, self.data.user_num)
-        ts = self._device_train_set(dev) if mode == 'device' else None
-        seed = int(getattr(self.args, 'seed', 0) or 0)
-        for epoch in range(maxEpoch):
-            if mode == 'device':
-                eng.sample_epoch(ts, seed, self._next_sample_epoch())
-            else:                                   # host sampler: the reference's RNG consumption
-                us, is_, js = [], [], []
-                for u, i, j in next_batch_pairwise(self.data, self.args.batch_size):
-                    us += u; is_ += i; js += j
-                eng.set_triples(us, is_, js)
-            losses = eng.run_steps(0, use_graph=self._graph_pays_off(maxEpoch))
-            host = losses[::1000, 0].cpu().tolist()
-            for k, v in enumerate(host):
-                print('training:', epoch + 1, 'batch', k * 1000, 'batch_loss:', v)
-            model.eval()
-            with torch.no_grad():
-                f = eng.forward_table(out=torch.empty_like(table))
-                self.user_emb, self.item_emb = f[:self.data.user_num], f[self.data.user_num:]
-            if epoch % evalNum == 0:
-                self.evaluate(epoch)
-        self.last_train_losses = eng.out4[:eng.n_batches].clone()
-        if optimizer is not None:
-            self._adam_state_from_engine(optimizer, model, eng, self.data.user_num)
+    def _fused_engine(self, model, table, adam, seed):
+        return LightGCNEngine(model._graph, table, self.data.user_num, model.layers, adam["lr"], self.args.reg,
+                              self.args.batch_size, len(self.data.training_data), betas=adam["betas"],
+                              adam_eps=adam["eps"])

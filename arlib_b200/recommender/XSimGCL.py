@@ -1,16 +1,21 @@
 """XSimGCL -- drop-in for the reference's recommender/XSimGCL.py (class :18-95, encoder
 :179-223).  Hard-coded hyper-parameters like the reference (:32-36: 2 layers, cl_rate
 0.2, eps 0.1, layer_cl 1, tau 0.1).  One noise-perturbed propagation per step on
-agcf_spmm_csr_f32 (noise fused into the epilogue, the layer_cl view kept)."""
+agcf_spmm_csr_f32 (noise fused into the epilogue, the layer_cl view kept).  The fused
+path of ``train()`` (GraphRecommender) runs arlib_b200.engine.ContrastiveEngine when
+1 <= layer_cl < n_layers, with the perturbation noise drawn by Philox in the SpMM
+epilogue instead of torch.rand_like."""
 import torch
 
 from ..encoder import TorchGraphInterface, XSimGCL_Encoder, unique_ids_like_reference  # noqa: F401
+from ..engine import ContrastiveEngine
 from ..util.loss import InfoNCE, bpr_l2_fused, bpr_loss, l2_reg_loss  # noqa: F401
 from ._base import GraphRecommender
 
 
 class XSimGCL(GraphRecommender):
     model_name = "XSimGCL"
+    LOSS_LABELS = ('rec_loss:', 'cl_loss')
 
     def _build_model(self):
         self.n_layers = 2
@@ -27,44 +32,22 @@ class XSimGCL(GraphRecommender):
         return InfoNCE(user_view1[u_idx], user_view2[u_idx], self.temp) + \
             InfoNCE(item_view1[i_idx], item_view2[i_idx], self.temp)
 
-    def train(self, requires_adjgrad=False, requires_embgrad=False, gradIterationNum=10, Epoch=0, optimizer=None,
-              evalNum=5):
-        self.bestPerformance = []
-        model = self.model.cuda()
-        maxEpoch = Epoch if Epoch else self.args.maxEpoch
-        exports = requires_adjgrad or requires_embgrad
-        adam = self._fusable_adam(optimizer, model) if optimizer is not None and not exports else None
-        if (optimizer is None or adam is not None) and not exports and self._fused_ok() \
-                and 1 <= self.layer_cl < self.n_layers:
-            self._train_fused_contrastive(model, maxEpoch, evalNum, "xsimgcl", self.layer_cl, optimizer=optimizer, adam=adam)
-            self.user_emb, self.item_emb = self.best_user_emb, self.best_item_emb
-            return None
-        if optimizer is None:
-            optimizer = torch.optim.Adam(model.parameters(), lr=self.args.lRate)
-        self._grad_buffers(requires_adjgrad, requires_embgrad, model)
-        maxEpoch = Epoch if Epoch else self.args.maxEpoch
-        dev = model.embedding_dict['user_emb'].device
-        for epoch in range(maxEpoch):
-            for n, batch in enumerate(self._epoch_batches(dev)):
-                user_idx, pos_idx, neg_idx = batch
-                model.train()
-                rec_user_emb, rec_item_emb, cl_user_emb, cl_item_emb = model(True)
-                rec_l2, parts = bpr_l2_fused(rec_user_emb, rec_item_emb, user_idx, pos_idx, neg_idx, self.args.reg,
-                                             return_parts=True)
-                rec_loss = parts[1]
-                cl_loss = self.cl_rate * self.cal_cl_loss([user_idx, pos_idx], rec_user_emb, cl_user_emb, rec_item_emb,
-                                                          cl_item_emb)
-                batch_loss = rec_l2 + cl_loss
-                optimizer.zero_grad()
-                batch_loss.backward()
-                self._accumulate_grads(requires_adjgrad, requires_embgrad, maxEpoch, epoch, gradIterationNum)
-                optimizer.step()
-                if n % 100 == 0:
-                    print('training:', epoch + 1, 'batch', n, 'rec_loss:', rec_loss.item(), 'cl_loss', cl_loss.item())
-            model.eval()
-            with torch.no_grad():
-                self.user_emb, self.item_emb = self.model()
-            if epoch % evalNum == 0:
-                self.evaluate(epoch)
-        self.user_emb, self.item_emb = self.best_user_emb, self.best_item_emb
-        return self._train_returns(requires_adjgrad, requires_embgrad)
+    def _batch_loss(self, model, user_idx, pos_idx, neg_idx):
+        rec_user_emb, rec_item_emb, cl_user_emb, cl_item_emb = model(True)
+        rec_l2, parts = bpr_l2_fused(rec_user_emb, rec_item_emb, user_idx, pos_idx, neg_idx, self.args.reg,
+                                     return_parts=True)
+        cl_loss = self.cl_rate * self.cal_cl_loss([user_idx, pos_idx], rec_user_emb, cl_user_emb, rec_item_emb,
+                                                  cl_item_emb)
+        return rec_l2 + cl_loss, (parts[1], cl_loss)
+
+    def _engine_accepts(self, model):
+        return 1 <= self.layer_cl < self.n_layers
+
+    def _fused_engine(self, model, table, adam, seed):
+        return ContrastiveEngine(model._graph, table, self.data.user_num, "xsimgcl", self.n_layers, self.eps,
+                                 self.cl_rate, self.temp, adam["lr"], self.args.reg, self.args.batch_size,
+                                 len(self.data.training_data), layer_cl=self.layer_cl,
+                                 noise_seed=self._next_noise_seed(seed), betas=adam["betas"], adam_eps=adam["eps"])
+
+    def _engine_losses(self, eng):
+        return torch.stack(eng.losses(), 1)

@@ -7,6 +7,17 @@ once.  Public surface kept: ``X(args, data)`` (re-callable on a live instance),
 evalNum)``, ``model``, ``user_emb / item_emb / best_user_emb / best_item_emb``,
 ``predict(user) -> np.ndarray``, ``test() -> (rec_list, [str])``, ``evaluate(epoch)``,
 ``save()``, ``data / args / topN / max_N / bestPerformance / recOutput``.
+
+``train()`` is written once here and has two paths with the same mathematics:
+  * fused (no gradient export; the recommender's own optimizer, or the caller's plain torch.optim.Adam over exactly
+    ``model.parameters()``): ``_train_fused`` runs the model's engine from arlib_b200.engine -- on-device Philox
+    sampling (or the host sampler for seed parity), one CUDA-graph replay per epoch, Adam state owned by the engine
+    and handed back to a caller's optimizer;
+  * general (any other optimizer, requires_adjgrad / requires_embgrad): the reference loop on torch autograd, with the
+    propagations on the agcf SpMM kernels and ``.grad`` populated on the real nn.Parameters.
+A model class supplies ``_build_model`` and what differs between the models: the batch loss of the general path
+(``_batch_loss``), its engine (``_fused_engine``, ``_engine_accepts``, ``_engine_losses``) and its print line
+(``LOSS_LABELS``, ``PRINT_EVERY``).
 """
 from __future__ import annotations
 
@@ -17,10 +28,17 @@ import torch
 
 from .. import ops
 from ..evaluator import FullRankEvaluator
+from ..util.loss import bpr_l2_fused
 
 
 class GraphRecommender(object):
     model_name = "GraphRecommender"
+    # the reference's print line of a training batch: the labels of the printed losses, every PRINT_EVERY batches
+    LOSS_LABELS = ('batch_loss:',)
+    PRINT_EVERY = 100
+    # the reference's LightGCN keeps its optimizer as self.optimizer and the others do not; the drop-ins mirror the
+    # reference's attribute set because callers pickle the whole object (ARLib.py:127-131)
+    KEEPS_OPTIMIZER = False
 
     def __init__(self, args, data):
         print("Recommender: " + self.model_name)
@@ -74,28 +92,16 @@ class GraphRecommender(object):
     def _fusable_adam(optimizer, model):
         """The attacks hand ``train()`` their own optimizer (18 call sites, e.g. attack/White/CLeaR.py:145-146), nearly
         always ``torch.optim.Adam(model.parameters(), lr)``.  If it is exactly that -- plain Adam (no amsgrad / weight
-        decay / maximize), ONE param group whose tensors ARE the model's two embedding parameters -- the fused engine
-        can stand in for ``optimizer.step()``: it starts from the optimizer's state and writes it back.  Anything
-        else (another optimizer class, stale parameters built before a re-``__init__`` -- a reference quirk callers
-        rely on, SURVEY.md 8b) returns None and takes the reference-shaped loop."""
-        if len(list(model.parameters())) != 2:
-            return None
-        return GraphRecommender._plain_adam(optimizer, [model.embedding_dict['user_emb'], model.embedding_dict['item_emb']])
-
-    @staticmethod
-    def _fusable_adam_all(optimizer, model):
-        """``_fusable_adam`` for a model with parameters besides the two tables (NGCF's 2L weight matrices): the one
-        param group must hold exactly the set ``model.parameters()``, every one of which the fused engine steps."""
-        return GraphRecommender._plain_adam(optimizer, list(model.parameters()))
-
-    @staticmethod
-    def _plain_adam(optimizer, want):
-        """{lr, betas, eps} of a plain torch.optim.Adam with one param group over exactly the tensors ``want`` whose state
-        is either empty or initialised for all of them at one step count; None for anything else."""
+        decay / maximize), ONE param group whose tensors ARE the set ``model.parameters()`` (the two embedding tables,
+        and NGCF's 2L weight matrices), state either empty or initialised for all of them at one step count -- the fused
+        engine can stand in for ``optimizer.step()``: it starts from the optimizer's state and writes it back; the
+        result is its {lr, betas, eps}.  Anything else (another optimizer class, a subset of the parameters, stale
+        parameters built before a re-``__init__`` -- a reference quirk callers rely on, SURVEY.md 8b) returns None and
+        takes the reference-shaped loop."""
         if type(optimizer) is not torch.optim.Adam or len(optimizer.param_groups) != 1:
             return None
         g = optimizer.param_groups[0]
-        params = list(g['params'])
+        params, want = list(g['params']), list(model.parameters())
         if len(params) != len(want) or {id(a) for a in params} != {id(b) for b in want}:
             return None
         if g.get('amsgrad') or g.get('weight_decay', 0) != 0 or g.get('maximize') or g.get('differentiable'):
@@ -173,8 +179,8 @@ class GraphRecommender(object):
         return cached[1]
 
     def _epoch_batches(self, dev):
-        """The batches of one epoch for the reference-shaped training loops (caller's optimizer, gradient export,
-        NGCF / SimGCL / XSimGCL): ``(user_idx, pos_idx, neg_idx)`` as device LongTensors drawn by the on-device
+        """The batches of one epoch for the reference-shaped training loop (caller's optimizer, gradient export):
+        ``(user_idx, pos_idx, neg_idx)`` as device LongTensors drawn by the on-device
         Philox sampler (agcf_bpr_sample_epoch, util/sampler.py:4-30), or -- sampler mode 'host' -- the reference's
         Python lists from util.sampler.next_batch_pairwise (same RNG consumption, in-place shuffle)."""
         from ..util.sampler import next_batch_pairwise
@@ -256,47 +262,101 @@ class GraphRecommender(object):
         return rec_list, measure
 
     # ------------------------------------------------------------------ training
-    def _train_fused_contrastive(self, model, maxEpoch, evalNum, kind, layer_cl=1, optimizer=None, adam=None):
-        """SimGCL / XSimGCL training when the recommender owns the optimizer and no gradient is exported: the fused
-        engine (arlib_b200.engine.ContrastiveEngine) -- device sampling (or the host sampler for seed parity), one
-        CUDA-graph replay per epoch, Adam state owned by the engine.  Same mathematics as the reference loop
-        (recommender/SimGCL.py:36-85, XSimGCL.py:46-95); the perturbation noise comes from Philox in the SpMM
-        epilogue instead of torch.rand_like."""
-        from ..engine import ContrastiveEngine
+    def train(self, requires_adjgrad=False, requires_embgrad=False, gradIterationNum=10, Epoch=0, optimizer=None,
+              evalNum=5):
+        """The reference's ``train()`` of all four recommenders: the fused engine when nothing is exported and the
+        engine can stand in for the optimizer, otherwise the reference-shaped loop."""
+        self.bestPerformance = []
+        model = self.model.cuda()
+        maxEpoch = Epoch if Epoch else self.args.maxEpoch
+        exports = requires_adjgrad or requires_embgrad
+        adam = self._fusable_adam(optimizer, model) if optimizer is not None and not exports else None
+        if (optimizer is None or adam is not None) and not exports and self._fused_ok() and self._engine_accepts(model):
+            self._train_fused(model, maxEpoch, evalNum, optimizer, adam)
+            self.user_emb, self.item_emb = self.best_user_emb, self.best_item_emb
+            return None
+        if optimizer is None:
+            optimizer = torch.optim.Adam(model.parameters(), lr=self.args.lRate)
+        if self.KEEPS_OPTIMIZER:
+            self.optimizer = optimizer
+        self._grad_buffers(requires_adjgrad, requires_embgrad, model)
+        dev = model.embedding_dict['user_emb'].device
+        for epoch in range(maxEpoch):
+            for n, (user_idx, pos_idx, neg_idx) in enumerate(self._epoch_batches(dev)):
+                model.train()
+                batch_loss, shown = self._batch_loss(model, user_idx, pos_idx, neg_idx)
+                optimizer.zero_grad()
+                batch_loss.backward()
+                self._accumulate_grads(requires_adjgrad, requires_embgrad, maxEpoch, epoch, gradIterationNum)
+                optimizer.step()
+                if n % self.PRINT_EVERY == 0:
+                    self._print_losses(epoch, n, [t.item() for t in shown])
+            model.eval()
+            with torch.no_grad():
+                self.user_emb, self.item_emb = self.model()
+            if epoch % evalNum == 0:
+                self.evaluate(epoch)
+        self.user_emb, self.item_emb = self.best_user_emb, self.best_item_emb
+        return self._train_returns(requires_adjgrad, requires_embgrad)
+
+    def _print_losses(self, epoch, n, values):
+        pairs = [x for label, v in zip(self.LOSS_LABELS, values) for x in (label, v)]
+        print('training:', epoch + 1, 'batch', n, *pairs)
+
+    def _batch_loss(self, model, user_idx, pos_idx, neg_idx):
+        """(loss to backpropagate, the tensors printed under LOSS_LABELS) of one batch of the reference-shaped loop.
+        BPR + L2 of LightGCN and NGCF: the three gathers + bpr_loss + l2_reg_loss(reg, user_emb, pos_item_emb) of the
+        reference, one fused op."""
+        rec_user_emb, rec_item_emb = model()
+        batch_loss = bpr_l2_fused(rec_user_emb, rec_item_emb, user_idx, pos_idx, neg_idx, self.args.reg)
+        return batch_loss, (batch_loss,)
+
+    def _fused_engine(self, model, table, adam, seed):
+        """the model's fused training engine (arlib_b200.engine) over ``table``, with Adam's {lr, betas, eps}"""
+        raise NotImplementedError
+
+    def _engine_accepts(self, model):
+        """whether ``_fused_engine`` can train this model's configuration"""
+        return True
+
+    def _engine_losses(self, eng):
+        """the engine's per-batch losses of the last epoch, [n_batches, k]; the first len(LOSS_LABELS) columns are the
+        printed ones.  Kept as ``last_train_losses``."""
+        return eng.out4[:eng.n_batches]
+
+    def _train_fused(self, model, maxEpoch, evalNum, optimizer=None, adam=None):
+        """train() on the model's fused engine.  optimizer / adam: the caller's plain torch.optim.Adam over
+        model.parameters() (_fusable_adam); the engine starts from its state and hands it back, so the caller can keep
+        stepping it."""
         from ..util.sampler import next_batch_pairwise
         table = model.parameter_table()
         dev = table.device
         seed = int(getattr(self.args, 'seed', 0) or 0)
-        tau = self.temp if kind == "xsimgcl" else 0.2
         adam = adam or {"lr": self.args.lRate, "betas": (0.9, 0.999), "eps": 1e-8}
-        eng = ContrastiveEngine(model._graph, table, self.data.user_num, kind, self.n_layers, self.eps, self.cl_rate, tau,
-                                adam["lr"], self.args.reg, self.args.batch_size, len(self.data.training_data),
-                                layer_cl=layer_cl, noise_seed=self._next_noise_seed(seed),
-                                betas=adam["betas"], adam_eps=adam["eps"])
+        eng = self._fused_engine(model, table, adam, seed)
         if optimizer is not None:
             self._adam_state_to_engine(optimizer, model, eng, self.data.user_num)
         mode = self._sampler_mode()
         ts = self._device_train_set(dev) if mode == 'device' else None
+        every, shown = self.PRINT_EVERY, len(self.LOSS_LABELS)
         for epoch in range(maxEpoch):
             if mode == 'device':
                 eng.sample_epoch(ts, seed, self._next_sample_epoch())
-            else:
+            else:                                   # host sampler: the reference's RNG consumption
                 us, is_, js = [], [], []
                 for u, i, j in next_batch_pairwise(self.data, self.args.batch_size):
                     us += u; is_ += i; js += j
                 eng.set_triples(us, is_, js)
             eng.run_steps(0, use_graph=self._graph_pays_off(maxEpoch))
-            rec, cl = eng.losses()
-            rec, cl = rec[::100].cpu().tolist(), cl[::100].cpu().tolist()
-            for k, (r, c) in enumerate(zip(rec, cl)):
-                print('training:', epoch + 1, 'batch', k * 100, 'rec_loss:', r, 'cl_loss', c)
+            for k, values in enumerate(self._engine_losses(eng)[::every, :shown].cpu().tolist()):
+                self._print_losses(epoch, k * every, values)
             model.eval()
             with torch.no_grad():
                 f = eng.forward_table(out=torch.empty_like(table))
                 self.user_emb, self.item_emb = f[:self.data.user_num], f[self.data.user_num:]
             if epoch % evalNum == 0:
                 self.evaluate(epoch)
-        self.last_train_losses = torch.stack(eng.losses(), 1).clone()
+        self.last_train_losses = self._engine_losses(eng).clone()
         if optimizer is not None:
             self._adam_state_from_engine(optimizer, model, eng, self.data.user_num)
 

@@ -212,8 +212,8 @@ def test_wide_engine_steps_match_fp64_steps(golden, golden_rows, d):
 def _spy(monkeypatch):
     from arlib_b200.recommender.NGCF import NGCF
     calls = []
-    orig = NGCF._train_fused_ngcf
-    monkeypatch.setattr(NGCF, "_train_fused_ngcf", lambda self, *a, **k: (calls.append(self), orig(self, *a, **k))[1])
+    orig = NGCF._train_fused
+    monkeypatch.setattr(NGCF, "_train_fused", lambda self, *a, **k: (calls.append(self), orig(self, *a, **k))[1])
     return calls
 
 
@@ -227,12 +227,11 @@ def _pairs(rec, tr):
 
 
 @pytest.mark.parametrize("d", ALL_WIDTHS)
-def test_callers_adam_drives_the_fused_engine(golden, golden_rows, monkeypatch, d):
+def test_callers_adam_drives_the_unified_fused_loop(golden, golden_rows, monkeypatch, d):
     """attack/White/CLeaR.py:145-146 on an NGCF victim: ``train(Epoch=1, optimizer=torch.optim.Adam(model.parameters(),
     ...))`` runs on the fused engine with the optimizer's lr / betas / eps, ends one epoch within the float64 oracle's
     rule, and hands every parameter's Adam state back: a second call continues it, and the caller's own step after that
     works.  Only one epoch is compared: NGCF parameters after many steps are not well conditioned (test_gpu_ngcf.py)."""
-    from arlib_b200.recommender.NGCF import FUSED_WIDTHS
     calls = _spy(monkeypatch)
     rec = _rec("NGCF", golden_rows, d)
     m = rec.model
@@ -245,7 +244,7 @@ def test_callers_adam_drives_the_fused_engine(golden, golden_rows, monkeypatch, 
     for b in _batches(golden):
         tr.step(*b)
     rec.train(Epoch=1, optimizer=opt)
-    assert calls == ([rec] if d in FUSED_WIDTHS else [])
+    assert calls == [rec]
     e = m.embedding_dict
     _assert_close_to_fp64(e["user_emb"].detach(), e["item_emb"].detach(), tr.user_emb.detach(), tr.item_emb.detach(),
                           "NGCF d=%d caller's Adam, tables" % d)
@@ -259,7 +258,7 @@ def test_callers_adam_drives_the_fused_engine(golden, golden_rows, monkeypatch, 
         assert float(st["step"]) == n_batches
         assert _rel(st["exp_avg"], so["exp_avg"]) < 1e-3, _rel(st["exp_avg"], so["exp_avg"])
     rec.train(Epoch=1, optimizer=opt)                      # continues from the handed-back state
-    assert len(calls) == (2 if d in FUSED_WIDTHS else 0)
+    assert len(calls) == 2
     assert all(float(opt.state[p]["step"]) == 2 * n_batches for p, _ in pairs)
     assert all(p is q for p, q in zip(opt.param_groups[0]["params"], m.parameters()))
     fu, fi = m()                                           # the caller keeps using its optimizer
@@ -269,7 +268,7 @@ def test_callers_adam_drives_the_fused_engine(golden, golden_rows, monkeypatch, 
 
 
 @pytest.mark.parametrize("d", [64, 256])
-def test_other_optimizers_keep_the_loop(golden_rows, monkeypatch, d):
+def test_other_optimizers_keep_the_reference_shaped_loop(golden_rows, monkeypatch, d):
     """a stale optimizer (built on tensors that are not the model's, as PGA.py:59-67 does), SGD, or Adam over the two
     tables only: the reference-shaped loop, which steps exactly what the optimizer holds"""
     calls = _spy(monkeypatch)
@@ -289,7 +288,7 @@ def test_other_optimizers_keep_the_loop(golden_rows, monkeypatch, d):
     assert all(p is not m.W["w1_0"] for p in tables.state)
 
 
-def test_deepcopy_then_callers_adam_repacks_the_weights(golden_rows, monkeypatch):
+def test_deepcopy_then_callers_adam_repacks_the_weights_on_the_engine(golden_rows, monkeypatch):
     """a deepcopy un-packs the weight views; the fused path re-packs them (weight_table) and the optimizer's parameter
     objects stay the model's, so the trained values and the handed-back state are on them"""
     calls = _spy(monkeypatch)

@@ -100,7 +100,7 @@ def test_fusable_adam_recognises_exactly_the_plain_optimizer_over_the_models_par
                 torch.optim.Adam([{'params': [m.embedding_dict['user_emb']]}, {'params': [m.embedding_dict['item_emb']]}], lr=0.1),
                 torch.optim.Adam([torch.nn.Parameter(torch.zeros(3, 4)), torch.nn.Parameter(torch.zeros(5, 4))], lr=0.1)):  # stale
         assert f(bad, m) is None, type(bad).__name__
-    # a model with extra parameters (NGCF's weight matrices) is not the two-table case
+    # the two tables alone are not all parameters of a model with more (NGCF's weight matrices)
     m2 = torch.nn.Module()
     m2.embedding_dict = m.embedding_dict
     m2.W = torch.nn.Parameter(torch.zeros(4, 4))

@@ -1,4 +1,4 @@
-"""NGCF's caller's-Adam recogniser (GraphRecommender._fusable_adam_all) and the state handover between a
+"""NGCF's caller's-Adam recogniser (GraphRecommender._fusable_adam) and the state handover between a
 torch.optim.Adam over all 2 + 2L parameters and the fused engine's packed moments, on CPU tensors."""
 import torch
 
@@ -16,9 +16,9 @@ def _ngcf_like(d=4, L=2, n_users=3, n_items=5):
     return m
 
 
-def test_recogniser_accepts_exactly_plain_adam_over_all_parameters():
+def test_single_recogniser_accepts_exactly_plain_adam_over_all_parameters():
     from arlib_b200.recommender._base import GraphRecommender
-    f = GraphRecommender._fusable_adam_all
+    f = GraphRecommender._fusable_adam
     m = _ngcf_like()
     got = f(torch.optim.Adam(m.parameters(), lr=0.003, betas=(0.8, 0.99), eps=1e-7), m)
     assert got == {"lr": 0.003, "betas": (0.8, 0.99), "eps": 1e-7}
@@ -47,9 +47,6 @@ def test_recogniser_accepts_exactly_plain_adam_over_all_parameters():
     for p in m.parameters():
         opt.state[p] = {'step': torch.tensor(7.0), 'exp_avg': torch.zeros_like(p), 'exp_avg_sq': torch.zeros_like(p)}
     assert f(opt, m) is not None
-    # the two-table recogniser keeps refusing a model with more parameters than the tables
-    assert GraphRecommender._fusable_adam(torch.optim.Adam(m.parameters(), lr=0.1), m) is None
-    assert GraphRecommender._fusable_adam(torch.optim.Adam(tables, lr=0.1), m) is None
 
 
 class _FakeEngine:
