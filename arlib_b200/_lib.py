@@ -78,6 +78,9 @@ SIGNATURES = {
     "agcf_ngcf_dense_forward": (c_int32, [P, P, P, P, P, P, F32, I32, I32, P]),
     "agcf_ngcf_dense_backward": (c_int32, [P, P, P, P, P, P, P, P, I32, I32, I32, P]),
     "agcf_ngcf_reduce_wgrad": (c_int32, [P, I32, P, I32, P]),
+    "agcf_ngcf_dense_forward_peers": (c_int32, [P, P, P, P, P, P, F32, I32, I32, P, P, I32, P, P, P]),
+    "agcf_ngcf_dense_backward_peers": (c_int32, [P, P, P, P, P, P, P, P, I32, I32, I32, P, I32, P, P]),
+    "agcf_ngcf_reduce_wgrad_peers": (c_int32, [P, I32, P, I32, P, I32, P, P]),
     "agcf_adam_step_f32": (c_int32, [P, P, P, P, I64, F32, F32, F32, F32, I32, P, P, I32, P, P]),
     "agcf_increment_i32": (c_int32, [P, P]),
     "agcf_score_topk_ws_bytes": (c_int64, [I32, I32, I32, I32]),

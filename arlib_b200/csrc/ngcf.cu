@@ -29,6 +29,49 @@ constexpr int kTM = 64;        // rows per tile
 constexpr int kKC = 64;        // k chunk staged in shared memory
 constexpr float kSlope = 0.01f;
 
+// Where a row-partitioned launch (one rank's rows of the multi-GPU layout) also stores an output: the other ranks'
+// copies (n device pointers over NVLink) or, when mc is set, one NVSwitch multicast address that reaches every copy.
+// Both are offset to the launch's first row like the local pointer, so a row has the same index in all of them.
+// Kernels take it under the compile-time flag PEERS: with PEERS false the argument is never read.
+struct RowPeers {
+  int n;
+  float* p[AGCF_MAX_PEERS];
+  float* mc;
+};
+
+// v[0 .. N) -> element `at` of every peer copy (at is a multiple of min(N, 4)); visible there after a barrier
+template <int N>
+__device__ __forceinline__ void store_peers(const RowPeers& pr, size_t at, const float (&v)[N]) {
+  if (pr.mc != nullptr) {
+    if constexpr (N % 4 == 0) {
+#pragma unroll
+      for (int i = 0; i < N; i += 4)
+        st_multicast_f4(reinterpret_cast<float4*>(pr.mc + at + i), make_float4(v[i], v[i + 1], v[i + 2], v[i + 3]));
+    } else if constexpr (N == 2) {
+      asm volatile("multimem.st.weak.global.v2.f32 [%0], {%1,%2};" :: "l"(pr.mc + at), "f"(v[0]), "f"(v[1]) : "memory");
+    } else {
+#pragma unroll
+      for (int i = 0; i < N; ++i)
+        asm volatile("multimem.st.weak.global.f32 [%0], %1;" :: "l"(pr.mc + at + i), "f"(v[i]) : "memory");
+    }
+    return;
+  }
+#pragma unroll
+  for (int q = 0; q < AGCF_MAX_PEERS; ++q) {        // static indices: the pointer array stays in the parameter bank
+    if (q >= pr.n) break;
+    if constexpr (N % 4 == 0) {
+#pragma unroll
+      for (int i = 0; i < N; i += 4)
+        *reinterpret_cast<float4*>(pr.p[q] + at + i) = make_float4(v[i], v[i + 1], v[i + 2], v[i + 3]);
+    } else if constexpr (N == 2) {
+      *reinterpret_cast<float2*>(pr.p[q] + at) = make_float2(v[0], v[1]);
+    } else {
+#pragma unroll
+      for (int i = 0; i < N; ++i) pr.p[q][at + i] = v[i];
+    }
+  }
+}
+
 template <int CN>
 __device__ __forceinline__ void load_cols(const float* __restrict__ src, float (&w)[CN]) {
   if constexpr (CN == 2) {
@@ -67,11 +110,11 @@ __device__ __forceinline__ void tile_mac(const float (*As)[kKC + 4], const float
 }
 
 // ---------------------------------------------------------------------------- forward
-template <int D>
+template <int D, bool PEERS>
 __global__ void __launch_bounds__(256) dense_fwd_kernel(const float* __restrict__ P, const float* __restrict__ E,
                                                         const float* __restrict__ W, float* __restrict__ Enext,
                                                         const float* __restrict__ acc_in, float* __restrict__ acc_out,
-                                                        float acc_div, int N) {
+                                                        float acc_div, int N, RowPeers peer_next, RowPeers peer_acc) {
   constexpr int CN = D / 16;                       // output columns per thread
   __shared__ __align__(16) float As[kTM][kKC + 4];
   __shared__ __align__(16) float Ws[kKC * D];
@@ -108,16 +151,23 @@ __global__ void __launch_bounds__(256) dense_fwd_kernel(const float* __restrict_
     const int row = row0 + ty * 4 + r;
     if (row >= N) continue;
     const size_t at = (size_t)row * D + tx * CN;
+    float ov[CN], mv[CN];                                            // the stored values, for the peer stores
 #pragma unroll
     for (int c = 0; c < CN; ++c) {
       const float z = acc[r][c];
       const float o = z > 0.f ? z : kSlope * z;                      // F.leaky_relu(z, 0.01)
       Enext[at + c] = o;
+      ov[c] = o;
       if (acc_out != nullptr) {
         float m = (acc_in != nullptr ? acc_in[at + c] : 0.f) + o;
         if (acc_div != 1.0f) m = __fdiv_rn(m, acc_div);
         acc_out[at + c] = m;
+        mv[c] = m;
       }
+    }
+    if constexpr (PEERS) {
+      store_peers<CN>(peer_next, at, ov);
+      if (acc_out != nullptr) store_peers<CN>(peer_acc, at, mv);
     }
   }
 }
@@ -129,11 +179,12 @@ struct BwdSmem {
   static constexpr size_t bytes = (size_t)(3 * kTM * LD + kKC * D) * 4 + (size_t)kTM * (kKC + 4) * 4;
 };
 
-template <int D>
+template <int D, bool PEERS>
 __global__ void __launch_bounds__(256, 2) dense_bwd_kernel(const float* __restrict__ dOut, const float* __restrict__ Enext,
                                                            const float* __restrict__ P, const float* __restrict__ E,
                                                            const float* __restrict__ WT, float* __restrict__ dP,
-                                                           float* __restrict__ dEdir, float* __restrict__ dWpart, int N) {
+                                                           float* __restrict__ dEdir, float* __restrict__ dWpart, int N,
+                                                           RowPeers peer_dP) {
   constexpr int CN = D / 16, LD = D + 4;
   constexpr int JW = 2 * D / 16, CW = D / 16;       // weight-gradient block of a thread: JW rows of dW x CW columns
   extern __shared__ __align__(16) unsigned char bwd_smem[];
@@ -201,13 +252,16 @@ __global__ void __launch_bounds__(256, 2) dense_bwd_kernel(const float* __restri
     for (int r = 0; r < 4; ++r) {
       const int lr = ty * 4 + r, row = row0 + lr;
       if (row >= N) continue;
+      float pv[CN];
 #pragma unroll
       for (int c = 0; c < CN; ++c) {
         const int col = tx * CN + c;
         const float e = Es[lr * LD + col], p = Ps[lr * LD + col];
-        dP[(size_t)row * D + col] = fmaf(accB[r][c], e, accA[r][c]);
+        pv[c] = fmaf(accB[r][c], e, accA[r][c]);
+        dP[(size_t)row * D + col] = pv[c];
         dEdir[(size_t)row * D + col] = fmaf(accB[r][c], p, accA[r][c]);
       }
+      if constexpr (PEERS) store_peers<CN>(peer_dP, (size_t)row * D + tx * CN, pv);
     }
     // dW[j'][c] += sum_n A'[n][j'] dZ[n][c]   with A' = [P + E | P * E] formed from the staged rows
     const int j0 = jy * JW, part = j0 / D, col0 = j0 - part * D;     // JW consecutive rows of dW stay inside one part
@@ -254,11 +308,12 @@ __device__ __forceinline__ void load_row(const float* __restrict__ src, size_t r
   }
 }
 
-template <int D>
+template <int D, bool PEERS>
 __global__ void __launch_bounds__(kSmallTM) dense_fwd_small_kernel(const float* __restrict__ P, const float* __restrict__ E,
                                                                    const float* __restrict__ W, float* __restrict__ Enext,
                                                                    const float* __restrict__ acc_in, float* __restrict__ acc_out,
-                                                                   float acc_div, int N) {
+                                                                   float acc_div, int N, RowPeers peer_next,
+                                                                   RowPeers peer_acc) {
   __shared__ __align__(16) float Ws[2 * D * D];
   for (int f = threadIdx.x; f < 2 * D * D; f += kSmallTM) Ws[f] = __ldg(W + f);
   __syncthreads();
@@ -276,24 +331,32 @@ __global__ void __launch_bounds__(kSmallTM) dense_fwd_small_kernel(const float* 
     for (int c = 0; c < D; ++c) acc[c] = fmaf(a, Ws[k * D + c], acc[c]);
   }
   const size_t at = (size_t)row * D;
+  float ov[D], mv[D];                                                // the stored values, for the peer stores
 #pragma unroll
   for (int c = 0; c < D; ++c) {
     const float z = acc[c];
     const float o = z > 0.f ? z : kSlope * z;                        // F.leaky_relu(z, 0.01)
     Enext[at + c] = o;
+    ov[c] = o;
     if (acc_out != nullptr) {
       float m = (acc_in != nullptr ? acc_in[at + c] : 0.f) + o;
       if (acc_div != 1.0f) m = __fdiv_rn(m, acc_div);
       acc_out[at + c] = m;
+      mv[c] = m;
     }
+  }
+  if constexpr (PEERS) {
+    store_peers<D>(peer_next, at, ov);
+    if (acc_out != nullptr) store_peers<D>(peer_acc, at, mv);
   }
 }
 
-template <int D>
+template <int D, bool PEERS>
 __global__ void __launch_bounds__(kSmallTM) dense_bwd_small_kernel(const float* __restrict__ dOut, const float* __restrict__ Enext,
                                                                    const float* __restrict__ P, const float* __restrict__ E,
                                                                    const float* __restrict__ WT, float* __restrict__ dP,
-                                                                   float* __restrict__ dEdir, float* __restrict__ dWpart, int N) {
+                                                                   float* __restrict__ dEdir, float* __restrict__ dWpart, int N,
+                                                                   RowPeers peer_dP) {
   constexpr int NW = 2 * D * D, WPT = NW / kSmallTM;                // dW entries, and per thread in the reduction (1 or 4)
   __shared__ __align__(16) float WTs[NW];                            // W^T: [D][2D]
   __shared__ float As[kSmallTM][2 * D + 1];                          // [P + E | P * E] of the tile's rows (+1: odd stride)
@@ -329,14 +392,17 @@ __global__ void __launch_bounds__(kSmallTM) dense_bwd_small_kernel(const float* 
           dB[j] = fmaf(z[k], WTs[k * 2 * D + D + j], dB[j]);
         }
       const size_t at = (size_t)row * D;
+      float pv[D];
 #pragma unroll
       for (int j = 0; j < D; ++j) {
-        dP[at + j] = fmaf(dB[j], e[j], dA[j]);
+        pv[j] = fmaf(dB[j], e[j], dA[j]);
+        dP[at + j] = pv[j];
         dEdir[at + j] = fmaf(dB[j], p[j], dA[j]);
         As[lr][j] = p[j] + e[j];
         As[lr][D + j] = p[j] * e[j];
         Zs[lr][j] = z[j];
       }
+      if constexpr (PEERS) store_peers<D>(peer_dP, at, pv);
     } else {
 #pragma unroll
       for (int j = 0; j < D; ++j) { As[lr][j] = 0.f; As[lr][D + j] = 0.f; Zs[lr][j] = 0.f; }
@@ -377,11 +443,11 @@ __device__ __forceinline__ float4 dz_of(float4 g, float4 y) {        // dZ = dE'
                      y.z > 0.f ? g.z : kSlope * g.z, y.w > 0.f ? g.w : kSlope * g.w);
 }
 
-template <int D>
+template <int D, bool PEERS>
 __global__ void __launch_bounds__(256) dense_fwd_wide_kernel(const float* __restrict__ P, const float* __restrict__ E,
                                                              const float* __restrict__ W, float* __restrict__ Enext,
                                                              const float* __restrict__ acc_in, float* __restrict__ acc_out,
-                                                             float acc_div, int N) {
+                                                             float acc_div, int N, RowPeers peer_next, RowPeers peer_acc) {
   extern __shared__ __align__(16) unsigned char wide_smem[];
   float (*As)[kKC + 4] = reinterpret_cast<float (*)[kKC + 4]>(wide_smem);   // [WM][KC + 4]: A' chunk
   float* Ws = reinterpret_cast<float*>(wide_smem) + kWM * (kKC + 4);         // [KC][WM]: W chunk of the column block
@@ -418,25 +484,32 @@ __global__ void __launch_bounds__(256) dense_fwd_wide_kernel(const float* __rest
     const int row = row0 + ty * kWR + r;
     if (row >= N) continue;
     const size_t at = (size_t)row * D + c0 + tx * kWR;
+    float ov[kWR], mv[kWR];                                          // the stored values, for the peer stores
 #pragma unroll
     for (int c = 0; c < kWR; ++c) {
       const float z = acc[r][c];
       const float o = z > 0.f ? z : kSlope * z;                      // F.leaky_relu(z, 0.01)
       Enext[at + c] = o;
+      ov[c] = o;
       if (acc_out != nullptr) {
         float m = (acc_in != nullptr ? acc_in[at + c] : 0.f) + o;
         if (acc_div != 1.0f) m = __fdiv_rn(m, acc_div);
         acc_out[at + c] = m;
+        mv[c] = m;
       }
+    }
+    if constexpr (PEERS) {
+      store_peers<kWR>(peer_next, at, ov);
+      if (acc_out != nullptr) store_peers<kWR>(peer_acc, at, mv);
     }
   }
 }
 
-template <int D>
+template <int D, bool PEERS>
 __global__ void __launch_bounds__(256) dense_dzwt_wide_kernel(const float* __restrict__ dOut, const float* __restrict__ Enext,
                                                               const float* __restrict__ P, const float* __restrict__ E,
                                                               const float* __restrict__ WT, float* __restrict__ dP,
-                                                              float* __restrict__ dEdir, int N) {
+                                                              float* __restrict__ dEdir, int N, RowPeers peer_dP) {
   extern __shared__ __align__(16) unsigned char wide_smem[];
   float (*As)[kKC + 4] = reinterpret_cast<float (*)[kKC + 4]>(wide_smem);   // [WM][KC + 4]: dZ chunk
   float* Bs = reinterpret_cast<float*>(wide_smem) + kWM * (kKC + 4);         // [KC][WM]: Bs[k][2j + h] = W^T[k][h D + j0 + j]
@@ -476,8 +549,13 @@ __global__ void __launch_bounds__(256) dense_dzwt_wide_kernel(const float* __res
     if (row >= N) continue;
     const size_t at = (size_t)row * D + j0 + 4 * tx;
     const float4 e = __ldg(reinterpret_cast<const float4*>(E + at)), p = __ldg(reinterpret_cast<const float4*>(P + at));
-    *reinterpret_cast<float4*>(dP + at) = make_float4(fmaf(acc[r][1], e.x, acc[r][0]), fmaf(acc[r][3], e.y, acc[r][2]),
-                                                      fmaf(acc[r][5], e.z, acc[r][4]), fmaf(acc[r][7], e.w, acc[r][6]));
+    const float4 g = make_float4(fmaf(acc[r][1], e.x, acc[r][0]), fmaf(acc[r][3], e.y, acc[r][2]),
+                                 fmaf(acc[r][5], e.z, acc[r][4]), fmaf(acc[r][7], e.w, acc[r][6]));
+    *reinterpret_cast<float4*>(dP + at) = g;
+    if constexpr (PEERS) {
+      const float pv[4] = {g.x, g.y, g.z, g.w};
+      store_peers<4>(peer_dP, at, pv);
+    }
     *reinterpret_cast<float4*>(dEdir + at) = make_float4(fmaf(acc[r][1], p.x, acc[r][0]), fmaf(acc[r][3], p.y, acc[r][2]),
                                                          fmaf(acc[r][5], p.z, acc[r][4]), fmaf(acc[r][7], p.w, acc[r][6]));
   }
@@ -538,12 +616,18 @@ __global__ void __launch_bounds__(256) dense_wgrad_wide_kernel(const float* __re
   }
 }
 
-__global__ void __launch_bounds__(256) reduce_wgrad_kernel(const float* __restrict__ part, int n_part, int n, float* __restrict__ dW) {
+template <bool PEERS>
+__global__ void __launch_bounds__(256) reduce_wgrad_kernel(const float* __restrict__ part, int n_part, int n, float* __restrict__ dW,
+                                                           RowPeers peer_dW) {
   const int k = blockIdx.x * 256 + threadIdx.x;
   if (k >= n) return;
   float s = 0.f;
   for (int b = 0; b < n_part; ++b) s += part[(size_t)b * n + k];      // CTA (d >= 128: slice) order: deterministic
   dW[k] = s;
+  if constexpr (PEERS) {
+    const float sv[1] = {s};
+    store_peers<1>(peer_dW, (size_t)k, sv);
+  }
 }
 
 }  // namespace ngcf
@@ -551,23 +635,38 @@ __global__ void __launch_bounds__(256) reduce_wgrad_kernel(const float* __restri
 
 using namespace agcf;
 
-extern "C" int agcf_ngcf_dense_forward(const float* P, const float* E, const float* W, float* Enext,
-                                       const float* acc_in, float* acc_out, float acc_div,
-                                       int32_t n_rows, int32_t d, agcf_stream_t stream) {
+namespace {
+
+// host arrays of peer pointers (+ multicast address) -> the kernel argument; false on a malformed list
+bool make_peers(void* const* host, int32_t n_peers, void* mc, ngcf::RowPeers& out) {
+  out = ngcf::RowPeers{};
+  out.mc = reinterpret_cast<float*>(mc);
+  if (mc != nullptr) return aligned16(mc);
+  if (host == nullptr) return true;
+  for (int q = 0; q < n_peers; ++q) {
+    if (host[q] == nullptr || !aligned16(host[q])) return false;
+    out.p[q] = reinterpret_cast<float*>(host[q]);
+  }
+  out.n = n_peers;
+  return true;
+}
+
+template <bool PEERS>
+int dense_forward(const float* P, const float* E, const float* W, float* Enext, const float* acc_in, float* acc_out,
+                  float acc_div, int32_t n_rows, int32_t d, ngcf::RowPeers pn, ngcf::RowPeers pa, cudaStream_t st) {
   if (!P || !E || !W || !Enext || n_rows < 0 || acc_div == 0.f) return AGCF_EINVAL;
   if (d != 8 && d != 16 && d != 32 && d != 64 && d != 128 && d != 256) return AGCF_EUNSUPPORTED;
   if (!aligned16(P) || !aligned16(E) || !aligned16(W) || !aligned16(Enext) || !aligned16(acc_in) || !aligned16(acc_out)) return AGCF_EINVAL;
   if (Enext == P || Enext == E) return AGCF_EINVAL;
   if (n_rows == 0) return AGCF_OK;
-  cudaStream_t st = (cudaStream_t)stream;
   if (d >= 128) {
     const dim3 grid((unsigned)((n_rows + ngcf::kWM - 1) / ngcf::kWM), (unsigned)(d / ngcf::kWM));
 #define AGCF_NGCF_FWD_WIDE(DD)                                                                                      \
   {                                                                                                                 \
-    AGCF_CUDA_OK(cudaFuncSetAttribute(ngcf::dense_fwd_wide_kernel<DD>, cudaFuncAttributeMaxDynamicSharedMemorySize,  \
-                                      (int)ngcf::kWideSmemBytes));                                                  \
-    ngcf::dense_fwd_wide_kernel<DD><<<grid, 256, ngcf::kWideSmemBytes, st>>>(P, E, W, Enext, acc_in, acc_out, acc_div, \
-                                                                             n_rows);                               \
+    AGCF_CUDA_OK(cudaFuncSetAttribute(ngcf::dense_fwd_wide_kernel<DD, PEERS>,                                       \
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ngcf::kWideSmemBytes));     \
+    ngcf::dense_fwd_wide_kernel<DD, PEERS><<<grid, 256, ngcf::kWideSmemBytes, st>>>(P, E, W, Enext, acc_in, acc_out, \
+                                                                                    acc_div, n_rows, pn, pa);       \
   }
     if (d == 256) AGCF_NGCF_FWD_WIDE(256) else AGCF_NGCF_FWD_WIDE(128)
 #undef AGCF_NGCF_FWD_WIDE
@@ -576,40 +675,40 @@ extern "C" int agcf_ngcf_dense_forward(const float* P, const float* E, const flo
   }
   if (d <= 16) {
     const unsigned small_blocks = (unsigned)((n_rows + ngcf::kSmallTM - 1) / ngcf::kSmallTM);
-    if (d == 16) ngcf::dense_fwd_small_kernel<16><<<small_blocks, ngcf::kSmallTM, 0, st>>>(P, E, W, Enext, acc_in, acc_out, acc_div, n_rows);
-    else ngcf::dense_fwd_small_kernel<8><<<small_blocks, ngcf::kSmallTM, 0, st>>>(P, E, W, Enext, acc_in, acc_out, acc_div, n_rows);
+    if (d == 16) ngcf::dense_fwd_small_kernel<16, PEERS><<<small_blocks, ngcf::kSmallTM, 0, st>>>(P, E, W, Enext, acc_in, acc_out, acc_div, n_rows, pn, pa);
+    else ngcf::dense_fwd_small_kernel<8, PEERS><<<small_blocks, ngcf::kSmallTM, 0, st>>>(P, E, W, Enext, acc_in, acc_out, acc_div, n_rows, pn, pa);
     AGCF_LAUNCH_OK();
     return AGCF_OK;
   }
   const unsigned blocks = (unsigned)((n_rows + ngcf::kTM - 1) / ngcf::kTM);
-  if (d == 64) ngcf::dense_fwd_kernel<64><<<blocks, 256, 0, st>>>(P, E, W, Enext, acc_in, acc_out, acc_div, n_rows);
-  else ngcf::dense_fwd_kernel<32><<<blocks, 256, 0, st>>>(P, E, W, Enext, acc_in, acc_out, acc_div, n_rows);
+  if (d == 64) ngcf::dense_fwd_kernel<64, PEERS><<<blocks, 256, 0, st>>>(P, E, W, Enext, acc_in, acc_out, acc_div, n_rows, pn, pa);
+  else ngcf::dense_fwd_kernel<32, PEERS><<<blocks, 256, 0, st>>>(P, E, W, Enext, acc_in, acc_out, acc_div, n_rows, pn, pa);
   AGCF_LAUNCH_OK();
   return AGCF_OK;
 }
 
-extern "C" int agcf_ngcf_dense_backward(const float* dOut, const float* Enext, const float* P, const float* E,
-                                        const float* WT, float* dP, float* dEdir, float* dW_partial,
-                                        int32_t n_partials, int32_t n_rows, int32_t d, agcf_stream_t stream) {
+template <bool PEERS>
+int dense_backward(const float* dOut, const float* Enext, const float* P, const float* E, const float* WT, float* dP,
+                   float* dEdir, float* dW_partial, int32_t n_partials, int32_t n_rows, int32_t d, ngcf::RowPeers pp,
+                   cudaStream_t st) {
   if (!dOut || !Enext || !P || !E || !WT || !dP || !dEdir || !dW_partial || n_rows < 0 || n_partials < 1) return AGCF_EINVAL;
   if (d != 8 && d != 16 && d != 32 && d != 64 && d != 128 && d != 256) return AGCF_EUNSUPPORTED;
   if (!aligned16(dOut) || !aligned16(Enext) || !aligned16(P) || !aligned16(E) || !aligned16(WT) || !aligned16(dP) ||
       !aligned16(dEdir) || !aligned16(dW_partial))
     return AGCF_EINVAL;
   if (dP == dOut || dEdir == dOut || dP == dEdir) return AGCF_EINVAL;
-  cudaStream_t st = (cudaStream_t)stream;
   if (d >= 128) {                       // [dA | dB] over row tiles, then dW split over n_partials row slices
     const dim3 grid_dz((unsigned)((n_rows + ngcf::kWM - 1) / ngcf::kWM), (unsigned)(d / (ngcf::kWM / 2)));
     const dim3 grid_w((unsigned)((2 * d / ngcf::kWM) * (d / ngcf::kWM)), (unsigned)n_partials);
 #define AGCF_NGCF_BWD_WIDE(DD)                                                                                       \
   {                                                                                                                  \
-    AGCF_CUDA_OK(cudaFuncSetAttribute(ngcf::dense_dzwt_wide_kernel<DD>, cudaFuncAttributeMaxDynamicSharedMemorySize,  \
-                                      (int)ngcf::kWideSmemBytes));                                                   \
+    AGCF_CUDA_OK(cudaFuncSetAttribute(ngcf::dense_dzwt_wide_kernel<DD, PEERS>,                                       \
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ngcf::kWideSmemBytes));      \
     AGCF_CUDA_OK(cudaFuncSetAttribute(ngcf::dense_wgrad_wide_kernel<DD>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
                                       (int)ngcf::kWideSmemBytes));                                                   \
     if (n_rows > 0)                                                                                                  \
-      ngcf::dense_dzwt_wide_kernel<DD><<<grid_dz, 256, ngcf::kWideSmemBytes, st>>>(dOut, Enext, P, E, WT, dP, dEdir,  \
-                                                                                   n_rows);                          \
+      ngcf::dense_dzwt_wide_kernel<DD, PEERS><<<grid_dz, 256, ngcf::kWideSmemBytes, st>>>(dOut, Enext, P, E, WT, dP,  \
+                                                                                          dEdir, n_rows, pp);        \
     ngcf::dense_wgrad_wide_kernel<DD><<<grid_w, 256, ngcf::kWideSmemBytes, st>>>(dOut, Enext, P, E, dW_partial,       \
                                                                                  n_rows);                            \
   }
@@ -619,17 +718,17 @@ extern "C" int agcf_ngcf_dense_backward(const float* dOut, const float* Enext, c
     return AGCF_OK;
   }
   if (d <= 16) {
-    if (d == 16) ngcf::dense_bwd_small_kernel<16><<<(unsigned)n_partials, ngcf::kSmallTM, 0, st>>>(dOut, Enext, P, E, WT, dP, dEdir, dW_partial, n_rows);
-    else ngcf::dense_bwd_small_kernel<8><<<(unsigned)n_partials, ngcf::kSmallTM, 0, st>>>(dOut, Enext, P, E, WT, dP, dEdir, dW_partial, n_rows);
+    if (d == 16) ngcf::dense_bwd_small_kernel<16, PEERS><<<(unsigned)n_partials, ngcf::kSmallTM, 0, st>>>(dOut, Enext, P, E, WT, dP, dEdir, dW_partial, n_rows, pp);
+    else ngcf::dense_bwd_small_kernel<8, PEERS><<<(unsigned)n_partials, ngcf::kSmallTM, 0, st>>>(dOut, Enext, P, E, WT, dP, dEdir, dW_partial, n_rows, pp);
     AGCF_LAUNCH_OK();
     return AGCF_OK;
   }
 #define AGCF_NGCF_BWD(DD)                                                                                      \
   {                                                                                                            \
-    AGCF_CUDA_OK(cudaFuncSetAttribute(ngcf::dense_bwd_kernel<DD>, cudaFuncAttributeMaxDynamicSharedMemorySize,  \
+    AGCF_CUDA_OK(cudaFuncSetAttribute(ngcf::dense_bwd_kernel<DD, PEERS>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
                                       (int)ngcf::BwdSmem<DD>::bytes));                                         \
-    ngcf::dense_bwd_kernel<DD><<<(unsigned)n_partials, 256, ngcf::BwdSmem<DD>::bytes, st>>>(                   \
-        dOut, Enext, P, E, WT, dP, dEdir, dW_partial, n_rows);                                                 \
+    ngcf::dense_bwd_kernel<DD, PEERS><<<(unsigned)n_partials, 256, ngcf::BwdSmem<DD>::bytes, st>>>(            \
+        dOut, Enext, P, E, WT, dP, dEdir, dW_partial, n_rows, pp);                                             \
   }
   if (d == 64) AGCF_NGCF_BWD(64) else AGCF_NGCF_BWD(32)
 #undef AGCF_NGCF_BWD
@@ -637,12 +736,66 @@ extern "C" int agcf_ngcf_dense_backward(const float* dOut, const float* Enext, c
   return AGCF_OK;
 }
 
-extern "C" int agcf_ngcf_reduce_wgrad(const float* dW_partial, int32_t n_partials, float* dW, int32_t d,
-                                      agcf_stream_t stream) {
+template <bool PEERS>
+int reduce_wgrad(const float* dW_partial, int32_t n_partials, float* dW, int32_t d, ngcf::RowPeers pw, cudaStream_t st) {
   if (!dW_partial || !dW || n_partials < 1) return AGCF_EINVAL;
   if (d != 8 && d != 16 && d != 32 && d != 64 && d != 128 && d != 256) return AGCF_EUNSUPPORTED;
   const int n = 2 * d * d;
-  ngcf::reduce_wgrad_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(dW_partial, n_partials, n, dW);
+  ngcf::reduce_wgrad_kernel<PEERS><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(dW_partial, n_partials, n, dW, pw);
   AGCF_LAUNCH_OK();
   return AGCF_OK;
+}
+
+}  // namespace
+
+extern "C" int agcf_ngcf_dense_forward(const float* P, const float* E, const float* W, float* Enext,
+                                       const float* acc_in, float* acc_out, float acc_div,
+                                       int32_t n_rows, int32_t d, agcf_stream_t stream) {
+  return dense_forward<false>(P, E, W, Enext, acc_in, acc_out, acc_div, n_rows, d, ngcf::RowPeers{}, ngcf::RowPeers{},
+                              (cudaStream_t)stream);
+}
+
+extern "C" int agcf_ngcf_dense_backward(const float* dOut, const float* Enext, const float* P, const float* E,
+                                        const float* WT, float* dP, float* dEdir, float* dW_partial,
+                                        int32_t n_partials, int32_t n_rows, int32_t d, agcf_stream_t stream) {
+  return dense_backward<false>(dOut, Enext, P, E, WT, dP, dEdir, dW_partial, n_partials, n_rows, d, ngcf::RowPeers{},
+                               (cudaStream_t)stream);
+}
+
+extern "C" int agcf_ngcf_reduce_wgrad(const float* dW_partial, int32_t n_partials, float* dW, int32_t d,
+                                      agcf_stream_t stream) {
+  return reduce_wgrad<false>(dW_partial, n_partials, dW, d, ngcf::RowPeers{}, (cudaStream_t)stream);
+}
+
+extern "C" int agcf_ngcf_dense_forward_peers(const float* P, const float* E, const float* W, float* Enext,
+                                             const float* acc_in, float* acc_out, float acc_div,
+                                             int32_t n_rows, int32_t d,
+                                             void* const* peer_Enext_host, void* const* peer_acc_host, int32_t n_peers,
+                                             void* mc_Enext, void* mc_acc, agcf_stream_t stream) {
+  if (n_peers < 0 || n_peers > AGCF_MAX_PEERS || (mc_acc != nullptr && acc_out == nullptr) ||
+      ((peer_acc_host != nullptr || mc_acc != nullptr) && acc_out == nullptr))
+    return AGCF_EINVAL;
+  ngcf::RowPeers pn, pa;
+  if (!make_peers(peer_Enext_host, n_peers, mc_Enext, pn) || !make_peers(peer_acc_host, n_peers, mc_acc, pa)) return AGCF_EINVAL;
+  return dense_forward<true>(P, E, W, Enext, acc_in, acc_out, acc_div, n_rows, d, pn, pa, (cudaStream_t)stream);
+}
+
+extern "C" int agcf_ngcf_dense_backward_peers(const float* dOut, const float* Enext, const float* P, const float* E,
+                                              const float* WT, float* dP, float* dEdir, float* dW_partial,
+                                              int32_t n_partials, int32_t n_rows, int32_t d,
+                                              void* const* peer_dP_host, int32_t n_peers, void* mc_dP,
+                                              agcf_stream_t stream) {
+  if (n_peers < 0 || n_peers > AGCF_MAX_PEERS) return AGCF_EINVAL;
+  ngcf::RowPeers pp;
+  if (!make_peers(peer_dP_host, n_peers, mc_dP, pp)) return AGCF_EINVAL;
+  return dense_backward<true>(dOut, Enext, P, E, WT, dP, dEdir, dW_partial, n_partials, n_rows, d, pp, (cudaStream_t)stream);
+}
+
+extern "C" int agcf_ngcf_reduce_wgrad_peers(const float* dW_partial, int32_t n_partials, float* dW, int32_t d,
+                                            void* const* peer_dW_host, int32_t n_peers, void* mc_dW,
+                                            agcf_stream_t stream) {
+  if (n_peers < 0 || n_peers > AGCF_MAX_PEERS) return AGCF_EINVAL;
+  ngcf::RowPeers pw;
+  if (!make_peers(peer_dW_host, n_peers, mc_dW, pw)) return AGCF_EINVAL;
+  return reduce_wgrad<true>(dW_partial, n_partials, dW, d, pw, (cudaStream_t)stream);
 }

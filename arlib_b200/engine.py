@@ -179,23 +179,24 @@ class LightGCNEngine:
             torch.cuda.synchronize()
             comm.barrier()
         else:
-            # row partition: this rank computes rows [r0, r1); layer tables live in one symmetric arena
-            bounds = graph.row_ranges(comm.world)
+            # row partition: this rank computes rows [r0, r1); the tables peers write live in one symmetric arena
+            bounds = self._row_ranges(graph, comm.world)
             self.bounds = bounds
             self.r0, self.r1 = bounds[comm.rank], bounds[comm.rank + 1]
             self.g = graph.partition(self.r0, self.r1)
-            shape = (self.N, self.d)
-            bufs = comm.allocate({k: (shape, torch.float32) for k in ("E0", "F", "fw0", "fw1", "bw0", "bw1")})
+            specs = self._symmetric_tables(comm.world)
+            bufs = comm.allocate(specs)
+            self.sym = bufs
             self.E0 = bufs["E0"]
             self.E0.copy_(table)
             self.F = bufs["F"]
-            self.fw = [bufs["fw0"], bufs["fw1"]]
-            self.bw = [bufs["bw0"], bufs["bw1"]]
+            self.fw = [bufs[k] for k in ("fw0", "fw1") if k in bufs]
+            self.bw = [bufs[k] for k in ("bw0", "bw1") if k in bufs]
             row_off = self.r0 * self.d * 4
-            self._peer = {k: comm.peers(k) for k in ("E0", "F", "fw0", "fw1", "bw0", "bw1")}
+            self._peer = {k: comm.peers(k) for k in specs}
             self._peer_E0_rows = comm.peers("E0", row_off)
             # NVSwitch multicast mappings of the same buffers (0 when unavailable): one store reaches all copies
-            self._mc = {k: comm.multicast_ptr(k) for k in ("E0", "F", "fw0", "fw1", "bw0", "bw1")}
+            self._mc = {k: comm.multicast_ptr(k) for k in specs}
             self._mc_E0_rows = comm.multicast_ptr("E0", row_off)
             torch.cuda.synchronize()
             comm.barrier()
@@ -247,6 +248,14 @@ class LightGCNEngine:
         self._refresh_adam_coefs()
 
     WL_SEGMENT = int(__import__('os').environ.get('ARLIB_B200_WL_SEGMENT', '64'))
+
+    def _row_ranges(self, graph, world):
+        """row boundaries of the row-partitioned layout: the step is a chain of SpMMs, whose time follows the nnz"""
+        return graph.row_ranges(world)
+
+    def _symmetric_tables(self, world):
+        """{name: (shape, dtype)} of the row-partitioned layout's symmetric arena: the tables peers store into"""
+        return {k: ((self.N, self.d), torch.float32) for k in ("E0", "F", "fw0", "fw1", "bw0", "bw1")}
 
     def _init_worklists(self, nbmax, dev):
         """Capacity of a batch's work list = the 3B rows with the most segments (an upper bound for any batch)."""
@@ -789,8 +798,8 @@ class ContrastiveEngine(LightGCNEngine):
 
 
 class NGCFEngine(LightGCNEngine):
-    """Fused NGCF training step (single GPU): the body of recommender/NGCF.py:48-66 with the encoder of :197-212 as a
-    fixed kernel sequence, capturable in a CUDA graph.
+    """Fused NGCF training step: the body of recommender/NGCF.py:48-66 with the encoder of :197-212 as a fixed kernel
+    sequence, capturable in a CUDA graph.
 
     Per layer ONE propagation P = A E (agcf_spmm_csr_f32; the reference runs two -- A (E W1) = (A E) W1) and one fused
     dense kernel  E' = leaky_relu([P + E | P * E] [W1 ; W2])  that also keeps the running layer mean
@@ -799,43 +808,106 @@ class NGCFEngine(LightGCNEngine):
     as addends).  Adam on the embedding table is fused into the last backward SpMM, Adam on the 2L weight matrices is
     one agcf_adam_step_f32 over their packed buffer ``W`` ([L, 2d, d], row block k = [W1_k ; W2_k]).
 
-    launches per step: L x (SpMM + dense) + loss fwd/bwd + L x (dense + reduce + SpMM) + W transpose + 2 optimizer."""
+    launches per step: L x (SpMM + dense) + loss fwd/bwd + L x (dense + reduce + SpMM) + W transpose + 2 optimizer.
+
+    ``comm`` (a DistContext, more than one rank): rows and adjacency rows split over the ranks (mode "rows"; the
+    column-sharded "dshard" layout cannot hold NGCF, whose [2d, d] weights mix every column of a row).  Rank r owns rows
+    [r0, r1) and runs every kernel of the step on them alone: the dense product is row-local, so it divides by the rank
+    count.  The dense kernels' epilogues store E_1 .. E_{L-1}, the finished layer mean F and dP into every rank's copy
+    (the next SpMM gathers them there), each rank's share of dW goes to its slot of every rank's [L, P, 2d*d] buffer, and
+    every rank sums the P slots in rank order: dW, the W step and so W are bit-identical everywhere.  Adam updates the
+    own rows of E0 in every copy.  One barrier per forward layer, one per backward layer, one closing the step."""
 
     # rows of the dW partial buffer.  d <= 64: the persistent CTAs of the backward dense kernel (two per SM).  d = 128 and
     # 256: the row slices of the split-K weight-gradient kernel, whose 2 / 8 output tiles times the slices fill the 148 SMs
     # once or twice; a partial is a whole 2d x d matrix (512 KB at d = 256), so 296 of them would be 150 MB
     N_PARTIALS = {8: 296, 16: 296, 32: 296, 64: 296, 128: 74, 256: 37}
+    # row-partitioned layout: the ranks' row ranges balance a * nnz + b * rows (graph.balanced_row_ranges), with a and b
+    # the single-GPU time in us per non-zero of a layer's two SpMMs and per row of its dense forward + backward, measured
+    # at the Gowalla shape on a B200 at 1000 W (profiles/r5_ngcf_rows_p1.jsonl, tools/ngcf_dist_bench.py); other widths
+    # balance the non-zeros
+    ROW_COST = {64: (4.42e-5, 2.29e-3), 128: (7.04e-5, 7.39e-3), 256: (1.84e-4, 2.40e-2)}
 
-    def __init__(self, graph, table, W, n_users, lr, reg, batch_size, max_triples, betas=(0.9, 0.999), adam_eps=1e-8):
+    def __init__(self, graph, table, W, n_users, lr, reg, batch_size, max_triples, betas=(0.9, 0.999), adam_eps=1e-8,
+                 comm=None, mode="rows"):
         n_layers = int(W.shape[0])
         d = table.shape[1]
         if d not in self.N_PARTIALS or tuple(W.shape) != (n_layers, 2 * d, d) or not W.is_contiguous():
             raise ValueError("NGCFEngine: d in {8, 16, 32, 64, 128, 256} and W packed as [L, 2d, d]")
+        if mode == "dshard":
+            raise ValueError("NGCFEngine cannot shard columns: its [2d, d] weight matrices mix every column of a row, so "
+                             "a column slice of a layer needs all columns of the previous one; use mode='rows'")
         super().__init__(graph, table, n_users, n_layers, lr, reg, batch_size, max_triples, betas=betas, adam_eps=adam_eps,
-                         sparse_layers=False)
+                         sparse_layers=False, comm=comm, mode=mode)
         f = lambda: torch.empty_like(table)
         self.W = W
         self.Wm, self.Wv, self.dW = torch.zeros_like(W), torch.zeros_like(W), torch.zeros_like(W)
         self.WT = torch.empty((n_layers, d, 2 * d), dtype=torch.float32, device=table.device)
         self.dW_partial = torch.empty((self.N_PARTIALS[d], 2 * d * d), dtype=torch.float32, device=table.device)
         self.P = [f() for _ in range(self.L)]            # A E_{k-1}
-        self.Ek = [f() for _ in range(self.L)]           # layer outputs E_1 .. E_L
-        self.dP, self.dEdir = f(), f()
+        self.dEdir = f()
         self.dOut = [f(), f()]
-        self.fuse_adam = True
-        self.launches_per_step = 5 * self.L + 6
+        if self.mode == "rows":
+            # E_1 .. E_{L-1} and dP (by layer parity: a fast rank writing layer k-1's dP must not overwrite the rows a slow
+            # one still gathers for layer k) are gathered by the next SpMM: symmetric; E_L is only read row-locally
+            self.Ek = [self.sym["E%d" % k] for k in range(1, self.L)] + [f()]
+            self.dPs = [self.sym["dP0"], self.sym["dP1"]]
+            self.dW_slots = self.sym["dW_slots"]             # [L, P, 2d*d]: slot r = rank r's share of dW
+            row_off = self.r0 * self.d * 4
+            tables = [k for k in self.sym if k != "dW_slots"]
+            self._peer_rows = {k: self.comm.peers(k, row_off) for k in tables}
+            self._mc_rows = {k: self.comm.multicast_ptr(k, row_off) for k in tables}
+            P_, r = self.comm.world, self.comm.rank
+            slot = lambda k: (k * P_ + r) * 2 * d * d * 4
+            self._peer_slot = [self.comm.peers("dW_slots", slot(k)) for k in range(self.L)]
+            self._mc_slot = [self.comm.multicast_ptr("dW_slots", slot(k)) for k in range(self.L)]
+            self.fuse_adam = False
+            # single-GPU count + the 2L + 1 barriers + L slot sums + zero_rows and the E0 Adam (not fused here)
+            self.launches_per_step = 5 * self.L + 6 + (2 * self.L + 1) + self.L + 2
+        else:
+            self.Ek = [f() for _ in range(self.L)]       # layer outputs E_1 .. E_L
+            self.dPs = [f()]
+            self.fuse_adam = True
+            self.launches_per_step = 5 * self.L + 6
+
+    def _row_ranges(self, graph, world):
+        return graph.row_ranges(world, cost=self.ROW_COST.get(self.d))
+
+    def _symmetric_tables(self, world):
+        t = ((self.N, self.d), torch.float32)
+        specs = {"E0": t, "F": t, "dP0": t, "dP1": t}
+        specs.update({"E%d" % k: t for k in range(1, self.L)})
+        specs["dW_slots"] = ((self.L, world, 2 * self.d * self.d), torch.float32)
+        return specs
 
     def _trained_state(self):
         return super()._trained_state() + [self.W, self.Wm, self.Wv]
 
+    def _rows(self, t):
+        return t[self.r0:self.r1]
+
     def forward_table(self, out=None, row_mask=None, worklist=None):
         F = self.F if out is None else out
+        rows = self.mode == "rows"
+        if rows and out is not None:
+            raise ValueError("row-partitioned forward writes the symmetric F table")
         x = self.E0
         for k in range(1, self.L + 1):
             last = k == self.L
             ops.spmm(self.g, x, Y=self.P[k - 1])
-            ops.ngcf_dense_forward(self.P[k - 1], x, self.W[k - 1], self.Ek[k - 1], acc_in=self.E0 if k == 1 else F,
-                                   acc_out=F, acc_div=float(self.L + 1) if last else 1.0)
+            if rows:
+                # own rows; E_k (k < L) and, at the last layer, F go to every rank's copy
+                peer = "F" if last else "E%d" % k
+                ops.ngcf_dense_forward(self._rows(self.P[k - 1]), self._rows(x), self.W[k - 1], self._rows(self.Ek[k - 1]),
+                                       acc_in=self._rows(self.E0 if k == 1 else F), acc_out=self._rows(F),
+                                       acc_div=float(self.L + 1) if last else 1.0,
+                                       peer_Enext=None if last else self._peer_rows[peer],
+                                       peer_acc=self._peer_rows[peer] if last else None,
+                                       mc_Enext=0 if last else self._mc_rows[peer], mc_acc=self._mc_rows[peer] if last else 0)
+                self._barrier()
+            else:
+                ops.ngcf_dense_forward(self.P[k - 1], x, self.W[k - 1], self.Ek[k - 1], acc_in=self.E0 if k == 1 else F,
+                                       acc_out=F, acc_div=float(self.L + 1) if last else 1.0)
             x = self.Ek[k - 1]
         return F
 
@@ -854,18 +926,47 @@ class NGCFEngine(LightGCNEngine):
         ops.bpr_forward(F, u, i, j, nb, self.U, self.reg, out4, self.coef, self.ws)
         # G = dLoss/dF / (L + 1): the share every layer output (and E0) receives through the mean
         ops.bpr_backward(F, u, i, j, nb, self.U, self.reg, 1.0 / (L + 1), out4, self.coef, occ, seg_off, seg_node, n_seg, self.G)
-        d_out = self.G
-        adam = (self.E0, self.m, self.v, self.adam_coefs, self.betas[0], self.betas[1], self.adam_eps)
-        for k in range(L, 0, -1):
-            x_prev = self.E0 if k == 1 else self.Ek[k - 2]
-            ops.ngcf_dense_backward(d_out, self.Ek[k - 1], self.P[k - 1], x_prev, self.WT[k - 1], self.dP, self.dEdir,
-                                    self.dW_partial, self.dW[k - 1])
-            if k > 1:                                    # dE_{k-1} = A dP + dE_direct + G
-                nxt = self.dOut[k % 2]
-                ops.spmm(self.g, self.dP, addend=self.dEdir, acc_in=self.G, acc_out=nxt)
-                d_out = nxt
-            else:                                        # dE_0 goes straight into Adam; the batch's rows of G are re-zeroed
-                ops.spmm(self.g, self.dP, addend=self.dEdir, acc_in=self.G, adam=adam, zero_acc_in=True)
+        if self.mode == "rows":
+            self._backward_rows(seg_node, n_seg, nb)
+        else:
+            d_out = self.G
+            dP = self.dPs[0]
+            adam = (self.E0, self.m, self.v, self.adam_coefs, self.betas[0], self.betas[1], self.adam_eps)
+            for k in range(L, 0, -1):
+                x_prev = self.E0 if k == 1 else self.Ek[k - 2]
+                ops.ngcf_dense_backward(d_out, self.Ek[k - 1], self.P[k - 1], x_prev, self.WT[k - 1], dP, self.dEdir,
+                                        self.dW_partial, self.dW[k - 1])
+                if k > 1:                                    # dE_{k-1} = A dP + dE_direct + G
+                    nxt = self.dOut[k % 2]
+                    ops.spmm(self.g, dP, addend=self.dEdir, acc_in=self.G, acc_out=nxt)
+                    d_out = nxt
+                else:                                        # dE_0 goes straight into Adam; the batch's rows of G are re-zeroed
+                    ops.spmm(self.g, dP, addend=self.dEdir, acc_in=self.G, adam=adam, zero_acc_in=True)
         ops.adam_step(self.W.view(-1), self.dW.view(-1), self.Wm.view(-1), self.Wv.view(-1), self.lr, self.betas[0],
                       self.betas[1], self.adam_eps, step_dev=self.step_dev)
         ops.adam_coefs(self.step_dev, self.adam_coefs, self.lr, self.betas[0], self.betas[1], increment=True)
+        self._barrier()
+
+    def _backward_rows(self, seg_node, n_seg, nb):
+        """the row-partitioned backward: own rows throughout, dP and the dW slots exchanged before each layer's barrier"""
+        R = self._rows
+        d_out = self.G
+        for k in range(self.L, 0, -1):
+            x_prev = self.E0 if k == 1 else self.Ek[k - 2]
+            dP, name = self.dPs[k % 2], "dP%d" % (k % 2)
+            ops.ngcf_dense_backward(R(d_out), R(self.Ek[k - 1]), R(self.P[k - 1]), R(x_prev), self.WT[k - 1], R(dP),
+                                    R(self.dEdir), self.dW_partial, self.dW_slots[k - 1, self.comm.rank],
+                                    peer_dP=self._peer_rows[name], mc_dP=self._mc_rows[name],
+                                    peer_dW=self._peer_slot[k - 1], mc_dW=self._mc_slot[k - 1])
+            self._barrier()
+            ops.ngcf_reduce_wgrad(self.dW_slots[k - 1], self.dW[k - 1])      # rank order: the same dW on every rank
+            # dE_{k-1} = A dP + dE_direct + G on own rows (k = 1: the gradient of E0)
+            nxt = self.dOut[k % 2] if k > 1 else self.dE0
+            ops.spmm(self.g, dP, addend=self.dEdir, acc_in=self.G, acc_out=nxt)
+            d_out = nxt
+        ops.zero_rows(seg_node, n_seg, 3 * nb, self.G)
+        # owner-computes: Adam on this rank's rows of E0, stored into every rank's copy
+        r0, r1 = self.r0, self.r1
+        ops.adam_step(self.E0[r0:r1], self.dE0[r0:r1], self.m[r0:r1], self.v[r0:r1], self.lr, self.betas[0],
+                      self.betas[1], self.adam_eps, step_dev=self.step_dev, peer_p=self._peer_E0_rows,
+                      mc_p=self._mc_E0_rows)

@@ -50,16 +50,28 @@ def default_segment(local_nnz, d=64):
     return (int(SPLIT_ENV) if SPLIT_ENV else seg), seg
 
 
-def balanced_row_ranges(indptr, world):
-    """Boundaries b[0..world] with b[0]=0, b[world]=n_rows and ~nnz/world non-zeros per range."""
+def balanced_row_ranges(indptr, world, cost=None):
+    """Boundaries b[0..world] with b[0]=0, b[world]=n_rows and ~nnz/world non-zeros per range.
+
+    cost = (a, b): balance a * nnz + b * rows per range instead -- for a step whose propagation time follows the
+    non-zeros and whose dense layer time follows the rows (NGCF), where nnz-balanced ranges give the ranks that hold
+    the many low-degree rows far more dense work."""
     indptr = np.asarray(indptr, dtype=np.int64)
     n = indptr.shape[0] - 1
-    nnz = int(indptr[-1])
+    if cost is None:
+        prefix, total = indptr, int(indptr[-1])
+        target_of = lambda p: total * p // world
+    else:
+        a, b = float(cost[0]), float(cost[1])
+        if a < 0 or b < 0 or a + b <= 0:
+            raise ValueError("row-range cost weights must be >= 0 and not both 0")
+        prefix = a * indptr.astype(np.float64) + b * np.arange(n + 1, dtype=np.float64)
+        total = float(prefix[-1])
+        target_of = lambda p: total * p / world
     bounds = [0]
     for p in range(1, world):
-        target = nnz * p // world
-        b = int(np.searchsorted(indptr, target, side="left"))
-        bounds.append(min(max(b, bounds[-1]), n))
+        b_ = int(np.searchsorted(prefix, target_of(p), side="left"))
+        bounds.append(min(max(b_, bounds[-1]), n))
     bounds.append(n)
     return bounds
 
@@ -141,10 +153,10 @@ class DeviceGraph:
         return self.val.device
 
     # -------------------------------------------------------------- partitioning
-    def row_ranges(self, world):
+    def row_ranges(self, world, cost=None):
         """world+1 boundaries of contiguous row ranges with ~equal nnz (power-law rows:
-        balance by non-zeros, not by rows)."""
-        return balanced_row_ranges(self.rowptr.cpu().numpy(), world)
+        balance by non-zeros, not by rows); cost = (a, b): ~equal a * nnz + b * rows."""
+        return balanced_row_ranges(self.rowptr.cpu().numpy(), world, cost)
 
     def partition(self, r0, r1, segment=None):
         """Graph that COMPUTES only rows [r0, r1) (one rank of the row-partitioned

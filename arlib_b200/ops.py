@@ -267,20 +267,38 @@ def infonce_backward(n, d, temperature, ws, grad_loss=None, scale=1.0, n_dev=Non
                "agcf_infonce_backward")
 
 
-def ngcf_dense_forward(P, E, W, Enext, acc_in=None, acc_out=None, acc_div=1.0):
-    """agcf_ngcf_dense_forward: Enext = leaky_relu([P + E | P * E] @ W, 0.01); acc_out = (acc_in + Enext) / acc_div."""
+def ngcf_dense_forward(P, E, W, Enext, acc_in=None, acc_out=None, acc_div=1.0, peer_Enext=None, peer_acc=None, mc_Enext=0,
+                       mc_acc=0):
+    """agcf_ngcf_dense_forward: Enext = leaky_relu([P + E | P * E] @ W, 0.01); acc_out = (acc_in + Enext) / acc_div.
+
+    Row-partitioned (agcf_ngcf_dense_forward_peers): P, E, Enext, acc_* are a rank's rows of the tables; peer_Enext /
+    peer_acc list the other ranks' copies of the same rows (device pointers), mc_Enext / mc_acc their multicast
+    addresses (0: none)."""
     for t, n in ((P, "P"), (E, "E"), (W, "W"), (Enext, "Enext"), (acc_in, "acc_in"), (acc_out, "acc_out")):
         _f32(t, n)
     n, d = P.shape
     if tuple(W.shape) != (2 * d, d) or tuple(E.shape) != (n, d) or tuple(Enext.shape) != (n, d):
         raise ValueError("NGCF layer shapes: P, E, Enext [N, d]; W [2d, d]")
-    _lib.check(_lib.load().agcf_ngcf_dense_forward(P.data_ptr(), E.data_ptr(), W.data_ptr(), Enext.data_ptr(), _p(acc_in),
-                                                   _p(acc_out), float(acc_div), n, d, _lib.stream_ptr()),
-               "agcf_ngcf_dense_forward")
+    lib = _lib.load()
+    if not (peer_Enext or peer_acc or mc_Enext or mc_acc):
+        _lib.check(lib.agcf_ngcf_dense_forward(P.data_ptr(), E.data_ptr(), W.data_ptr(), Enext.data_ptr(), _p(acc_in),
+                                               _p(acc_out), float(acc_div), n, d, _lib.stream_ptr()),
+                   "agcf_ngcf_dense_forward")
+        return
+    if peer_Enext and peer_acc and len(peer_Enext) != len(peer_acc):
+        raise ValueError("peer lists must have equal length")
+    pe, n1 = _lib.ptr_array(peer_Enext)
+    pa, n2 = _lib.ptr_array(peer_acc)
+    _lib.check(lib.agcf_ngcf_dense_forward_peers(P.data_ptr(), E.data_ptr(), W.data_ptr(), Enext.data_ptr(), _p(acc_in),
+                                                 _p(acc_out), float(acc_div), n, d, pe, pa, max(n1, n2), mc_Enext or None,
+                                                 mc_acc or None, _lib.stream_ptr()), "agcf_ngcf_dense_forward_peers")
 
 
-def ngcf_dense_backward(dOut, Enext, P, E, WT, dP, dEdir, dW_partial, dW):
-    """agcf_ngcf_dense_backward + agcf_ngcf_reduce_wgrad: dP, dEdir [N, d] and dW [2d, d] (dW_partial: [n_partials, 2d*d])."""
+def ngcf_dense_backward(dOut, Enext, P, E, WT, dP, dEdir, dW_partial, dW, peer_dP=None, mc_dP=0, peer_dW=None, mc_dW=0):
+    """agcf_ngcf_dense_backward + agcf_ngcf_reduce_wgrad: dP, dEdir [N, d] and dW [2d, d] (dW_partial: [n_partials, 2d*d]).
+
+    Row-partitioned (the _peers entry points): the row operands are a rank's rows; dP also goes to the other ranks'
+    copies (peer_dP / mc_dP) and the reduced dW -- this rank's share -- to its slot in theirs (peer_dW / mc_dW)."""
     for t, n in ((dOut, "dOut"), (Enext, "Enext"), (P, "P"), (E, "E"), (WT, "WT"), (dP, "dP"), (dEdir, "dEdir"),
                  (dW_partial, "dW_partial"), (dW, "dW")):
         _f32(t, n)
@@ -288,11 +306,35 @@ def ngcf_dense_backward(dOut, Enext, P, E, WT, dP, dEdir, dW_partial, dW):
     if tuple(WT.shape) != (d, 2 * d) or dW_partial.shape[1] != 2 * d * d or dW.numel() != 2 * d * d:
         raise ValueError("NGCF backward shapes: WT [d, 2d]; dW_partial [n_partials, 2d*d]; dW [2d, d]")
     lib = _lib.load()
-    _lib.check(lib.agcf_ngcf_dense_backward(dOut.data_ptr(), Enext.data_ptr(), P.data_ptr(), E.data_ptr(), WT.data_ptr(),
-                                            dP.data_ptr(), dEdir.data_ptr(), dW_partial.data_ptr(), dW_partial.shape[0], n, d,
-                                            _lib.stream_ptr()), "agcf_ngcf_dense_backward")
-    _lib.check(lib.agcf_ngcf_reduce_wgrad(dW_partial.data_ptr(), dW_partial.shape[0], dW.data_ptr(), d, _lib.stream_ptr()),
-               "agcf_ngcf_reduce_wgrad")
+    st = _lib.stream_ptr()
+    if peer_dP or mc_dP:
+        pp, npp = _lib.ptr_array(peer_dP)
+        _lib.check(lib.agcf_ngcf_dense_backward_peers(dOut.data_ptr(), Enext.data_ptr(), P.data_ptr(), E.data_ptr(),
+                                                      WT.data_ptr(), dP.data_ptr(), dEdir.data_ptr(), dW_partial.data_ptr(),
+                                                      dW_partial.shape[0], n, d, pp, npp, mc_dP or None, st),
+                   "agcf_ngcf_dense_backward_peers")
+    else:
+        _lib.check(lib.agcf_ngcf_dense_backward(dOut.data_ptr(), Enext.data_ptr(), P.data_ptr(), E.data_ptr(), WT.data_ptr(),
+                                                dP.data_ptr(), dEdir.data_ptr(), dW_partial.data_ptr(), dW_partial.shape[0],
+                                                n, d, st), "agcf_ngcf_dense_backward")
+    if peer_dW or mc_dW:
+        pw, npw = _lib.ptr_array(peer_dW)
+        _lib.check(lib.agcf_ngcf_reduce_wgrad_peers(dW_partial.data_ptr(), dW_partial.shape[0], dW.data_ptr(), d, pw, npw,
+                                                    mc_dW or None, st), "agcf_ngcf_reduce_wgrad_peers")
+    else:
+        _lib.check(lib.agcf_ngcf_reduce_wgrad(dW_partial.data_ptr(), dW_partial.shape[0], dW.data_ptr(), d, st),
+                   "agcf_ngcf_reduce_wgrad")
+
+
+def ngcf_reduce_wgrad(dW_partial, dW):
+    """agcf_ngcf_reduce_wgrad: dW = sum of the rows of dW_partial [n, 2d*d] in row order (the row-partitioned step sums
+    the ranks' slots with it, the same bits on every rank)."""
+    _f32(dW_partial, "dW_partial"); _f32(dW, "dW")
+    d = dW.shape[-1]
+    if dW_partial.shape[-1] != 2 * d * d or dW.numel() != 2 * d * d:
+        raise ValueError("NGCF weight-gradient shapes: dW_partial [n, 2d*d]; dW [2d, d]")
+    _lib.check(_lib.load().agcf_ngcf_reduce_wgrad(dW_partial.data_ptr(), dW_partial.numel() // (2 * d * d), dW.data_ptr(),
+                                                  d, _lib.stream_ptr()), "agcf_ngcf_reduce_wgrad")
 
 
 def adam_step(p, g, m, v, lr, beta1=0.9, beta2=0.999, eps=1e-8, step=0, step_dev=None, peer_p=None, mc_p=None):

@@ -321,6 +321,28 @@ int agcf_ngcf_dense_backward(const float* dOut, const float* Enext, const float*
                              int32_t n_partials, int32_t n_rows, int32_t d, agcf_stream_t stream);
 int agcf_ngcf_reduce_wgrad(const float* dW_partial, int32_t n_partials, float* dW, int32_t d,
                            agcf_stream_t stream);
+/* Row-partitioned variants (multi-GPU, one rank's rows [r0, r1) of the row-partitioned layout): the same
+ * computation, and every stored row also goes to the other ranks' copies, so that the next propagation can gather
+ * it there.  Every row pointer (P, E, Enext, acc_*, dOut, dP, dEdir) points at row r0 of its table and n_rows =
+ * r1 - r0; the peer pointers are offset the same way, so a row sits at the same index everywhere.
+ *   peer_*_host  HOST arrays of n_peers device pointers to the other ranks' copies (peer-mapped over NVLink), each
+ *                nullable: forward -- of Enext and of acc_out (the finished layer mean); backward -- of dP;
+ *                reduce -- of dW (this rank's slot of every rank's symmetric [P, 2d*d] slot buffer);
+ *   mc_*         nullable NVSwitch multicast addresses of the same ranges: one multimem.st reaches every copy and
+ *                the peer arrays are ignored for that output.
+ * The local outputs are bit-equal to the plain entry points'.  Visibility on the peers needs a barrier after.
+ * Summing the P slots in rank order (agcf_ngcf_reduce_wgrad with n_partials = P) gives every rank the same dW. */
+int agcf_ngcf_dense_forward_peers(const float* P, const float* E, const float* W, float* Enext,
+                                  const float* acc_in, float* acc_out, float acc_div,
+                                  int32_t n_rows, int32_t d,
+                                  void* const* peer_Enext_host, void* const* peer_acc_host, int32_t n_peers,
+                                  void* mc_Enext, void* mc_acc, agcf_stream_t stream);
+int agcf_ngcf_dense_backward_peers(const float* dOut, const float* Enext, const float* P, const float* E,
+                                   const float* WT, float* dP, float* dEdir, float* dW_partial,
+                                   int32_t n_partials, int32_t n_rows, int32_t d,
+                                   void* const* peer_dP_host, int32_t n_peers, void* mc_dP, agcf_stream_t stream);
+int agcf_ngcf_reduce_wgrad_peers(const float* dW_partial, int32_t n_partials, float* dW, int32_t d,
+                                 void* const* peer_dW_host, int32_t n_peers, void* mc_dW, agcf_stream_t stream);
 
 /* ------------------------------------------------------------------ optimizer
  * torch.optim.Adam step (defaults: amsgrad=False, weight_decay=0, maximize=False)
