@@ -77,17 +77,21 @@ def _mean_powers(A, X, L):
     return acc / (L + 1)
 
 
-def loss_grad_bounds(Fa, cF, F, u, i, j, U, reg):
+def loss_grad_bounds(Fa, cF, F, u, i, j, U, reg, eF=None):
     """Bounds of the fp32 loss row, the coefficients coef_t = d loss / d x_t and G = d loss / d F, when the fp32 table
-    the kernels read is within cF * UNIT * Fa of the float64 table F elementwise (Fa >= |F|).  First order in UNIT.
-    Returns loss4 (bound per entry), coef (bound per triple), Gabs (a magnitude >= |G|) and G (bound per element)."""
+    the kernels read is within eF of the float64 table F elementwise (default eF = cF * UNIT * Fa; Fa >= |F|).  First
+    order in UNIT.  Returns loss4 (bound per entry), coef (bound per triple), Gabs (a magnitude >= |G|) and G (bound
+    per element)."""
     d, nb, N = F.shape[1], u.numel(), F.shape[0]
     iu, ii, ij = u, U + i, U + j
+    if eF is None:
+        eF = cF * UNIT * Fa
     Pu, Pi, Pj = Fa[iu], Fa[ii], Fa[ij]
+    Eu, Ei, Ej = eF[iu], eF[ii], eF[ij]
     # x_t = <F_u, F_i> - <F_u, F_j>: two d-term dot products (d UNIT of the sum of |products| in any summation order)
-    # and a difference; each factor carries cF UNIT of its magnitude
+    # and a difference; each factor carries its error eF
     Px = (Pu * (Pi + Pj)).sum(1)
-    dx = (d + 1 + 2 * cF) * UNIT * Px
+    dx = (d + 1) * UNIT * Px + (Eu * (Pi + Pj) + Pu * (Ei + Ej)).sum(1)
     x = (F[iu] * (F[ii] - F[ij])).sum(1)
     s = torch.sigmoid(x)
     dl = s * (1 - s) / (1e-7 + s)                     # |d l_t / d x_t| <= 1
@@ -96,9 +100,9 @@ def loss_grad_bounds(Fa, cF, F, u, i, j, U, reg):
     # where l_t ~ 0, 8 UNIT absolute (the error of s relative to s); the batch mean is taken in double
     bpr_b = (dl * dx).mean() + 8 * UNIT * (lt.mean() + 1)
     nu, ni = F[iu].norm(), F[ii].norm()
-    # ||F[u_.]||_F: the table's error (cF UNIT of ||Fa[u_.]||), d + 4 UNIT for the sums of squares and the square root
-    nu_b = cF * UNIT * Pu.norm() + (d + 4) * UNIT * nu
-    ni_b = cF * UNIT * Pi.norm() + (d + 4) * UNIT * ni
+    # ||F[u_.]||_F: the table's error (||eF[u_.]||), d + 4 UNIT for the sums of squares and the square root
+    nu_b = Eu.norm() + (d + 4) * UNIT * nu
+    ni_b = Ei.norm() + (d + 4) * UNIT * ni
     loss = lt.mean() + reg * (nu + ni)
     loss4 = torch.stack([bpr_b + reg * (nu_b + ni_b) + 2 * UNIT * loss, bpr_b, nu_b, ni_b])
     # coef_t = -s (1 - s) / ((1e-7 + s) nb): |d coef / d x| <= 1 / (4 nb); expf and 7 roundings: 16 UNIT
@@ -106,14 +110,15 @@ def loss_grad_bounds(Fa, cF, F, u, i, j, U, reg):
     ec = dx / (4 * nb) + 16 * UNIT * cu
     # rows of G: user  sum_t coef_t (F_i - F_j) + reg F_u / nu, positive item  coef_t F_u + reg F_i / ni, negative item
     # -coef_t F_u.  Per term: the coefficient's error times |F|, |coef| times the table's error, three roundings
-    cF3 = (cF + 3) * UNIT
+    U3 = 3 * UNIT
     Gabs, Gerr = torch.zeros_like(F), torch.zeros_like(F)
     Gabs.index_add_(0, iu, cu[:, None] * (Pi + Pj) + reg * Pu / nu)
-    Gerr.index_add_(0, iu, (ec + cF3 * cu)[:, None] * (Pi + Pj) + reg * (cF3 * Pu / nu + Pu * nu_b / nu ** 2))
+    Gerr.index_add_(0, iu, ec[:, None] * (Pi + Pj) + cu[:, None] * (Ei + Ej + U3 * (Pi + Pj))
+                    + reg * ((Eu + U3 * Pu) / nu + Pu * nu_b / nu ** 2))
     Gabs.index_add_(0, ii, cu[:, None] * Pu + reg * Pi / ni)
-    Gerr.index_add_(0, ii, (ec + cF3 * cu)[:, None] * Pu + reg * (cF3 * Pi / ni + Pi * ni_b / ni ** 2))
+    Gerr.index_add_(0, ii, ec[:, None] * Pu + cu[:, None] * (Eu + U3 * Pu) + reg * ((Ei + U3 * Pi) / ni + Pi * ni_b / ni ** 2))
     Gabs.index_add_(0, ij, cu[:, None] * Pu)
-    Gerr.index_add_(0, ij, (ec + cF3 * cu)[:, None] * Pu)
+    Gerr.index_add_(0, ij, ec[:, None] * Pu + cu[:, None] * (Eu + U3 * Pu))
     # a node's occurrences are summed in fp32: (occurrences) UNIT of its magnitude
     occ = torch.bincount(torch.cat([iu, ii, ij]), minlength=N).double()
     Gerr += occ[:, None] * UNIT * Gabs
