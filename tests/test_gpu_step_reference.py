@@ -174,29 +174,40 @@ def _ratio(err, tol):
 def check_step(got, ref, bnd, p0, m0, v0, rows):
     """max(error / bound) per output of one step; > 1 is a failure.  got: the kernel's loss4, F (valid at ``rows``, the
     batch's nodes), m, v, p after the step and, when the step writes it, g = dE0; p0 / m0 / v0: the state before it."""
-    b1, b2, c1, c2, eps = ref["b1"], ref["b2"], ref["c1"], ref["c2"], ref["eps"]
     g, eg = ref["g"], bnd["g"]
-    gm = g.abs() + eg
-    m0d, v0d = m0.double(), v0.double()
-    m, v, p = got["m"].double(), got["v"].double(), got["p"].double()
     r = {"loss": _ratio((got["loss4"].double() - ref["loss4"]).abs(), bnd["loss4"]),
          "F": _ratio((got["F"][rows].double() - ref["F"][rows]).abs(), bnd["F"][rows])}
     if "g" in got:                                           # the unfused step writes dE0
         r["g"] = _ratio((got["g"].double() - g).abs(), eg)
+    r.update(adam_ratios(ref, g, eg, ref["m"], ref["v"], p0, m0, v0, got["m"], got["v"], got["p"]))
+    r["exact"] = 0.0 if far_exact(g, bnd["far"], p0, m0, v0, got["m"], got["v"], got["p"]) else math.inf
+    return r
+
+
+def adam_ratios(s, g, eg, m_ref, v_ref, p0, m0, v0, m, v, p):
+    """max(error / bound) of one Adam update of parameters p0 with moments m0, v0 by a gradient within eg of the float64
+    g: the kernel's m, v against the float64 m_ref, v_ref, and its p against the update of its own m, v.  s holds the
+    scalars b1, b2, c1, c2, eps the update used."""
+    b1, b2, c1, c2, eps = s["b1"], s["b2"], s["c1"], s["c2"], s["eps"]
+    gm = g.abs() + eg
+    m0d, v0d = m0.double(), v0.double()
+    md, vd, pd = m.double(), v.double(), p.double()
+    r = {}
     # m' = m + (1 - b1) (g - m): three roundings; v' = fma((1 - b2) g, g, b2 v): three roundings
-    r["m"] = _ratio((m - ref["m"]).abs(), (1 - b1) * eg + 3 * UNIT * ((1 - b1) * gm + m0d.abs()))
-    r["v"] = _ratio((v - ref["v"]).abs(), (1 - b2) * (2 * g.abs() + eg) * eg + 3 * UNIT * (b2 * v0d + (1 - b2) * gm * gm))
+    r["m"] = _ratio((md - m_ref).abs(), (1 - b1) * eg + 3 * UNIT * ((1 - b1) * gm + m0d.abs()))
+    r["v"] = _ratio((vd - v_ref).abs(), (1 - b2) * (2 * g.abs() + eg) * eg + 3 * UNIT * (b2 * v0d + (1 - b2) * gm * gm))
     # p' from the kernel's own m', v': c1, c2 rounded to float, sqrt, two divisions, + eps, the product: 8 UNIT of the
     # update, and the final subtraction rounds to p' (a few ulps of p)
-    upd = c1 * m / (v.sqrt() / c2 + eps)
-    r["p"] = _ratio((p - (p0.double() - upd)).abs(), 2 * _ulp32(got["p"]) + 8 * UNIT * upd.abs())
-    # exact: far from the batch the gradient is zero; where the moments are zero too nothing may change, to the bit
-    far = bnd["far"]
-    fresh = far & (m0 == 0).all(1) & (v0 == 0).all(1)
-    exact = bool((g[far] == 0).all()) and not _bits(got["m"][fresh]).any() and not _bits(got["v"][fresh]).any() \
-        and np.array_equal(_bits(got["p"][fresh]), _bits(p0[fresh]))
-    r["exact"] = 0.0 if exact else math.inf
+    upd = c1 * md / (vd.sqrt() / c2 + eps)
+    r["p"] = _ratio((pd - (p0.double() - upd)).abs(), 2 * _ulp32(p) + 8 * UNIT * upd.abs())
     return r
+
+
+def far_exact(g, far, p0, m0, v0, m, v, p):
+    """far from the batch the gradient is zero; where the moments are zero too nothing may change, to the bit"""
+    fresh = far & (m0 == 0).all(1) & (v0 == 0).all(1)
+    return bool((g[far] == 0).all()) and not _bits(m[fresh]).any() and not _bits(v[fresh]).any() \
+        and np.array_equal(_bits(p[fresh]), _bits(p0[fresh]))
 
 
 def _bits(t):
