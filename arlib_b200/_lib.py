@@ -83,6 +83,7 @@ SIGNATURES = {
     "agcf_ngcf_reduce_wgrad_peers": (c_int32, [P, I32, P, I32, P, I32, P, P]),
     "agcf_adam_step_f32": (c_int32, [P, P, P, P, I64, F32, F32, F32, F32, I32, P, P, I32, P, P]),
     "agcf_increment_i32": (c_int32, [P, P]),
+    "agcf_group_handoff": (c_int32, [P, P, I32, I32, P, P, P]),
     "agcf_score_topk_ws_bytes": (c_int64, [I32, I32, I32, I32]),
     "agcf_score_topk": (c_int32, [P, P, I32, P, I32, I32, P, P, I32, I32, I32, P, P, P, P, I64, P]),
     "agcf_score_group_max": (c_int32, [P, P, I32, P, I32, I32, P, P, I32, I32, P, P, I64, P]),

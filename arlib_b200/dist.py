@@ -55,15 +55,29 @@ class DistContext:
             self._off[name] = off
         return out
 
-    def peers(self, name, extra_bytes=0):
-        """device pointers of buffer ``name`` on all OTHER ranks (+ byte offset)"""
+    def peers(self, name, extra_bytes=0, ranks=None):
+        """device pointers of buffer ``name`` on all OTHER ranks (+ byte offset); ``ranks``: only those of this
+        subset, in its order"""
         base = self._off[name] + int(extra_bytes)
-        return [int(self.hdl.buffer_ptrs[r]) + base for r in range(self.world) if r != self.rank]
+        ranks = range(self.world) if ranks is None else ranks
+        return [int(self.hdl.buffer_ptrs[r]) + base for r in ranks if r != self.rank]
 
-    def all_ptrs(self, name, extra_bytes=0):
-        """device pointers of buffer ``name`` on ALL ranks in rank order (own copy included)"""
+    def all_ptrs(self, name, extra_bytes=0, ranks=None):
+        """device pointers of buffer ``name`` on ALL ranks in rank order (own copy included); ``ranks``: on the ranks
+        of this subset, in its order"""
         base = self._off[name] + int(extra_bytes)
-        return [int(self.hdl.buffer_ptrs[r]) + base for r in range(self.world)]
+        ranks = range(self.world) if ranks is None else ranks
+        return [int(self.hdl.buffer_ptrs[r]) + base for r in ranks]
+
+    def subgroups(self, groups):
+        """NCCL process groups of the disjoint rank lists ``groups`` (ranks of this context's group); returns the one
+        that holds this rank.  Every rank must call this with the same lists in the same order."""
+        mine = None
+        for ranks in groups:
+            pg = dist.new_group([dist.get_global_rank(self.group, r) for r in ranks])
+            if self.rank in ranks:
+                mine = pg
+        return mine
 
     def multicast_ptr(self, name, extra_bytes=0):
         """NVSwitch multicast address of buffer ``name`` (a store to it lands in every rank's copy), or 0

@@ -31,6 +31,29 @@ def dshard_columns(d, world, rank):
     return rank * w, (rank + 1) * w
 
 
+def grid_shape(grid, world):
+    """(R, C) of the grid layout on ``world`` ranks: R row blocks x C column slices, R >= 2, C >= 2, R * C = world
+    ((P, 1) and (1, P) are the modes "rows" and "dshard")."""
+    try:
+        R, C = (int(x) for x in grid)
+    except (TypeError, ValueError):
+        raise ValueError("grid must be a pair (R, C) of row blocks and column slices, got %r" % (grid,)) from None
+    if R < 2 or C < 2:
+        raise ValueError("grid (%d, %d): R >= 2 row blocks and C >= 2 column slices (a single row block is mode "
+                         "'dshard', a single column slice mode 'rows')" % (R, C))
+    if R * C != world:
+        raise ValueError("grid (%d, %d): R * C = %d ranks, the process group has %d" % (R, C, R * C, world))
+    return R, C
+
+
+def grid_groups(R, C, rank):
+    """Rank r * C + c of the grid owns row block r and column slice c.  Returns (r, c, column group, row group): the
+    column group is the R ranks with slice c (they exchange layer rows), the row group the C ranks with block r (they
+    exchange the loss's partial scores)."""
+    r, c = divmod(rank, C)
+    return r, c, [q * C + c for q in range(R)], [r * C + q for q in range(C)]
+
+
 class DeviceTrainSet:
     """Device mirror of what util/sampler.py:4-30 reads from ``data``: the edge list
     (data.training_data through data.user / data.item) and, per user, the sorted item
@@ -124,17 +147,23 @@ class LightGCNEngine:
                   [r*d/P, (r+1)*d/P)): propagation, backward and Adam need no communication at all, the
                   only exchange of a step is 32 bytes per triple per peer (the partial scores, each value
                   stamped with the step so that the consumer needs no barrier).  Needs d/P in {8, 16, 32, ...}
-                  and the graph to fit on one GPU."""
+                  and the graph to fit on one GPU;
+      "grid"   -- ``grid=(R, C)``: rank r*C + c owns row block r and column slice c.  Inside each column group (the R
+                  ranks of slice c) the step is the "rows" step on [N, d/C] tables, each layer closed by a hand-off
+                  among those R ranks (agcf_group_handoff) instead of an all-rank barrier; inside each row group (the
+                  C ranks of block r) the loss is the "dshard" exchange.  Tables are N x d/C per GPU."""
 
     def __init__(self, graph: DeviceGraph, table: torch.Tensor, n_users: int, n_layers: int,
                  lr: float, reg: float, batch_size: int, max_triples: int,
-                 betas=(0.9, 0.999), adam_eps=1e-8, sparse_layers=True, comm=None, mode="rows"):
+                 betas=(0.9, 0.999), adam_eps=1e-8, sparse_layers=True, comm=None, mode="rows", grid=None):
         if 3 * batch_size > 16384:
             raise ValueError("batch_size %d too large for the single-CTA batch grouping (max 5461)" % batch_size)
         if n_layers < 1:
             raise ValueError("n_layers must be >= 1")
-        if mode not in ("rows", "dshard"):
-            raise ValueError("mode must be 'rows' or 'dshard'")
+        if mode not in ("rows", "dshard", "grid"):
+            raise ValueError("mode must be 'rows', 'dshard' or 'grid'")
+        if mode == "grid":
+            grid_shape(grid, comm.world if comm is not None else 1)
         self.N, self.d_full = table.shape
         self.d = self.d_full
         self.U, self.L = int(n_users), int(n_layers)
@@ -176,6 +205,50 @@ class LightGCNEngine:
             # optimizer state -- a stamp is used once
             self.xchg_ctr = torch.zeros(1, dtype=torch.int32, device=dev)
             self._xchg_all = comm.all_ptrs("xchg")
+            self.xchg_rank = comm.rank
+            torch.cuda.synchronize()
+            comm.barrier()
+        elif self.mode == "grid":
+            R, C = grid_shape(grid, comm.world)
+            self.grid = (R, C)
+            self.grid_r, self.grid_c, self.col_group, self.row_group = grid_groups(R, C, comm.rank)
+            c0, c1 = dshard_columns(self.d_full, C, self.grid_c)
+            self.d = c1 - c0
+            self.col0, self.col1 = c0, c1
+            self.bounds = self._row_ranges(graph, R)
+            self.r0, self.r1 = self.bounds[self.grid_r], self.bounds[self.grid_r + 1]
+            self.g = graph.partition(self.r0, self.r1).planned_for(self.d)
+            specs = self._symmetric_tables(R)
+            tables = list(specs)
+            specs["xchg"] = ((ops.bpr_xchg_bytes(self.B),), torch.uint8)
+            specs["handoff"] = ((8,), torch.int32)
+            bufs = comm.allocate(specs)
+            self.sym = bufs
+            self.E0 = bufs["E0"]
+            self.E0.copy_(table[:, c0:c1])
+            table = self.E0
+            f = lambda: torch.empty_like(self.E0)
+            self.F = bufs["F"]
+            self.fw = [bufs[k] for k in ("fw0", "fw1") if k in bufs]
+            self.bw = [bufs[k] for k in ("bw0", "bw1") if k in bufs]
+            # layer rows go to the column group's partners (no multicast: a multicast object spans every rank)
+            self._peer = {k: comm.peers(k, ranks=self.col_group) for k in tables}
+            self._peer_E0_rows = comm.peers("E0", self.r0 * self.d * 4, ranks=self.col_group)
+            self._mc = {k: 0 for k in tables}
+            self._mc_E0_rows = 0
+            # the loss's partial scores go to the row group (bpr_partial / bpr_finish with group rank and pointers)
+            self.xchg = bufs["xchg"]
+            self.xchg.zero_()
+            self.xchg_ctr = torch.zeros(1, dtype=torch.int32, device=dev)
+            self._xchg_all = comm.all_ptrs("xchg", ranks=self.row_group)
+            self.xchg_rank = self.grid_c
+            # column-group hand-off: flag words (slot = position in the group), its own stamp counter, never restored
+            self.handoff_flags = bufs["handoff"]
+            self.handoff_flags.zero_()
+            self._handoff_peers = comm.peers("handoff", ranks=self.col_group)
+            self.handoff_ctr = torch.zeros(1, dtype=torch.int32, device=dev)
+            self.handoff_err = torch.zeros(1, dtype=torch.int32, device=dev)
+            self.row_pg = comm.subgroups([grid_groups(R, C, q * C)[3] for q in range(R)])
             torch.cuda.synchronize()
             comm.barrier()
         else:
@@ -233,7 +306,7 @@ class LightGCNEngine:
             self._init_worklists(nbmax, dev)
         # Adam fused into the epilogue of the last backward SpMM (own rows == all rows: not in "rows" mode,
         # where the updated rows also go to the peers)
-        self.fuse_adam = self.mode != "rows" and flag("ARLIB_B200_FUSE_ADAM")
+        self.fuse_adam = self.mode not in ("rows", "grid") and flag("ARLIB_B200_FUSE_ADAM")
         self.adam_coefs = torch.zeros(2, dtype=torch.float32, device=dev)
         self.out4 = torch.zeros((nbmax, 4), dtype=torch.float32, device=dev)
         self.coef = torch.empty(self.B, dtype=torch.float32, device=dev)
@@ -242,7 +315,8 @@ class LightGCNEngine:
         self._ext = None
         self._loss_eager = None
         self.dist_graphs = _os.environ.get("ARLIB_B200_DIST_GRAPHS", "1") == "1"
-        self.launches_per_step = {"single": 2 * self.L + 5, "rows": 4 * self.L + 5, "dshard": 2 * self.L + 6}[self.mode]
+        self.launches_per_step = {"single": 2 * self.L + 5, "rows": 4 * self.L + 5, "dshard": 2 * self.L + 6,
+                                  "grid": 4 * self.L + 6}[self.mode]
         if self.fuse_adam:       # no adam kernel; no zero_rows kernel either when the last backward layer re-zeroes G
             self.launches_per_step -= 2 if self.L > 1 else 1
         self._refresh_adam_coefs()
@@ -301,7 +375,7 @@ class LightGCNEngine:
         ops.adam_coefs(self.step_dev, self.adam_coefs, self.lr, self.betas[0], self.betas[1], increment=False)
 
     def _peers(self, name):
-        return self._peer[name] if self.mode == "rows" else None
+        return self._peer[name] if self.mode in ("rows", "grid") else None
 
     def _mcast(self, name):
         return self._mc[name] if self.mode == "rows" else 0
@@ -309,17 +383,32 @@ class LightGCNEngine:
     def _barrier(self):
         if self.mode == "rows":
             self.comm.barrier()
+        elif self.mode == "grid":
+            ops.group_handoff(self.handoff_flags, self._handoff_peers, self.grid_r, self.handoff_ctr, self.handoff_err)
+
+    def check_handoff(self):
+        """Grid layout: wait for the device and raise if a column-group hand-off gave up on a partner (4 s without
+        its stamp: a rank that crashed or issued another launch sequence); the tables are then not to be trusted."""
+        if self.mode == "grid":
+            torch.cuda.current_stream().synchronize()
+            if int(self.handoff_err.item()):
+                raise RuntimeError("grid layout: rank %d waited 4 s for a column-group partner in a hand-off; the "
+                                   "training state is inconsistent" % self.comm.rank)
 
     def full_table(self, local: torch.Tensor) -> torch.Tensor:
         """[N, d] table from this rank's copy: identity except in "dshard" mode, where the P column
-        slices are all-gathered (NCCL) and interleaved back -- used once per evaluation / export,
-        never inside a training step."""
-        if self.mode != "dshard":
+        slices are all-gathered (NCCL) and interleaved back, and in "grid" mode, where the C slices of the
+        row group are -- used once per evaluation / export, never inside a training step."""
+        if self.mode not in ("dshard", "grid"):
             return local
         import torch.distributed as dist
-        w = self.comm.world
+        if self.mode == "dshard":
+            w, group = self.comm.world, self.comm.group
+        else:
+            self.check_handoff()
+            w, group = self.grid[1], self.row_pg
         parts = torch.empty((w * local.shape[0], local.shape[1]), dtype=local.dtype, device=local.device)
-        dist.all_gather_into_tensor(parts, local.contiguous(), group=self.comm.group)
+        dist.all_gather_into_tensor(parts, local.contiguous(), group=group)
         return parts.view(w, self.N, -1).permute(1, 0, 2).reshape(self.N, self.d_full).contiguous()
 
     # ------------------------------------------------------------ epoch set-up
@@ -368,7 +457,7 @@ class LightGCNEngine:
         Multi-GPU: every layer's rows are also stored into the peers' tables by the SpMM
         epilogue and a barrier closes the layer (``out`` must then be self.F)."""
         F = self.F if out is None else out
-        if self.mode == "rows" and out is not None:
+        if self.mode in ("rows", "grid") and out is not None:
             raise ValueError("row-partitioned forward writes the symmetric F table")
         x = self.E0
         for k in range(1, self.L + 1):
@@ -390,7 +479,7 @@ class LightGCNEngine:
         1 .. L-1 write only E_k; the last layer's epilogue forms ((E0 + E1) + ... + E_{L-1} + t) / (L + 1), the same
         adds in the same order as the running sum of forward_table, so F is bit-identical on those rows.  The
         row-partitioned layout (whose layers also go to the peers) and more than 8 layers keep forward_table."""
-        if self.mode == "rows" or self.L > 8:
+        if self.mode in ("rows", "grid") or self.L > 8:
             return self.forward_table(row_mask=row_mask, worklist=worklist)
         x = self.E0
         for k in range(1, self.L):
@@ -415,11 +504,11 @@ class LightGCNEngine:
             F = self._forward_batch(mask, self._worklist(b))
         else:
             F = self.forward_table()
-        if self.mode == "dshard":
+        if self.mode in ("dshard", "grid"):
             # the step's only exchange: 32 B per triple to every peer, stamped with the step -- bpr_finish spins on
-            # the words it needs, no barrier launch (csrc/bpr.cu)
-            ops.bpr_partial(F, u, i, j, nb, self.U, self.comm.rank, self.B, self.xchg_ctr, self._xchg_all)
-            ops.bpr_finish(self.xchg, self.comm.world, self.B, nb, self.reg, self.xchg_ctr, out4, self.coef, self.ws)
+            # the words it needs, no barrier launch (csrc/bpr.cu).  Grid: among the row group's C column slices
+            ops.bpr_partial(F, u, i, j, nb, self.U, self.xchg_rank, self.B, self.xchg_ctr, self._xchg_all)
+            ops.bpr_finish(self.xchg, len(self._xchg_all), self.B, nb, self.reg, self.xchg_ctr, out4, self.coef, self.ws)
         else:
             ops.bpr_forward(F, u, i, j, nb, self.U, self.reg, out4, self.coef, self.ws)
         ops.bpr_backward(F, u, i, j, nb, self.U, self.reg, 1.0, out4, self.coef, occ, seg_off, seg_node, n_seg, self.G)
@@ -429,7 +518,7 @@ class LightGCNEngine:
         # middle layer 43.2 -> 42.2 us); where it covers many, the bitmap load per work item costs more than the loads it
         # saves (ml-1m, 42 %: 37.1 -> 39.0 us), so graphs with fewer than 4 x 3B rows read G everywhere.  The
         # row-partitioned layout keeps the full reads too.
-        g_mask = mask if self.mode != "rows" and 12 * self.B <= self.N else None
+        g_mask = mask if self.mode not in ("rows", "grid") and 12 * self.B <= self.N else None
         # first backward layer: only the batch's gradient rows of H are non-zero.  The column-masked kernel skips the others
         # (27 vs 44 us at d = 64); on 8-column slices its extra bitmap round trip per chunk costs more than the zero rows it
         # avoids (26.4 vs 23.4 us, profiles/r2_summary.md section 5), so there the plain kernel gathers the zeros
@@ -462,7 +551,7 @@ class LightGCNEngine:
         r0, r1 = self.r0, self.r1
         ops.adam_step(self.E0[r0:r1], self.dE0[r0:r1], self.m[r0:r1], self.v[r0:r1], self.lr, self.betas[0],
                       self.betas[1], self.adam_eps, step_dev=self.step_dev,
-                      peer_p=self._peer_E0_rows if self.mode == "rows" else None,
+                      peer_p=self._peer_E0_rows if self.mode in ("rows", "grid") else None,
                       mc_p=self._mc_E0_rows if self.mode == "rows" else 0)
         ops.increment(self.step_dev)
         self._barrier()
@@ -509,6 +598,7 @@ class LightGCNEngine:
                 self._join_coefs()
                 self._restore(state)
                 torch.cuda.synchronize()
+                self.check_handoff()
                 with torch.cuda.graph(g):
                     for b in range(first_batch, first_batch + n_steps):
                         self._launch_step(b)
@@ -834,7 +924,7 @@ class NGCFEngine(LightGCNEngine):
         d = table.shape[1]
         if d not in self.N_PARTIALS or tuple(W.shape) != (n_layers, 2 * d, d) or not W.is_contiguous():
             raise ValueError("NGCFEngine: d in {8, 16, 32, 64, 128, 256} and W packed as [L, 2d, d]")
-        if mode == "dshard":
+        if mode in ("dshard", "grid"):
             raise ValueError("NGCFEngine cannot shard columns: its [2d, d] weight matrices mix every column of a row, so "
                              "a column slice of a layer needs all columns of the previous one; use mode='rows'")
         super().__init__(graph, table, n_users, n_layers, lr, reg, batch_size, max_triples, betas=betas, adam_eps=adam_eps,

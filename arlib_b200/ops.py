@@ -350,6 +350,17 @@ def increment(counter):
     _lib.check(_lib.load().agcf_increment_i32(counter.data_ptr(), _lib.stream_ptr()), "agcf_increment_i32")
 
 
+def group_handoff(flags, peer_flags, my_slot, stamp_dev, err):
+    """agcf_group_handoff: publish the next stamp into slot ``my_slot`` of every partner's flag words (``peer_flags``:
+    device pointers) and wait until every partner's stamp is in ``flags``; *err becomes 1 if one never arrives."""
+    _i32(flags, "flags"); _i32(stamp_dev, "stamp_dev"); _i32(err, "err")
+    if flags.numel() < len(peer_flags) + 1:
+        raise ValueError("flags needs one word per group member")
+    arr, n = _lib.ptr_array(peer_flags)
+    _lib.check(_lib.load().agcf_group_handoff(flags.data_ptr(), arr, n, int(my_slot), stamp_dev.data_ptr(), err.data_ptr(),
+                                              _lib.stream_ptr()), "agcf_group_handoff")
+
+
 def score_topk(user_emb, item_emb, K, user_rows=None, mask_rowptr=None, mask_items=None, item_offset=0, impl=0,
                n_u=None, ws=None, return_flags=False, out=None, keep_mask_bits=False):
     """agcf_score_topk over users ``user_rows`` (or the first n_u rows).  Returns

@@ -360,6 +360,18 @@ int agcf_adam_step_f32(float* p, const float* g, float* m, float* v, int64_t n,
                        int32_t step, const int32_t* step_dev,
                        void* const* peer_p_host, int32_t n_peers, void* mc_p, agcf_stream_t stream);
 int agcf_increment_i32(int32_t* counter, agcf_stream_t stream);
+
+/* Hand-off inside a group of ranks that store into each other's tables (the column group of the grid layout: the
+ * ranks that share a column slice), in place of an all-rank barrier launch.  flags: this rank's AGCF_MAX_PEERS int32
+ * flag words (peer-mapped, ZERO before the first use, slot s written only by group member s); peer_flags_host: HOST
+ * array of the n_peers partners' flag words (n_peers = group size - 1); my_slot: this rank's position in the group.
+ * stamp = *stamp_dev + 1 is stored with a system-scope release into slot my_slot of every partner, then the kernel
+ * waits (acquire) until every partner's slot of `flags` carries it, and sets *stamp_dev = stamp.  stamp_dev is a
+ * device int32 private to the group and never restored, so no stamp is used twice; every member must issue the same
+ * sequence of hand-offs.  Stores a kernel made before the hand-off (peer_Y / peer_acc / peer_p) are visible to every
+ * partner's kernels after it.  A partner missing for 4 s sets *err = 1 (never cleared here) and the wait gives up. */
+int agcf_group_handoff(int32_t* flags, void* const* peer_flags_host, int32_t n_peers, int32_t my_slot,
+                       int32_t* stamp_dev, int32_t* err, agcf_stream_t stream);
 /* if (increment) *step_dev += 1;  t = *step_dev + 1;  coefs = {lr / (1 - b1^t), sqrt(1 - b2^t)} -- the two
  * step-dependent scalars of the Adam update, for the optimizer fused into the last backward SpMM. */
 int agcf_adam_coefs(int32_t* step_dev, int32_t increment, float lr, float beta1, float beta2, float* coefs,
